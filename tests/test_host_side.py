@@ -287,6 +287,27 @@ def test_closest_gates_without_cuda_uses_the_reference_expression():
     assert app.closest_gates(gates, [], None, 4.0) == []
 
 
+def test_bench_dump_outputs_keeps_a_fixed_sample_under_the_budget(tmp_path):
+    """bench.py --dump-outputs: below the budget every array is written whole; above it, every array of more than one row
+    keeps the same seeded sample of its rows (row numbers written beside it), the same in every run."""
+    import bench
+
+    rng = np.random.default_rng(1)
+    arrays = {"assign": rng.integers(0, 1000, 200_000).astype(np.float64), "cen": rng.random((5000, 12)), "w": np.ones(1)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget=1_000_000)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(os.listdir(tmp_path / "b")) == ["assign.npy", "assign_rows.npy", "cen.npy", "cen_rows.npy", "w.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 1_000_000 + 128 * len(files)  # (+ .npy headers)
+    for name in ("assign", "cen"):
+        rows = np.load(tmp_path / "a" / f"{name}_rows.npy").astype(np.int64)
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert len(rows) > 0 and (got == arrays[name][rows]).all() and (got == np.load(tmp_path / "b" / f"{name}.npy")).all()
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    assert sorted(os.listdir(tmp_path / "whole")) == ["assign.npy", "cen.npy", "w.npy"]
+    assert (np.load(tmp_path / "whole" / "assign.npy") == arrays["assign"]).all()
+
+
 def test_generated_documents_carry_no_unfilled_field():
     """DESIGN.md / README.md are generated from tools/templates/*.in by tools/fill_docs.py: no @FIELD@ may survive, and
     the text around the numbers must be the template's."""
