@@ -61,8 +61,7 @@ SYMBOLS = {
     "ccb_assoc_nearest2": (C.c_int, [i32, vp, vp, vp, i64, vp, i64, i32, f64, vp, vp, vp]),
     "ccb_colminmax": (C.c_int, [i32, vp, vp, i64, i64, i32, vp, vp]),
     "ccb_ingest_scaled": (C.c_int, [vp, vp, i64, i64, vp, vp, vp, vp]),
-    "ccb_off_neighbours": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, f64, vp, vp, vp, i32, vp]),
-    "ccb_off_patch": (C.c_int, [i32, vp, vp, vp, vp, vp, i32, i64, i64]),
+    "ccb_off_neighbours": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, f64, f64, vp, vp, vp, C.POINTER(i64)]),
     "ccb_off_subspace": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, vp, vp, f64, vp]),
     "ccb_off_weighted": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, vp, vp, f64, f64, vp]),
     "ccb_off_clusters": (C.c_int, [i32, vp, i64, vp, vp, vp, f64, i64, i32, vp, vp, vp, vp]),

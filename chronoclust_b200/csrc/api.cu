@@ -115,8 +115,8 @@ struct ccb_handle {
         void *p = nullptr;
         size_t bytes = 0;
     };
-    enum { OB_CORE, OB_CLS, OB_NBR, OB_WNBR, OB_CNT, OB_BORDER, OB_NBORDER, OB_QUEUE, OB_LABEL, OB_ORDER, OB_CLOFF, OB_NCL,
-           OB_SUBMASK, OB_OMASK, OB_D1, OB_D2, OB_DC, OB_DW, OB_DEC, OB_COUNT };
+    enum { OB_CORE, OB_CLS, OB_NBR, OB_WNBR, OB_CNT, OB_QUEUE, OB_LABEL, OB_ORDER, OB_CLOFF, OB_NCL, OB_SUBMASK, OB_OMASK,
+           OB_D1, OB_D2, OB_DC, OB_DW, OB_COUNT };
     OffBuf ob[OB_COUNT];
     int off_csr_min_m = 0;
     ccb_stats st{};
@@ -820,13 +820,6 @@ double builtin_nrm2(const double *x, int n) {
     return (double)sqrtl(s);
 }
 
-template <typename T>
-struct DevBuf {
-    T *p = nullptr;
-    ~DevBuf() { cudaFree(p); }
-    cudaError_t alloc(size_t n) { return cudaMalloc(&p, std::max<size_t>(n, 1) * sizeof(T)); }
-};
-
 // grow-only buffer of the handle's offline workspace (contents are NOT preserved across a growth)
 int off_buf(ccb_handle *h, int which, size_t bytes) {
     ccb_handle::OffBuf &b = h->ob[which];
@@ -842,6 +835,15 @@ int off_buf(ccb_handle *h, int which, size_t bytes) {
     b.bytes = cap;
     return CCB_OK;
 }
+
+// status of the launches just made (h may be NULL: the stateless entry points)
+int launched(ccb_handle *h, const char *what) {
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? CCB_OK : fail(h, CCB_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+}
+
+// ---- the launchers of the offline stages, shared by ccb_offline and the stateless ccb_off_* entry points -------------
+// Rows [r0, r1) of M; the row-indexed outputs (nbr, cnt, submask, wnbr, iso, nnz) hold the rows from r0 on.
 
 int launch_off_neighbours(ccb_handle *h, cudaStream_t s, const double *cen, int M, int D, int r0, int r1, double E2,
                           uint32_t *nbr, int32_t *cnt, int32_t *border, int border_cap, int32_t *n_border) {
@@ -873,9 +875,92 @@ int launch_off_neighbours(ccb_handle *h, cudaStream_t s, const double *cen, int 
         ok = 1;
     })
     if (!ok) return fail(h, CCB_ELIMIT, "unsupported dimensionality %d", D);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(h, CCB_ECUDA, "k_off_neighbours launch: %s", cudaGetErrorString(e));
+    return launched(h, "k_off_neighbours launch");
+}
+
+// Kernel 4b with its borderline pairs settled: the pairs whose squared distance lies inside the guard band are decided on
+// the host with the BLAS dnrm2 the reference itself calls (NULL: builtin_nrm2), `<= E` inclusive, and patched into nbr /
+// cnt.  The pair list is scratch from the stream-ordered pool and grows to whatever the data needs (e.g. many coincident
+// centroids with upsilon = 0).  Synchronises s once, and once more when pairs exist.  *n_border = the number of pairs.
+int off_neighbours_settled(ccb_handle *h, cudaStream_t s, const double *cen, int M, int D, int r0, int r1, double E,
+                           double E2, void *dnrm2, uint32_t *nbr, int32_t *cnt, int64_t *n_border) {
+    int32_t *buf = nullptr; // [0] pair count | [1, 1 + 2 cap) pairs (row, col) | cap bytes of decisions
+    int32_t nb = 0;
+    int rc = CCB_OK;
+    auto done = [&](int r) {
+        cudaFreeAsync(buf, s);
+        return r;
+    };
+    for (int cap = 1 << 16;; cap = nb) {
+        cudaError_t e;
+        if ((e = cudaMallocAsync(&buf, 4 + (size_t)cap * 9, s)) != cudaSuccess)
+            return fail(h, CCB_ENOMEM, "borderline pairs (%d): %s", cap, cudaGetErrorString(e));
+        if (cudaMemsetAsync(buf, 0, 4, s) != cudaSuccess) return done(fail(h, CCB_ECUDA, "borderline count: clear failed"));
+        if ((rc = launch_off_neighbours(h, s, cen, M, D, r0, r1, E2, nbr, cnt, buf + 1, cap, buf))) return done(rc);
+        if (h) h->st.kernel_launches++;
+        if ((e = cudaMemcpyAsync(&nb, buf, 4, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
+            (e = cudaStreamSynchronize(s)) != cudaSuccess)
+            return done(fail(h, CCB_ECUDA, "borderline count: %s", cudaGetErrorString(e)));
+        if (nb <= cap) break;
+        cudaFreeAsync(buf, s);
+    }
+    *n_border = nb;
+    if (nb == 0) return done(CCB_OK);
+    std::vector<int32_t> pairs(2 * (size_t)nb);
+    std::vector<double> hc((size_t)M * D), x(D);
+    std::vector<uint8_t> dec(nb);
+    cudaError_t e;
+    if ((e = cudaMemcpy(pairs.data(), buf + 1, pairs.size() * 4, cudaMemcpyDeviceToHost)) != cudaSuccess ||
+        (e = cudaMemcpy(hc.data(), cen, hc.size() * 8, cudaMemcpyDeviceToHost)) != cudaSuccess)
+        return done(fail(h, CCB_ECUDA, "borderline pairs: %s", cudaGetErrorString(e)));
+    typedef double (*nrm2_fn)(int *, double *, int *);
+    for (int i = 0; i < nb; ++i) {
+        const int p_ = pairs[2 * i], q_ = pairs[2 * i + 1];
+        for (int d = 0; d < D; ++d) x[d] = hc[(size_t)q_ * D + d] - hc[(size_t)p_ * D + d];
+        int n = D, inc = 1;
+        const double r = dnrm2 ? ((nrm2_fn)dnrm2)(&n, x.data(), &inc) : builtin_nrm2(x.data(), D);
+        dec[i] = r <= E;
+    }
+    uint8_t *ddec = reinterpret_cast<uint8_t *>(buf + 1 + 2 * (size_t)nb);
+    if ((e = cudaMemcpyAsync(ddec, dec.data(), nb, cudaMemcpyHostToDevice, s)) != cudaSuccess)
+        return done(fail(h, CCB_ECUDA, "borderline decisions: %s", cudaGetErrorString(e)));
+    k_off_patch<<<(nb + 127) / 128, 128, 0, s>>>(nbr, cnt, buf + 1, ddec, nb, r0, (M + 31) / 32);
+    if ((rc = launched(h, "k_off_patch"))) return done(rc);
+    if (h) h->st.kernel_launches++;
+    cudaFreeAsync(buf, s);
+    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) // dec (host) is read by the copy above
+        return fail(h, CCB_ECUDA, "k_off_patch: %s", cudaGetErrorString(e));
     return CCB_OK;
+}
+
+int launch_off_subspace(ccb_handle *h, cudaStream_t s, const double *cen, int M, int D, int r0, int r1, const uint32_t *nbr,
+                        const int32_t *cnt, double delta, uint64_t *submask) {
+    if (r1 == r0) return CCB_OK;
+    if (cudaMemsetAsync(submask, 0, (size_t)(r1 - r0) * 8, s) != cudaSuccess)
+        return fail(h, CCB_ECUDA, "k_off_subspace: clearing the masks failed");
+    const int64_t t = (int64_t)(r1 - r0) * D;
+    k_off_subspace<<<(unsigned)((t + 127) / 128), 128, 0, s>>>(cen, M, D, r0, r1, nbr, cnt, delta, submask);
+    return launched(h, "k_off_subspace");
+}
+
+int launch_off_weighted(ccb_handle *h, cudaStream_t s, const double *cen, int M, int D, int r0, int r1, const uint32_t *nbr,
+                        const uint64_t *submask_all, double k, double E2, uint32_t *wnbr) {
+    if (r1 == r0) return CCB_OK;
+    k_off_weighted<<<(unsigned)((r1 - r0 + 3) / 4), OFFW_THREADS, 0, s>>>(cen, M, D, r0, r1, nbr, submask_all, k, E2, wnbr);
+    return launched(h, "k_off_weighted");
+}
+
+int launch_offc_rowinfo(ccb_handle *h, cudaStream_t s, const uint32_t *wnbr, int M, int r0, int r1, uint8_t *iso,
+                        int32_t *nnz) {
+    if (r1 > r0) k_offc_rowinfo<<<(unsigned)((r1 - r0 + 3) / 4), 128, 0, s>>>(wnbr, r0, r1, (M + 31) / 32, iso, nnz);
+    return launched(h, "k_offc_rowinfo");
+}
+
+// iso / off: of all M rows (global CSR)
+int launch_offc_fill(ccb_handle *h, cudaStream_t s, const uint32_t *wnbr, int M, int r0, int r1, const uint8_t *iso,
+                     const int64_t *off, int32_t *col) {
+    if (r1 > r0) k_offc_fill<<<(unsigned)((r1 - r0 + 3) / 4), 128, 0, s>>>(wnbr, r0, r1, (M + 31) / 32, iso, off, col);
+    return launched(h, "k_offc_fill");
 }
 
 // The stateless entry points take their scratch from the device's stream-ordered pool; raise its release threshold once
@@ -937,62 +1022,75 @@ void offc_grow_and_merge(cudaStream_t s, int M, const int64_t *off, const int32_
     k_offc_scatter_serial<<<148, 256, 0, s>>>(seed_of, cl_off_s, n_cl_s, order_s, rank, cl_off, order, label);
 }
 
+// off[M] -- the CSR size, the last entry of the exclusive prefix of the row lengths -- read back to the host
+int csr_total(ccb_handle *h, cudaStream_t s, const int64_t *off, int M, int64_t *total) {
+    cudaError_t e;
+    if ((e = cudaMemcpyAsync(total, off + M, 8, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
+        (e = cudaStreamSynchronize(s)) != cudaSuccess)
+        return fail(h, CCB_ECUDA, "offline CSR size: %s", cudaGetErrorString(e));
+    return CCB_OK;
+}
+
+// offc_grow_and_merge over a CSR of `total` entries (iso / off / col of all M rows), its scratch from the stream-ordered pool
+int off_clusters_csr(ccb_handle *h, cudaStream_t s, int M, const int64_t *off, const int32_t *col, int64_t total,
+                     const uint8_t *iso, const uint8_t *core, const uint64_t *submask, int cnt_gt1, int64_t pi,
+                     int32_t *label, int32_t *order, int32_t *cl_off, int32_t *n_cl) {
+    // int32 scratch of offc_grow_and_merge (7 M + 16) | queue (2 M + 2) | cls (M bytes)
+    const size_t m = (size_t)M;
+    int32_t *i32 = nullptr;
+    cudaError_t e;
+    if ((e = cudaMallocAsync(&i32, (9 * m + 18) * 4 + m, s)) != cudaSuccess)
+        return fail(h, CCB_ENOMEM, "offline scratch: %s", cudaGetErrorString(e));
+    int32_t *queue = i32 + 7 * m + 16;
+    uint8_t *cls = reinterpret_cast<uint8_t *>(queue + 2 * m + 2);
+    cudaMemsetAsync(cls, 0, m, s);
+    offc_grow_and_merge(s, M, off, col, core, iso, submask, cnt_gt1, pi, cls, queue, i32, label, order, cl_off, n_cl, total);
+    const int rc = launched(h, "offline cluster growth");
+    cudaFreeAsync(i32, s);
+    return rc;
+}
+
+// cls [M] and queue [2 M + 2]: scratch of the bit-row scan
 int launch_off_clusters(ccb_handle *h, cudaStream_t s, int M, const uint32_t *wnbr, const uint8_t *core,
                         const uint64_t *submask, int cnt_gt1, int64_t pi, uint8_t *cls, int32_t *queue, int32_t *label,
                         int32_t *order, int32_t *cl_off, int32_t *n_cl, int *launches, int csr_min_m) {
-    const int words = (M + 31) / 32;
     *launches = 0;
-    cudaMemsetAsync(cls, 0, (size_t)std::max(M, 1), s);
-    auto old_path = [&]() {
+    auto bit_rows = [&]() {
+        cudaMemsetAsync(cls, 0, (size_t)std::max(M, 1), s);
         k_off_clusters<<<1, OFFC_THREADS, 0, s>>>(M, wnbr, core, submask, cnt_gt1, pi, cls, queue, label, order, cl_off, n_cl);
         *launches += 1;
-        cudaError_t e = cudaGetLastError();
-        return e == cudaSuccess ? CCB_OK : fail(h, CCB_ECUDA, "k_off_clusters: %s", cudaGetErrorString(e));
+        return launched(h, "k_off_clusters");
     };
-    if (M < (csr_min_m > 0 ? csr_min_m : OFF_CSR_MIN_M) || M == 0) return old_path();
-    uint8_t *iso = nullptr;
-    int32_t *i32 = nullptr, *col = nullptr;
-    int64_t *off = nullptr;
-    // int32 scratch: nnz | order_s | cl_off_s (M + 1) | seed_of (M + 1) | n_cl_s (1) | seedflag | size_by_node |
-    //                rank (M + 1) | size_by_cluster
+    if (M < (csr_min_m > 0 ? csr_min_m : OFF_CSR_MIN_M) || M == 0) return bit_rows();
+    // off (M + 1) | nnz (M int32) | iso (M bytes)
     const size_t m = (size_t)M;
-    const size_t n32 = 8 * m + 16;
+    int64_t *off = nullptr;
+    int32_t *col = nullptr;
     cudaError_t e;
-    if ((e = cudaMallocAsync(&iso, m, s)) != cudaSuccess || (e = cudaMallocAsync(&i32, n32 * 4, s)) != cudaSuccess ||
-        (e = cudaMallocAsync(&off, (m + 1) * 8, s)) != cudaSuccess)
+    if ((e = cudaMallocAsync(&off, (m + 1) * 8 + m * 5, s)) != cudaSuccess)
         return fail(h, CCB_ENOMEM, "offline scratch: %s", cudaGetErrorString(e));
-    int32_t *nnz = i32; // the remaining 7 m + 16 entries are the scratch of offc_grow_and_merge
-    auto release = [&]() {
-        cudaFreeAsync(iso, s);
-        cudaFreeAsync(i32, s);
+    int32_t *nnz = reinterpret_cast<int32_t *>(off + m + 1);
+    uint8_t *iso = reinterpret_cast<uint8_t *>(nnz + m);
+    auto done = [&](int r) {
         cudaFreeAsync(off, s);
         if (col) cudaFreeAsync(col, s);
+        return r;
     };
-    const int wgrid = (M + 3) / 4;
-    k_offc_rowinfo<<<wgrid, 128, 0, s>>>(wnbr, 0, M, words, iso, nnz);
+    int rc;
+    int64_t total = 0;
+    if ((rc = launch_offc_rowinfo(h, s, wnbr, M, 0, M, iso, nnz))) return done(rc);
     k_offc_scan<int64_t><<<1, OFFG_THREADS, 0, s>>>(nnz, M, off);
     *launches += 2;
-    int64_t total = 0;
-    if ((e = cudaMemcpyAsync(&total, off + M, 8, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
-        (e = cudaStreamSynchronize(s)) != cudaSuccess) {
-        release();
-        return fail(h, CCB_ECUDA, "offline CSR sizes: %s", cudaGetErrorString(e));
-    }
-    if (total > (int64_t)INT32_MAX - 1) { // a CSR that large buys nothing over the bit rows
-        release();
-        return old_path();
-    }
-    if ((e = cudaMallocAsync(&col, (size_t)std::max<int64_t>(total, 1) * 4, s)) != cudaSuccess) {
-        release();
-        return fail(h, CCB_ENOMEM, "offline CSR (%lld entries): %s", (long long)total, cudaGetErrorString(e));
-    }
-    k_offc_fill<<<wgrid, 128, 0, s>>>(wnbr, 0, M, words, iso, off, col);
+    if ((rc = csr_total(h, s, off, M, &total))) return done(rc);
+    if (total > (int64_t)INT32_MAX - 1) // a CSR that large buys nothing over the bit rows
+        return done(bit_rows());
+    if ((e = cudaMallocAsync(&col, (size_t)std::max<int64_t>(total, 1) * 4, s)) != cudaSuccess)
+        return done(fail(h, CCB_ENOMEM, "offline CSR (%lld entries): %s", (long long)total, cudaGetErrorString(e)));
+    if ((rc = launch_offc_fill(h, s, wnbr, M, 0, M, iso, off, col))) return done(rc);
     *launches += 1;
-    offc_grow_and_merge(s, M, off, col, core, iso, submask, cnt_gt1, pi, cls, queue, i32 + m, label, order, cl_off, n_cl, total);
+    rc = off_clusters_csr(h, s, M, off, col, total, iso, core, submask, cnt_gt1, pi, label, order, cl_off, n_cl);
     *launches += 8;
-    e = cudaGetLastError();
-    release();
-    return e == cudaSuccess ? CCB_OK : fail(h, CCB_ECUDA, "offline cluster growth: %s", cudaGetErrorString(e));
+    return done(rc);
 }
 
 // Probes of the pcore replay pattern (mode 3 of ccb_fp64_peak): one warp runs the CLEAN-stage schedule of k_bs_chain_p over
@@ -1664,9 +1762,8 @@ int ccb_offline(ccb_handle *h, int64_t *n_clusters) {
     Timed tm_off(h, CCB_CAT_OFFLINE);
     uint8_t *core, *cls;
     uint32_t *nbr, *wnbr;
-    int32_t *cnt, *border, *nborder, *queue, *label, *order, *cloff, *ncl;
+    int32_t *cnt, *queue, *label, *order, *cloff, *ncl;
     uint64_t *submask;
-    int border_cap = (int)std::max<size_t>(h->ob[ccb_handle::OB_BORDER].bytes / 8, (size_t)1 << 16);
 #define OBUF(var, which, n)                                                      \
     if ((rc = off_buf(h, ccb_handle::which, (size_t)(n) * sizeof(*var)))) return rc; \
     var = (decltype(var))h->ob[ccb_handle::which].p
@@ -1675,73 +1772,28 @@ int ccb_offline(ccb_handle *h, int64_t *n_clusters) {
     OBUF(nbr, OB_NBR, (size_t)M * words);
     OBUF(wnbr, OB_WNBR, (size_t)M * words);
     OBUF(cnt, OB_CNT, M);
-    OBUF(border, OB_BORDER, 2 * (size_t)border_cap);
-    OBUF(nborder, OB_NBORDER, 1);
     OBUF(queue, OB_QUEUE, 2 * (size_t)M + 2);
     OBUF(label, OB_LABEL, M);
     OBUF(order, OB_ORDER, M);
     OBUF(cloff, OB_CLOFF, (size_t)M + 2);
     OBUF(ncl, OB_NCL, 1);
     OBUF(submask, OB_SUBMASK, M);
-    CK(h, cudaMemsetAsync(submask, 0, (size_t)M * 8, s));
-    CK(h, cudaMemsetAsync(cls, 0, (size_t)M, s));
 
     k_off_core<<<(M + 127) / 128, 128, 0, s>>>(P.cf1, P.cf2, P.w, P.mask, M, D, h->prm.k, h->wsel, h->div_mode, h->cnt_gt1,
                                                h->prm.eps2, h->mu, h->pi, core);
     CKL(h);
     h->st.kernel_launches++;
-    int32_t nb = 0;
-    for (;;) { // the borderline list grows to whatever the data needs (e.g. many coincident centroids with upsilon = 0)
-        CK(h, cudaMemsetAsync(nborder, 0, 4, s));
-        if ((rc = launch_off_neighbours(h, s, P.cen, M, D, 0, M, E2, nbr, cnt, border, border_cap, nborder))) return rc;
-        h->st.kernel_launches++;
-        CK(h, cudaMemcpyAsync(&nb, nborder, 4, cudaMemcpyDeviceToHost, s));
-        CK(h, cudaStreamSynchronize(s));
-        if (nb <= border_cap) break;
-        border_cap = nb;
-        OBUF(border, OB_BORDER, 2 * (size_t)border_cap);
-    }
-    if (nb > 0) {
-        // settle the pairs inside the guard band with the BLAS dnrm2 the reference itself calls
-        std::vector<int32_t> pairs(2 * (size_t)nb);
-        std::vector<double> hc((size_t)M * D), x(D);
-        std::vector<uint8_t> dec(nb);
-        CK(h, cudaMemcpy(pairs.data(), border, pairs.size() * 4, cudaMemcpyDeviceToHost));
-        CK(h, cudaMemcpy(hc.data(), P.cen, hc.size() * 8, cudaMemcpyDeviceToHost));
-        typedef double (*nrm2_fn)(int *, double *, int *);
-        for (int i = 0; i < nb; ++i) {
-            const int p_ = pairs[2 * i], q_ = pairs[2 * i + 1];
-            for (int d = 0; d < D; ++d) x[d] = hc[(size_t)q_ * D + d] - hc[(size_t)p_ * D + d];
-            double r;
-            if (h->dnrm2) {
-                int n = D, inc = 1;
-                r = ((nrm2_fn)h->dnrm2)(&n, x.data(), &inc);
-            } else {
-                r = builtin_nrm2(x.data(), D);
-            }
-            dec[i] = r <= h->prm.upsilon_eps;
-        }
-        uint8_t *ddec;
-        OBUF(ddec, OB_DEC, nb);
-        CK(h, cudaMemcpyAsync(ddec, dec.data(), nb, cudaMemcpyHostToDevice, s));
-        k_off_patch<<<(nb + 127) / 128, 128, 0, s>>>(nbr, cnt, border, ddec, nb, 0, words);
-        CKL(h);
-        CK(h, cudaStreamSynchronize(s)); // dec (host) is read by the copy above
-        h->st.borderline_pairs += nb;
-        h->st.kernel_launches++;
-    }
-    {
-        const int64_t t = (int64_t)M * D;
-        k_off_subspace<<<(unsigned)((t + 127) / 128), 128, 0, s>>>(P.cen, M, D, 0, M, nbr, cnt, h->prm.delta, submask);
-        CKL(h);
-        k_off_weighted<<<(unsigned)((M + 3) / 4), OFFW_THREADS, 0, s>>>(P.cen, M, D, 0, M, nbr, submask, h->prm.k, E2, wnbr);
-        CKL(h);
-        int nl = 0, rc2;
-        if ((rc2 = launch_off_clusters(h, s, M, wnbr, core, submask, h->cnt_gt1, h->pi, cls, queue, label, order, cloff, ncl, &nl,
-                                       h->off_csr_min_m)))
-            return rc2;
-        h->st.kernel_launches += 2 + nl;
-    }
+    int64_t nb = 0;
+    int nl = 0;
+    if ((rc = off_neighbours_settled(h, s, P.cen, M, D, 0, M, h->prm.upsilon_eps, E2, h->dnrm2, nbr, cnt, &nb)))
+        return rc;
+    h->st.borderline_pairs += nb;
+    if ((rc = launch_off_subspace(h, s, P.cen, M, D, 0, M, nbr, cnt, h->prm.delta, submask)) ||
+        (rc = launch_off_weighted(h, s, P.cen, M, D, 0, M, nbr, submask, h->prm.k, E2, wnbr)) ||
+        (rc = launch_off_clusters(h, s, M, wnbr, core, submask, h->cnt_gt1, h->pi, cls, queue, label, order, cloff, ncl, &nl,
+                                  h->off_csr_min_m)))
+        return rc;
+    h->st.kernel_launches += 2 + nl;
     int32_t nc_raw = 0;
     CK(h, cudaMemcpyAsync(&nc_raw, ncl, 4, cudaMemcpyDeviceToHost, s));
     CK(h, cudaStreamSynchronize(s));
@@ -2043,23 +2095,14 @@ int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, 
 }
 
 int ccb_off_neighbours(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
-                       double E2, uint32_t *nbr, int32_t *cnt, int32_t *border, int32_t border_cap, int32_t *n_border) {
-    if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
+                       double E, double E2, void *dnrm2, uint32_t *nbr, int32_t *cnt, int64_t *n_border) {
+    if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M || !n_border)
+        return fail(nullptr, CCB_EINVAL, "bad arguments");
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    return launch_off_neighbours(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, E2, nbr, cnt, border,
-                                 border_cap, n_border);
-}
-
-int ccb_off_patch(int32_t device, void *stream, uint32_t *nbr, int32_t *cnt, const int32_t *pairs, const uint8_t *decision,
-                  int32_t n, int64_t r0, int64_t M) {
-    if (n < 0 || M < 0) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    if (n == 0) return CCB_OK;
-    k_off_patch<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(nbr, cnt, pairs, decision, n, (int)r0, (int)((M + 31) / 32));
-    e = cudaGetLastError();
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_off_patch: %s", cudaGetErrorString(e));
+    tune_pool(device);
+    return off_neighbours_settled(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, E, E2, dnrm2, nbr, cnt,
+                                  n_border);
 }
 
 int ccb_off_subspace(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
@@ -2067,13 +2110,7 @@ int ccb_off_subspace(int32_t device, void *stream, const double *cen, int64_t M,
     if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    cudaStream_t s = (cudaStream_t)stream;
-    if (r1 == r0) return CCB_OK;
-    cudaMemsetAsync(submask, 0, (size_t)(r1 - r0) * 8, s);
-    const int64_t t = (r1 - r0) * D;
-    k_off_subspace<<<(unsigned)((t + 127) / 128), 128, 0, s>>>(cen, (int)M, D, (int)r0, (int)r1, nbr, cnt, delta, submask);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_off_subspace: %s", cudaGetErrorString(e));
+    return launch_off_subspace(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, nbr, cnt, delta, submask);
 }
 
 int ccb_off_weighted(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
@@ -2081,11 +2118,7 @@ int ccb_off_weighted(int32_t device, void *stream, const double *cen, int64_t M,
     if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    if (r1 == r0) return CCB_OK;
-    k_off_weighted<<<(unsigned)((r1 - r0 + 3) / 4), OFFW_THREADS, 0, (cudaStream_t)stream>>>(cen, (int)M, D, (int)r0, (int)r1, nbr,
-                                                                                             submask_all, k, E2, wnbr);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_off_weighted: %s", cudaGetErrorString(e));
+    return launch_off_weighted(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, nbr, submask_all, k, E2, wnbr);
 }
 
 int ccb_off_clusters(int32_t device, void *stream, int64_t M, const uint32_t *wnbr, const uint8_t *core,
@@ -2114,11 +2147,7 @@ int ccb_offc_rowinfo(int32_t device, void *stream, const uint32_t *wnbr_rows, in
     if (M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    if (r1 > r0)
-        k_offc_rowinfo<<<(unsigned)((r1 - r0 + 3) / 4), 128, 0, (cudaStream_t)stream>>>(wnbr_rows, (int)r0, (int)r1,
-                                                                                       (int)((M + 31) / 32), iso, nnz);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_offc_rowinfo: %s", cudaGetErrorString(e));
+    return launch_offc_rowinfo(nullptr, (cudaStream_t)stream, wnbr_rows, (int)M, (int)r0, (int)r1, iso, nnz);
 }
 
 int ccb_offc_fill(int32_t device, void *stream, const uint32_t *wnbr_rows, int64_t M, int64_t r0, int64_t r1,
@@ -2126,11 +2155,7 @@ int ccb_offc_fill(int32_t device, void *stream, const uint32_t *wnbr_rows, int64
     if (M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    if (r1 > r0)
-        k_offc_fill<<<(unsigned)((r1 - r0 + 3) / 4), 128, 0, (cudaStream_t)stream>>>(wnbr_rows, (int)r0, (int)r1,
-                                                                                    (int)((M + 31) / 32), iso_all, off_all, col);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_offc_fill: %s", cudaGetErrorString(e));
+    return launch_offc_fill(nullptr, (cudaStream_t)stream, wnbr_rows, (int)M, (int)r0, (int)r1, iso_all, off_all, col);
 }
 
 int ccb_off_clusters_csr(int32_t device, void *stream, int64_t M, const int64_t *off, const int32_t *col, const uint8_t *iso,
@@ -2146,23 +2171,11 @@ int ccb_off_clusters_csr(int32_t device, void *stream, int64_t M, const int64_t 
         cudaMemsetAsync(cl_off, 0, 4, s);
         return CCB_OK;
     }
-    uint8_t *cls = nullptr;
-    int32_t *queue = nullptr, *i32 = nullptr;
-    const size_t m = (size_t)M;
-    if ((e = cudaMallocAsync(&cls, m, s)) != cudaSuccess || (e = cudaMallocAsync(&queue, (2 * m + 2) * 4, s)) != cudaSuccess ||
-        (e = cudaMallocAsync(&i32, (7 * m + 16) * 4, s)) != cudaSuccess)
-        return fail(nullptr, CCB_ENOMEM, "scratch allocation: %s", cudaGetErrorString(e));
-    cudaMemsetAsync(cls, 0, m, s);
-    int64_t total = -1; // list lengths decide between the one-warp and the 1024-thread walk
-    if (cudaMemcpyAsync(&total, off + M, 8, cudaMemcpyDeviceToHost, s) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess)
-        total = -1;
-    offc_grow_and_merge(s, (int)M, off, col, core, iso, submask_all, k > 1.0, pi, cls, queue, i32, label, order, cl_off, n_cl,
-                        total);
-    e = cudaGetLastError();
-    cudaFreeAsync(cls, s);
-    cudaFreeAsync(queue, s);
-    cudaFreeAsync(i32, s);
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "offline cluster growth (CSR): %s", cudaGetErrorString(e));
+    int64_t total = 0; // list lengths decide between the walks
+    const int rc = csr_total(nullptr, s, off, (int)M, &total);
+    return rc ? rc
+              : off_clusters_csr(nullptr, s, (int)M, off, col, total, iso, core, submask_all, k > 1.0, pi, label, order, cl_off,
+                                 n_cl);
 }
 
 } // extern "C"

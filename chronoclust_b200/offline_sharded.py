@@ -3,8 +3,8 @@
 BASELINE.json config 4: M pcore MCs x D dims, the pairwise eps-neighbourhood (predecon.py:161-188) is the
 O(M^2 D) part.  Rank g owns the contiguous rows [g*R, (g+1)*R), R = ceil(M/G):
 
-  stage 1 (local)   N(p) bit rows + |N(p)| for own rows            ccb_off_neighbours  (kernel 4b)
-                    borderline pairs settled on the host via dnrm2, patched back    ccb_off_patch
+  stage 1 (local)   N(p) bit rows + |N(p)| for own rows, the pairs  ccb_off_neighbours  (kernel 4b)
+                    inside the guard band settled with dnrm2
   stage 2 (local)   subspace preference masks w_p of own rows       ccb_off_subspace    (kernel 4c)
   all-gather        w_p masks of every row (M * 8 B)                NCCL all_gather_into_tensor
   stage 3 (local)   weighted-neighbour bit rows WN(p) of own rows   ccb_off_weighted    (kernel 4d)
@@ -22,8 +22,6 @@ communicator); every stage is a kernel of this repo.
 The compute backend is injectable so that the sharding / gather logic is testable on CPU with gloo.
 """
 import ctypes as C
-
-import numpy as np
 
 from . import _lib
 
@@ -47,36 +45,10 @@ class CudaStages:
         return self.torch.zeros(shape, dtype=dtype, device=self.dev)
 
     def neighbours(self, cen, M, D, r0, r1, E, E2, nbr, cnt):
-        t = self.torch
-        cap = 1 << 16
-        while True:  # the borderline list grows to whatever the data needs (e.g. many coincident centroids)
-            border = t.zeros(2 * cap, dtype=t.int32, device=self.dev)
-            nb = t.zeros(1, dtype=t.int32, device=self.dev)
-            _lib.check(self.L.ccb_off_neighbours(self.device, self.stream(), cen.data_ptr(), M, D, r0, r1, E2,
-                                                 nbr.data_ptr(), cnt.data_ptr(), border.data_ptr(), cap, nb.data_ptr()))
-            n = int(nb.item())
-            if n <= cap:
-                break
-            cap = n
-        if n:
-            pairs = border[:2 * n].cpu().numpy().reshape(n, 2)
-            hc = cen.cpu().numpy()
-            dec = np.zeros(n, np.uint8)
-            fn = None
-            if self.dnrm2_ptr:
-                fn = C.CFUNCTYPE(C.c_double, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_int))(self.dnrm2_ptr)
-            for i, (p, q) in enumerate(pairs):
-                x = np.ascontiguousarray(hc[q] - hc[p])
-                if fn is not None:
-                    nn, inc = C.c_int(D), C.c_int(1)
-                    r = fn(C.byref(nn), x.ctypes.data_as(C.POINTER(C.c_double)), C.byref(inc))
-                else:
-                    r = float(np.sqrt(np.sum(x.astype(np.longdouble) ** 2)))
-                dec[i] = r <= E
-            ddec = t.from_numpy(dec).to(self.dev)
-            _lib.check(self.L.ccb_off_patch(self.device, self.stream(), nbr.data_ptr(), cnt.data_ptr(), border.data_ptr(),
-                                            ddec.data_ptr(), n, r0, M))
-        return n
+        n = C.c_int64()
+        _lib.check(self.L.ccb_off_neighbours(self.device, self.stream(), cen.data_ptr(), M, D, r0, r1, E, E2,
+                                             self.dnrm2_ptr, nbr.data_ptr(), cnt.data_ptr(), C.byref(n)))
+        return n.value
 
     def subspace(self, cen, M, D, r0, r1, nbr, cnt, delta, submask):
         _lib.check(self.L.ccb_off_subspace(self.device, self.stream(), cen.data_ptr(), M, D, r0, r1, nbr.data_ptr(),
@@ -86,18 +58,21 @@ class CudaStages:
         _lib.check(self.L.ccb_off_weighted(self.device, self.stream(), cen.data_ptr(), M, D, r0, r1, nbr.data_ptr(),
                                            submask_all.data_ptr(), k, E2, wnbr.data_ptr()))
 
-    def clusters(self, M, wnbr_all, core, submask_all, k, pi, csr_min_m=0):
+    def _grow(self, M, call):
+        """label / order / cl_off / n_cl of the cluster growth `call(label, order, cl_off, n_cl)`, read back"""
         t = self.torch
         label = t.empty(max(M, 1), dtype=t.int32, device=self.dev)
         order = t.empty(max(M, 1), dtype=t.int32, device=self.dev)
         cl_off = t.zeros(M + 2, dtype=t.int32, device=self.dev)
         ncl = t.zeros(1, dtype=t.int32, device=self.dev)
-        _lib.check(self.L.ccb_off_clusters(self.device, self.stream(), M, wnbr_all.data_ptr(), core.data_ptr(),
-                                           submask_all.data_ptr(), k, pi, csr_min_m, label.data_ptr(), order.data_ptr(),
-                                           cl_off.data_ptr(), ncl.data_ptr()))
+        _lib.check(call(label.data_ptr(), order.data_ptr(), cl_off.data_ptr(), ncl.data_ptr()))
         n = int(ncl.item())
         return label[:M].cpu().numpy(), order.cpu().numpy(), cl_off[:n + 1].cpu().numpy(), n
 
+    def clusters(self, M, wnbr_all, core, submask_all, k, pi, csr_min_m=0):
+        return self._grow(M, lambda *out: self.L.ccb_off_clusters(
+            self.device, self.stream(), M, wnbr_all.data_ptr(), core.data_ptr(), submask_all.data_ptr(), k, pi, csr_min_m,
+            *out))
 
     def rowinfo(self, wn_rows, M, r0, r1, iso, nnz):
         _lib.check(self.L.ccb_offc_rowinfo(self.device, self.stream(), wn_rows.data_ptr(), M, r0, r1, iso.data_ptr(),
@@ -108,16 +83,9 @@ class CudaStages:
                                         off_all.data_ptr(), col.data_ptr()))
 
     def clusters_csr(self, M, off_all, col, iso_all, core, submask_all, k, pi):
-        t = self.torch
-        label = t.empty(max(M, 1), dtype=t.int32, device=self.dev)
-        order = t.empty(max(M, 1), dtype=t.int32, device=self.dev)
-        cl_off = t.zeros(M + 2, dtype=t.int32, device=self.dev)
-        ncl = t.zeros(1, dtype=t.int32, device=self.dev)
-        _lib.check(self.L.ccb_off_clusters_csr(self.device, self.stream(), M, off_all.data_ptr(), col.data_ptr(),
-                                               iso_all.data_ptr(), core.data_ptr(), submask_all.data_ptr(), k, pi,
-                                               label.data_ptr(), order.data_ptr(), cl_off.data_ptr(), ncl.data_ptr()))
-        n = int(ncl.item())
-        return label[:M].cpu().numpy(), order.cpu().numpy(), cl_off[:n + 1].cpu().numpy(), n
+        return self._grow(M, lambda *out: self.L.ccb_off_clusters_csr(
+            self.device, self.stream(), M, off_all.data_ptr(), col.data_ptr(), iso_all.data_ptr(), core.data_ptr(),
+            submask_all.data_ptr(), k, pi, *out))
 
 
 def row_range(M, world, rank):

@@ -217,15 +217,12 @@ int ccb_fp64_peak(int32_t device, void *stream, int32_t mode, int32_t iters, int
                   double *flops_out);
 
 /* Offline stage 1 for rows [r0, r1) of M pcore MCs: neighbourhood bit rows nbr [(r1-r0)][words]
- * (words = ceil(M/32), uint32), neighbour counts cnt [(r1-r0)], and the list of borderline pairs
- * (row, col) whose squared distance is within the guard band of E2 (border [2*border_cap] int32,
- * n_border [1] int32, counted even beyond border_cap). */
+ * (words = ceil(M/32), uint32) and neighbour counts cnt [(r1-r0)] of the test dnrm2(c_q - c_p) <= E.  The device decides
+ * every pair whose squared distance is outside a guard band around E2 = E^2; the pairs inside it are settled on the host
+ * with dnrm2 (as for ccb_set_dnrm2; NULL = the built-in restatement).  *n_border (host) = the number of such pairs.
+ * Synchronises the stream. */
 int ccb_off_neighbours(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
-                       double E2, uint32_t *nbr, int32_t *cnt, int32_t *border, int32_t border_cap, int32_t *n_border);
-/* Settles borderline pairs on the device after the host decided them with dnrm2: pairs [2*n] (row, col) as
- * reported by ccb_off_neighbours, decision [n] (1 = neighbour). */
-int ccb_off_patch(int32_t device, void *stream, uint32_t *nbr, int32_t *cnt, const int32_t *pairs, const uint8_t *decision,
-                  int32_t n, int64_t r0, int64_t M);
+                       double E, double E2, void *dnrm2, uint32_t *nbr, int32_t *cnt, int64_t *n_border);
 /* Offline stage 2: subspace preference masks submask [(r1-r0)] from the neighbour rows (delta, not delta^2). */
 int ccb_off_subspace(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
                      const uint32_t *nbr, const int32_t *cnt, double delta, uint64_t *submask);

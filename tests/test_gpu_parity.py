@@ -374,7 +374,11 @@ def test_stateless_offline_stages_match_handle_path():
 
 def test_offline_borderline_pairs_resolved_by_dnrm2():
     """Centroids placed exactly on the eps-boundary (3-4-5 triangles): the device must flag them and the
-    host must settle them with dnrm2 (<= E is inclusive)."""
+    host must settle them with dnrm2 (<= E is inclusive) -- in the handle's offline phase and in the stateless
+    row-sharded stage, with the scipy dnrm2 and with the built-in one, over all rows and over two row halves."""
+    import torch
+
+    from chronoclust_b200.offline_sharded import CudaStages
     cfg = {"beta": 0.0, "delta": 0.5, "epsilon": 1.0, "lambda": 0, "k": 4.0, "mu": 0.0, "pi": 0, "omicron": 0.0,
            "upsilon": 5.0}
     h = make(cfg)
@@ -392,25 +396,29 @@ def test_offline_borderline_pairs_resolved_by_dnrm2():
     assert h.stats()["borderline_pairs"] >= 2
     assert nbr[0, 1] == 1 and nbr[1, 0] == 1 and nbr[1, 2] == 1  # distance exactly E is a neighbour
     assert nbr[0, 2] == 0 and nbr[0, 3] == 0  # 10 > 5; 5.000000000000003 > 5
+    tc = torch.from_numpy(cen).cuda()
+    E = h.upsilon
+    for st in (CudaStages(0, dnrm2_ptr=None), CudaStages(0, dnrm2_ptr=_lib.scipy_dnrm2_pointer())):
+        for r0, r1 in ((0, M), (0, 2), (2, M)):
+            rows = st.empty((r1 - r0, 1), torch.int32)
+            cnt = st.empty((r1 - r0,), torch.int32)
+            n = st.neighbours(tc, M, D, r0, r1, E, E ** 2, rows, cnt)
+            got = np.unpackbits(rows.cpu().numpy().view(np.uint8), axis=1, bitorder="little")[:, :M]
+            assert n >= 1, (st.dnrm2_ptr, r0, r1)
+            assert (got == nbr[r0:r1]).all(), (st.dnrm2_ptr, r0, r1, got)
+            assert (cnt.cpu().numpy() == nbr[r0:r1].sum(axis=1)).all(), (st.dnrm2_ptr, r0, r1)
 
 
-def test_cluster_growth_formulations_agree():
-    """Kernel 4e has two formulations (bit-row scan; isolated pre-pass + CSR + merge by seed rank).  On a random
-    symmetric weighted-neighbourhood graph with isolated MCs, noise, border MCs shared between clusters and core MCs
-    whose pdim exceeds pi (relay but are never claimed), both must give the same labels, claim order and offsets."""
-    import torch
-    from chronoclust_b200 import _lib
-    from chronoclust_b200.offline_sharded import CudaStages
-
-    rng = np.random.default_rng(11)
-    M, D = 3000, 12
+def _growth_graph(rng, M, D, ngroups, p_edge, p_iso):
+    """A random symmetric weighted-neighbourhood graph with isolated MCs, noise, border MCs shared between clusters and
+    core MCs whose pdim exceeds pi: (bit rows, core flags, subspace masks, CSR entries of the non-isolated rows)."""
     words = (M + 31) // 32
-    grp = rng.integers(0, 60, size=M)
-    grp[rng.random(M) < 0.3] = -1  # isolated
+    grp = rng.integers(0, ngroups, size=M)
+    grp[rng.random(M) < p_iso] = -1  # isolated
     A = np.zeros((M, M), bool)
-    for g in range(60):
+    for g in range(ngroups):
         idx = np.flatnonzero(grp == g)
-        sub = rng.random((len(idx), len(idx))) < 0.08
+        sub = rng.random((len(idx), len(idx))) < p_edge
         A[np.ix_(idx, idx)] = sub | sub.T
     bridges = rng.integers(0, M, size=(40, 2))  # a few edges between groups (border MCs reachable from two clusters)
     bridges = bridges[(grp[bridges[:, 0]] >= 0) & (grp[bridges[:, 1]] >= 0)]
@@ -422,19 +430,42 @@ def test_cluster_growth_formulations_agree():
     core = (rng.random(M) < 0.6).astype(np.uint8)
     pd = rng.integers(0, D + 1, size=M)
     sub = np.array([sum(1 << int(d) for d in rng.choice(D, size=int(k), replace=False)) for k in pd], np.int64)
-    pi = 8
+    deg = A.sum(axis=1)
+    nnz = int(deg[deg > 1].sum())  # an isolated row (WN(p) = {p}) owns no CSR entry
+    return wn, core, sub, nnz
+
+
+def test_cluster_growth_formulations_agree():
+    """Kernel 4e has two formulations (bit-row scan; isolated pre-pass + CSR + merge by seed rank), and the CSR one walks
+    the graph in one of three ways by its size: one warp over a shared-memory copy (22 bytes per entry fit 200 KB), one
+    warp over global memory (mean list length <= 16), the 1024-thread walk (longer lists).  On a random graph for each
+    walk, the CSR formulation must give the bit-row scan's labels, claim order and offsets."""
+    import torch
+    from chronoclust_b200.offline_sharded import CudaStages
+
+    rng = np.random.default_rng(11)
+    D, pi = 12, 8
     st = CudaStages(0)
-    twn = torch.from_numpy(wn.view(np.int32)).cuda()
-    tcore, tsub = torch.from_numpy(core).cuda(), torch.from_numpy(sub).cuda()
-    res = []
-    for min_m in (10 ** 8, 1):
-        lab, order, cl_off, ncl = st.clusters(M, twn, tcore, tsub, 4.0, pi, csr_min_m=min_m)
-        res.append((lab.copy(), order[:cl_off[-1]].copy(), cl_off.copy(), ncl))
-    (l0, o0, c0, n0), (l1, o1, c1, n1) = res
-    assert n0 == n1 and n0 > 100
-    assert (c0 == c1).all() and (o0 == o1).all() and (l0 == l1).all()
-    sizes = np.diff(c0)
-    assert (sizes > 1).sum() > 20 and (sizes == 0).sum() > 0 and (l0 < 0).sum() > 0  # the fixture exercises every case
+    for walk, M, ngroups, p_edge, p_iso in (("warp", 3000, 60, 0.08, 0.3), ("smem", 1500, 60, 0.08, 0.3),
+                                            ("block", 2000, 20, 0.3, 0.1)):
+        wn, core, sub, nnz = _growth_graph(rng, M, D, ngroups, p_edge, p_iso)
+        regime = "block" if nnz > 16 * M else "smem" if nnz * 22 + 64 <= 200 * 1024 else "warp"
+        assert regime == walk, f"test construction: {nnz} CSR entries over {M} rows reach the {regime} walk"
+        twn = torch.from_numpy(wn.view(np.int32)).cuda()
+        tcore, tsub = torch.from_numpy(core).cuda(), torch.from_numpy(sub).cuda()
+        res = []
+        for min_m in (10 ** 8, 1):
+            lab, order, cl_off, ncl = st.clusters(M, twn, tcore, tsub, 4.0, pi, csr_min_m=min_m)
+            res.append((lab.copy(), order[:cl_off[-1]].copy(), cl_off.copy(), ncl))
+        (l0, o0, c0, n0), (l1, o1, c1, n1) = res
+        assert n0 == n1, walk
+        assert (c0 == c1).all() and (o0 == o1).all() and (l0 == l1).all(), walk
+        sizes = np.diff(c0)
+        if walk == "warp":
+            assert n0 > 100
+            assert (sizes > 1).sum() > 20 and (sizes == 0).sum() > 0 and (l0 < 0).sum() > 0  # the fixture exercises every case
+        else:
+            assert (sizes > 1).sum() > 0 and (l0 < 0).sum() > 0, walk
 
 
 @pytest.mark.parametrize("D,Q,P,k", [(3, 7, 5, 4.0), (12, 300, 257, 4.0), (40, 130, 999, 16.0), (12, 64, 100, 3.0),
