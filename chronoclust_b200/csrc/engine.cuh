@@ -1023,20 +1023,27 @@ __device__ __noinline__ bool bs_radius_test(double nv0, uint32_t rec_addr, int l
 // the tentative MC <= eps^2: absorbed), 0 (rejected) or 2 (too close to call: the caller runs bs_radius_test).
 // Multiplied through by W'^2 the test of mc_functions.py:45-56 reads  sum_d w_d (CF2'_d W' - CF1'_d^2)  <=  eps^2 W'^2
 // with w_d = 1/k where CF2'_d W' - CF1'_d^2 <= delta^2 W'^2, else 1 -- no division.  Lane d evaluates its term in fp64 (one
-// DMUL + one DFMA), scales it so that the right-hand side is at most TH = 2^25 (2^23 for D > 16), rounds it to an integer and
-// the warp adds the integers with ONE redux.sync instead of a chain of D shuffles and dependent adds.  The approximation
-// differs from the reference's rounding sequence by a few ulp of the terms; with coordinates of magnitude <= ~1e3 eps that
-// is far below one integer unit, and the decision is only taken when the sum is D + 8 units clear of the threshold and no
-// variance is within 2^-24 (relative) of delta^2; anything else -- including NaNs -- is "undecided".  The approximation
-// cannot corrupt results in any case: k_bs_verify_p recomputes every decision of the chain with the reference's exact
-// arithmetic (a wrong one would merely cost a round), and the first member of every chain always takes the exact test, so
-// every block advances.  D > 16: the integer is split into a high and a low part (two redux.sync) to keep 2^-20 units.
+// DMUL + one DFMA), scales it so that the right-hand side is at most TH = 2^25 (2^23 for DP > 16), rounds it to an integer and
+// the warp adds the integers with ONE redux.sync instead of a chain of D shuffles and dependent adds.  DP > 16: the integer
+// is split into a high and a low part (two redux.sync) to keep 2^-20 units.
+// Bound.  In these units the fast sum and the reference's r^2 W'^2 fs each differ from the exact value by at most ~6 ulp per
+// term of CF2'_d W' fs (the rounding of CF2' W' and of the fma; of CF2'/W', (CF1'/W')^2 and their difference), which sum
+// to <= 12 * 2^-53 * TH * sum_d (CF2'_d / W') / eps^2, plus the rounding of the integer (1/2 a term unsplit, 2^-21 split)
+// and ~D ulp of thr for the reference's own sum.  The decision is taken only when the sum is mg units clear of the
+// threshold, mg = (D + 8 unsplit, 0.01 split) + 2^-48 * TH * sum_d (CF2_d / W) / eps^2 from the chain's start state (the
+// tentative records of a chain stay near its centroid; the factor 32 over 2^-53 leaves 2.5x for that drift), and when no
+// variance is within 2^-24 (relative) of delta^2; anything else -- including NaNs -- is "undecided".  So the decision is
+// the reference's at any distance from the origin where the preference test itself is still resolvable (CF2 W / (delta^2
+// W^2) < ~2^27, i.e. coordinates below ~1e4 delta); far from the origin the fast test only leaves more records undecided.
+// A wrong decision could not corrupt results in any case: k_bs_verify_p recomputes every decision of the chain with the
+// reference's exact arithmetic (a wrong one would merely cost a round), and the first member of every chain always takes
+// the exact test, so every block advances.
 struct ChainFast {
     double F;    // TH / Wmax^2, Wmax = W at the start of the chain + its members + 1 (>= every W' of the chain)
     double fs;   // F / eps^2: scale of the terms
     double invk; // weight of a preferred dimension (approximate for a k that is not a power of two)
     double delta2;
-    double mg;   // D + 8 integer units: clearance a decision needs
+    double mg;   // clearance a decision needs, in integer units (see the bound above)
 };
 template <int DP, int NH>
 __device__ __forceinline__ int bs_radius_fast(double nv0, uint32_t rec_addr, int lane, int D, const ChainFast cf) {
@@ -1087,8 +1094,8 @@ __device__ __forceinline__ int bs_radius_fast(double nv0, uint32_t rec_addr, int
     if (SPLIT) {
         const int L = __reduce_add_sync(0xffffffffu, lo_sum);
         const double tot = dadd((double)S, dmul((double)L, 0x1p-20));
-        if (tot < dsub(thr, 0.01)) return 1;
-        if (tot > dadd(thr, 0.01)) return 0;
+        if (tot < dsub(thr, cf.mg)) return 1;
+        if (tot > dadd(thr, cf.mg)) return 0;
         return 2;
     }
     return S < t_lo ? 1 : (S > t_hi ? 0 : 2);
@@ -1150,7 +1157,7 @@ __device__ __noinline__ ChainRec<NH> bs_chain_slow_group(ChainRec<NH> rec, uint3
     return rec;
 }
 
-// The same group when the record is one register per lane (NH == 1, D <= 15) and CONTESTED cells come in runs -- the cold
+// The same group when the record is one register per lane (NH == 1: DP <= 12) and CONTESTED cells come in runs -- the cold
 // start and the saturated parameter corners, where whole chains are CONTESTED: TWO cells per step.  The verdict of cell q + 1
 // depends on that of cell q only through which state it is added to, so its test is evaluated for BOTH outcomes of cell q
 // next to cell q's own test (three independent instruction streams for the in-order warp instead of one dependent one)
@@ -1501,7 +1508,16 @@ __global__ void __launch_bounds__(BS_CHAINP_THREADS) k_bs_chain_p(Eng e) {
         cfast.fs = ddiv(cfast.F, nm.eps2);
         cfast.invk = nm.div_mode ? ddiv(1.0, nm.k) : nm.wsel;
         cfast.delta2 = nm.delta2;
-        cfast.mg = (double)(D + 8);
+        // sum_d CF2_d / W of the chain's start state (any order: it only feeds the error bound of the clearance)
+        double q2 = 0.0;
+#pragma unroll
+        for (int h = 0; h < NH; ++h) {
+            const int el = lane + 32 * h;
+            q2 = dadd(q2, el >= DP && el < DP + D ? v[h] : 0.0);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) q2 = dadd(q2, __shfl_xor_sync(0xffffffffu, q2, o));
+        cfast.mg = dadd(DP > 16 ? 0.01 : (double)(D + 8), dmul(0x1p-48 * TH, ddiv(ddiv(q2, e.P.w[j]), nm.eps2)));
     }
 #if defined(CCB_CHAIN_PAIRS)
     bool bmode = false;

@@ -1,8 +1,10 @@
 /* CPU model of the CONTESTED-group logic of the pcore replay (chronoclust_b200/csrc/engine.cuh: bs_radius_test,
- * bs_radius_fast, bs_chain_slow_group_pairs, bs_chain_slow_group_batch) -- TEST INFRASTRUCTURE, plain loops, one "lane" per
+ * bs_radius_fast, bs_chain_slow_group, bs_chain_slow_group_pairs, bs_chain_slow_group_batch, the ChainFast setup of
+ * k_bs_chain_p) -- TEST INFRASTRUCTURE, plain loops, one "lane" per
  * record element.  It answers two questions no GPU is needed for:
  *   (1) is the division-free FAST radius test decision-exact, i.e. does it agree with the exact test of
- *       utilities/mc_functions.py:45-56 (objects/microcluster.py:213-233) whenever it takes a decision?
+ *       utilities/mc_functions.py:45-56 (objects/microcluster.py:213-233) whenever it takes a decision -- unsplit (padded
+ *       width DP <= 16) and split (DP > 16), at any distance from the origin?
  *   (2) does the EIGHT-CELLS-PER-PASS schedule (tentative records laid along predicted verdicts, -0.0 as the addend of a
  *       cell that does not join, restart behind the first deviation) leave bit for bit the state and the verdicts of the
  *       one-by-one replay, whatever the predictions are?
@@ -12,7 +14,7 @@
 #include <stdint.h>
 #include <string.h>
 
-#define MAXD 16
+#define MAXD 64
 #define GS 8
 
 typedef struct {
@@ -20,11 +22,18 @@ typedef struct {
 } Rec;
 
 typedef struct {
-    int D, div_mode;
+    int D, DP, div_mode;
     double delta2, eps2, k, wsel;
     /* ChainFast */
     double F, fs, invk, mg;
 } Prm;
+
+static int round_dp(int D) { /* csrc/api.cu: the padded width the kernels are instantiated for */
+    static const int dps[] = {4, 8, 12, 16, 24, 32, 40, 48, 64};
+    for (int i = 0; i < 9; ++i)
+        if (D <= dps[i]) return dps[i];
+    return -1;
+}
 
 static uint64_t rng_s;
 static double urand(void) { /* xorshift64* -> (0, 1) */
@@ -55,7 +64,7 @@ static Rec rec_add_negzero(const Rec *v, int D) { /* the addend of a cell that d
 }
 
 /* bs_radius_test: the reference's radius test on the tentative record, terms summed in index order */
-static int exact_test(const Rec *nv, const Prm *p) {
+static double exact_r2(const Rec *nv, const Prm *p) {
     double r2 = 0.0;
     for (int d = 0; d < p->D; ++d) {
         const double q2 = nv->cf2[d] / nv->w;
@@ -65,8 +74,9 @@ static int exact_test(const Rec *nv, const Prm *p) {
         const double t = bit ? (p->div_mode ? var / p->k : var * p->wsel) : var;
         r2 = r2 + t;
     }
-    return r2 <= p->eps2;
+    return r2;
 }
+static int exact_test(const Rec *nv, const Prm *p) { return exact_r2(nv, p) <= p->eps2; }
 
 static int d2i_rn_sat(double v) { /* cvt.rni.s32.f64: saturating, NaN -> 0 */
     if (v != v) return 0;
@@ -78,16 +88,19 @@ static int d2i_rn_sat(double v) { /* cvt.rni.s32.f64: saturating, NaN -> 0 */
 static int d2i_rd_sat(double v) { return d2i_rn_sat(floor(v)); }
 static int d2i_ru_sat(double v) { return d2i_rn_sat(ceil(v)); }
 
-/* bs_radius_fast (NT == 1, unsplit): 1 absorbed, 0 rejected, 2 too close to call */
+/* bs_radius_fast: 1 absorbed, 0 rejected, 2 too close to call.  DP <= 16: one integer per term, TH = 2^25; DP > 16: the
+ * term is split into a high integer and a low part in 2^-20 units (two redux.sync), TH = 2^23.  NT == 2 (DP > 32) only
+ * changes which lane holds a term; the integer sums do not depend on it. */
 static int fast_test(const Rec *nv, const Prm *p) {
-    const int CL = 1 << 26;
+    const int split = p->DP > 16;
+    const int CL = split ? (1 << 24) : (1 << 26);
     const double wn = nv->w;
     const double wn2 = wn * wn;
     const double thr = wn2 * p->F;
     const double d2w = p->delta2 * wn2;
     const double tol = d2w * 0x1p-24;
     const int t_lo = d2i_rd_sat(thr - p->mg), t_hi = d2i_ru_sat(thr + p->mg);
-    long long S = 0; /* redux.sync.add.s32 of at most 16 terms of magnitude <= 2^26: no overflow */
+    long long S = 0, L = 0; /* redux.sync.add.s32 of at most 64 terms of magnitude <= 2^24 (2^26 unsplit, <= 16 terms) */
     int amb = 0;
     for (int d = 0; d < p->D; ++d) {
         const double c1 = nv->cf1[d], c2 = nv->cf2[d];
@@ -100,9 +113,35 @@ static int fast_test(const Rec *nv, const Prm *p) {
         hi = hi > CL ? CL : hi;
         hi = hi < -(1 << 20) ? -(1 << 20) : hi;
         S += hi;
+        if (split) {
+            int lo = d2i_rn_sat((v - (double)hi) * 0x1p20);
+            lo = lo > (1 << 20) ? (1 << 20) : lo;
+            lo = lo < -(1 << 20) ? -(1 << 20) : lo;
+            L += lo;
+        }
     }
     if (amb) return 2;
+    if (split) {
+        const double tot = (double)(int)S + (double)(int)L * 0x1p-20;
+        if (tot < thr - p->mg) return 1;
+        if (tot > thr + p->mg) return 0;
+        return 2;
+    }
     return S < t_lo ? 1 : (S > t_hi ? 0 : 2);
+}
+
+/* ChainFast of a chain of n cells that starts at state v (engine.cuh, chain setup of k_bs_chain_p) */
+static void chain_fast(Prm *p, const Rec *v, int n) {
+    const double TH = p->DP > 16 ? 0x1p23 : 0x1p25;
+    const double wmax = v->w + (double)(n + 1);
+    p->F = TH / (wmax * wmax);
+    p->fs = p->F / p->eps2;
+    p->invk = p->div_mode ? 1.0 / p->k : p->wsel;
+    /* clearance: rounding of the integer terms (unsplit) or of the low parts (split), plus the bound on the fp64 error of
+     * the terms from the chain's start state, sum_d CF2_d / W (summed here in another order than the warp's: a bound) */
+    double q2 = 0.0;
+    for (int d = 0; d < p->D; ++d) q2 += v->cf2[d];
+    p->mg = (p->DP > 16 ? 0.01 : (double)(p->D + 8)) + 0x1p-48 * TH * (q2 / v->w) / p->eps2;
 }
 
 /* one by one with the EXACT test: the semantics everything else has to reproduce */
@@ -120,6 +159,33 @@ static void group_reference(Rec *v, const double x[GS][MAXD], unsigned cg, int n
 typedef struct {
     long long fast_decided, fast_undecided, fast_wrong, passes, groups, contested, rejected;
 } Stats;
+
+/* bs_chain_slow_group: cell by cell, the fast test first, the exact test where it cannot call (and for the first member of
+ * the chain).  The only schedule at DP >= 16, where the record takes more than one register per lane. */
+static void group_onebyone(Rec *vio, const double x[GS][MAXD], unsigned cg, int ncell, const Prm *p, int exact_first,
+                           unsigned *rej_out, Stats *st) {
+    Rec v = *vio;
+    unsigned rej = 0u;
+    for (int q = 0; q < ncell; ++q) {
+        const Rec nv = rec_add(&v, x[q], p->D);
+        int keep = 1;
+        if ((cg >> q) & 1u) {
+            int r = (q == 0 && exact_first) ? 2 : fast_test(&nv, p);
+            if (r == 2) {
+                if (!(q == 0 && exact_first)) ++st->fast_undecided;
+                r = exact_test(&nv, p);
+            } else {
+                ++st->fast_decided;
+                if (exact_test(&nv, p) != r) ++st->fast_wrong;
+            }
+            keep = r != 0;
+        }
+        if (keep) v = nv;
+        else rej |= 1u << q;
+    }
+    *vio = v;
+    *rej_out = rej;
+}
 
 /* bs_chain_slow_group_batch */
 static void group_batch(Rec *vio, const double x[GS][MAXD], unsigned cg, unsigned pg, int ncell, const Prm *p, int exact_first,
@@ -247,6 +313,7 @@ long long cgm_run(uint64_t seed, int D, int div_mode, double kk, double eps, dou
     Prm p;
     memset(&p, 0, sizeof p);
     p.D = D;
+    p.DP = round_dp(D);
     p.div_mode = div_mode;
     p.k = kk;
     p.wsel = 1.0 / kk;
@@ -265,12 +332,7 @@ long long cgm_run(uint64_t seed, int D, int div_mode, double kk, double eps, dou
         const Rec nv = rec_add(&v, x, D);
         if (exact_test(&nv, &p)) v = nv;
     }
-    const double TH = 0x1p25;
-    const double wmax = v.w + (double)(ngroups * GS + 1);
-    p.F = TH / (wmax * wmax);
-    p.fs = p.F / p.eps2;
-    p.invk = div_mode ? 1.0 / kk : p.wsel;
-    p.mg = (double)(D + 8);
+    chain_fast(&p, &v, ngroups * GS);
     Stats st;
     memset(&st, 0, sizeof st);
     long long bad = 0;
@@ -297,8 +359,14 @@ long long cgm_run(uint64_t seed, int D, int div_mode, double kk, double eps, dou
         case 3: pg = rej_ref; break;
         default: pg = rej_ref ^ 0x88u; break;
         }
-        group_batch(&vb, x, cg, pg, ncell, &p, g == 0, &rej_b, &st);
-        group_pairs(&vp, x, cg, ncell, &p, g == 0, &rej_p, &st);
+        if (p.DP <= 12) { /* the record is one register per lane (NH == 1): the two group schedules */
+            group_batch(&vb, x, cg, pg, ncell, &p, g == 0, &rej_b, &st);
+            group_pairs(&vp, x, cg, ncell, &p, g == 0, &rej_p, &st);
+        } else {
+            group_onebyone(&vb, x, cg, ncell, &p, g == 0, &rej_b, &st);
+            vp = vb;
+            rej_p = rej_b;
+        }
         ++st.groups;
         st.contested += __builtin_popcount(cg);
         st.rejected += __builtin_popcount(rej_ref);
@@ -315,4 +383,49 @@ long long cgm_run(uint64_t seed, int D, int div_mode, double kk, double eps, dou
     out[5] = st.contested;
     out[6] = st.rejected;
     return bad;
+}
+
+/* The fast test AT the decision boundary: a record of W cells drawn around a centre (coordinates centre_scale * U(0, 1)) with
+ * spread sigma, and eps^2 placed at the reference's own r^2 of that record times 1 +- rho, rho log-uniform in
+ * [1e-11, 1e-5] -- where the fp64 error of the fast test's terms decides.  ntrials records; out[0..2] = fast decided /
+ * undecided / wrong. */
+void cgm_boundary(uint64_t seed, int D, int div_mode, double kk, double delta, double W, double centre_scale, double sigma,
+                  int ntrials, long long *out) {
+    rng_s = seed * 0x9E3779B97F4A7C15ULL + 0x7654321ULL;
+    Prm p;
+    memset(&p, 0, sizeof p);
+    p.D = D;
+    p.DP = round_dp(D);
+    p.div_mode = div_mode;
+    p.k = kk;
+    p.wsel = 1.0 / kk;
+    p.delta2 = delta * delta;
+    Stats st;
+    memset(&st, 0, sizeof st);
+    for (int it = 0; it < ntrials; ++it) {
+        double centre[MAXD];
+        for (int d = 0; d < D; ++d) centre[d] = centre_scale * urand();
+        Rec v;
+        memset(&v, 0, sizeof v);
+        for (int i = 0; i < (int)W; ++i) {
+            double x[MAXD];
+            for (int d = 0; d < D; ++d) x[d] = centre[d] + sigma * nrand();
+            v = rec_add(&v, x, D);
+        }
+        p.eps2 = 1.0; /* (exact_r2 does not read eps^2) */
+        const double r2 = exact_r2(&v, &p);
+        const double rho = exp(log(1e-11) + urand() * (log(1e-5) - log(1e-11)));
+        p.eps2 = r2 * (urand() < 0.5 ? 1.0 - rho : 1.0 + rho);
+        chain_fast(&p, &v, 0); /* (Wmax = W + 1, as for a chain whose last member brings W' to W) */
+        const int r = fast_test(&v, &p);
+        if (r == 2) {
+            ++st.fast_undecided;
+            continue;
+        }
+        ++st.fast_decided;
+        if (r != exact_test(&v, &p)) ++st.fast_wrong;
+    }
+    out[0] = st.fast_decided;
+    out[1] = st.fast_undecided;
+    out[2] = st.fast_wrong;
 }
