@@ -12,7 +12,9 @@
 #include <cstdio>
 #include <cstring>
 #include <functional>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "nearest.cuh"
@@ -54,70 +56,163 @@ bool is_pow2(double k) {
 
 constexpr int MAX_SLABS = 148;
 
+// ---- owners of device memory, page-locked host memory, streams, events and graphs -----------------------------------
+// Move-only; the destructor releases what the owner holds.  An owner takes what a call made only when the call succeeded
+// (the runtime does not promise what a failed call leaves in its output argument).  An owner converts to the raw pointer
+// or handle, which is what the kernels and the runtime take.
+template <typename T, auto Release>
+struct Own {
+    T p{};
+    Own() = default;
+    explicit Own(T q) : p(q) {}
+    Own(Own &&o) noexcept : p(o.p) { o.p = T{}; }
+    Own &operator=(Own &&o) noexcept { // (what this held goes to o and is released with it)
+        std::swap(p, o.p);
+        return *this;
+    }
+    ~Own() {
+        if (p) Release(p);
+    }
+    operator T() const { return p; }
+    T operator->() const { return p; }
+};
+template <typename T> using Dev = Own<T *, cudaFree>;
+template <typename T> using Pinned = Own<T *, cudaFreeHost>;
+using Stream = Own<cudaStream_t, cudaStreamDestroy>;
+using Event = Own<cudaEvent_t, cudaEventDestroy>;
+
+template <typename O, typename F>
+cudaError_t make(O &o, F create) {
+    decltype(o.p) q{};
+    const cudaError_t e = create(&q);
+    if (e == cudaSuccess) o = O(q);
+    return e;
+}
+template <typename T> cudaError_t alloc(Dev<T> &o, size_t bytes) { return make(o, [=](T **q) { return cudaMalloc(q, bytes); }); }
+template <typename T> cudaError_t alloc(Pinned<T> &o, size_t bytes) { return make(o, [=](T **q) { return cudaMallocHost(q, bytes); }); }
+cudaError_t create(Stream &o, int prio) {
+    return make(o, [=](cudaStream_t *q) { return cudaStreamCreateWithPriority(q, cudaStreamNonBlocking, prio); });
+}
+cudaError_t create(Event &o, unsigned flags) { return make(o, [=](cudaEvent_t *q) { return cudaEventCreateWithFlags(q, flags); }); }
+
+// Grow-only buffer.  ensure(bytes) does nothing when the capacity suffices; a growth allocates the new memory before it
+// releases the old, and a failed one keeps the old memory and capacity.  Contents are not preserved.
+template <typename O>
+struct Grow : O {
+    size_t cap = 0;
+    cudaError_t ensure(size_t bytes) {
+        if (bytes <= cap) return cudaSuccess;
+        O n;
+        const cudaError_t e = alloc(n, bytes);
+        if (e != cudaSuccess) return e;
+        O::operator=(std::move(n));
+        cap = bytes;
+        return cudaSuccess;
+    }
+};
+
+// Stream-ordered pool memory for the length of a scope: cudaMallocAsync on s, cudaFreeAsync on s when the scope ends.
+struct Scratch {
+    const cudaStream_t s;
+    void *p = nullptr;
+    explicit Scratch(cudaStream_t st) : s(st) {}
+    Scratch(const Scratch &) = delete;
+    ~Scratch() {
+        if (p) cudaFreeAsync(p, s);
+    }
+    cudaError_t alloc(size_t bytes) {
+        void *q;
+        const cudaError_t e = cudaMallocAsync(&q, bytes, s);
+        if (e == cudaSuccess) p = q;
+        return e;
+    }
+    template <typename T> T *as() const { return static_cast<T *>(p); }
+};
+
+// the arrays of one microcluster list; Store is their view for the kernels
+struct StoreMem {
+    Dev<double> cf1, cf2, cen, w;
+    Dev<uint64_t> mask;
+    Dev<int64_t> id;
+    Dev<int32_t> uid;
+    Dev<double2> cw;
+    int cap = 0;
+    Store view() const {
+        Store s;
+        memset(&s, 0, sizeof s); // (Eng holds Stores and is compared with memcmp)
+        s.cf1 = cf1, s.cf2 = cf2, s.cen = cen, s.w = w, s.mask = mask, s.id = id, s.uid = uid, s.cw = cw;
+        s.cap = cap;
+        return s;
+    }
+};
+
+// what the block-speculative engine allocates once per handle: control blocks, the arrays of BsWs, kernel 1's slab lists
+struct BsMem {
+    Dev<BsCtl> bc;
+    Pinned<BsCtl> h_bc;
+    Dev<EngIo> io;
+    Pinned<EngIo> h_io;
+    std::vector<Dev<void>> arrays;
+    double *tk_dist_slab = nullptr;
+    int32_t *tk_idx_slab = nullptr;
+};
+
+struct GraphSlot { // a graph of the engine, its executable and the Eng it was captured with
+    Own<cudaGraph_t, cudaGraphDestroy> graph;
+    Own<cudaGraphExec_t, cudaGraphExecDestroy> exec;
+    Eng eng{};
+};
+
 } // namespace
 
 struct ccb_handle {
     ccb_params prm{};
     int D = 0, DP = 0, div_mode = 0, cnt_gt1 = 0;
     double wsel = 1.0;
-    cudaStream_t stream = nullptr;
-    Store P[2]{}, O[2]{};
+    Stream stream; // first member: destroyed last, after everything that was enqueued on it
+    StoreMem Pm[2], Om[2];
+    Store P[2]{}, O[2]{}; // their views
     int pcur = 0, ocur = 0;
-    Ctl *d_ctl = nullptr, *h_ctl = nullptr;
+    Dev<Ctl> d_ctl;
+    Pinned<Ctl> h_ctl;
     double mu = 0, omicron = 0;
     int64_t pi = 0;
     bool have_params = false;
     // ingest buffers
-    double *d_X = nullptr;
-    size_t x_cap = 0;
-    int32_t *d_assign = nullptr;
-    uint8_t *d_stage = nullptr;
-    size_t n_cap = 0;
-    int32_t *d_pnew = nullptr, *d_pfin = nullptr, *d_onew = nullptr; // kernel 3 plan codes
+    Grow<Dev<double>> d_X;
+    Grow<Dev<int32_t>> d_assign;
+    Grow<Dev<uint8_t>> d_stage;
+    Grow<Dev<int32_t>> d_pnew, d_pfin, d_onew; // kernel 3 plan codes
     // block-speculative engine (engine.cuh)
     int bs_bmax = 32768, bs_bmin = 1024, bs_iters = 3;
-    BsCtl *d_bc = nullptr, *h_bc = nullptr;
-    BsWs ws{};
-    std::vector<void *> ws_allocs;
-    void *ws_tiles[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    int32_t *ws_first = nullptr;
+    BsMem bs;
+    BsWs ws{}; // view of bs, ws_tiles, ws_dbg and ws_first
+    Dev<void> ws_tiles[7];
+    Dev<int64_t> ws_dbg;
+    Dev<int32_t> ws_first;
     int ws_first_cap = 0;
-    double *d_bs_tk_dist_slab = nullptr;
-    int32_t *d_bs_tk_idx_slab = nullptr;
     BsCtl bc_base{}; // counters folded in by ccb_reset
     bool bs_use_graph = true;   // CUDA graph with device-driven WHILE nodes (stream launches when per-kernel timing is on)
     // Two cached graphs: the double-buffered stores flip at every ccb_begin_timepoint with decay, so consecutive timepoints
     // alternate between two sets of (baked-in) pointers -- with one slot the graph was re-captured and re-instantiated at
-    // every timepoint (~1 ms each).
-    // programmatic dependent launch between the engine's kernels: measured neutral on B200 (profiles/r2zc_pdl_experiment.md:
-    // the gaps between the kernels of a round are not launch latency), so it is off; the kernels keep CCB_PDL() (a no-op then)
-    bool pdl = false;
-    cudaGraph_t bs_graph = nullptr, bs_graph_alt = nullptr;
-    cudaGraphExec_t bs_exec = nullptr, bs_exec_alt = nullptr;
-    Eng bs_graph_eng_alt{};
-    cudaStream_t cap1 = nullptr, cap2 = nullptr, cap3 = nullptr; // capture streams: block loop, round loop, side branch
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    cudaStream_t copy_stream = nullptr; // host -> device segments of ccb_ingest, ahead of the engine
-    cudaStream_t res_stream = nullptr;  // device -> host copies of the per-cell results of a finished segment, behind the engine
-    unsigned char *h_res = nullptr;     // page-locked bounce buffer of those results ([n] int32 assignments, then [n] stages)
-    size_t res_cap = 0;                 // (rows)
-    double *d_scale = nullptr;          // [2][CCB_MAX_D] scale_ / min_ of ccb_ingest_scaled
-    cudaEvent_t ev_seg[8] = {nullptr};
-    Eng bs_graph_eng{};         // the pointers / capacities the graph was captured with
-    EngIo *d_io = nullptr, *h_io = nullptr;
+    // every timepoint (~1 ms each).  [0] is the current slot.
+    GraphSlot graphs[2];
+    Stream cap[3]; // capture streams: block loop, round loop, side branch
+    Event ev_fork, ev_join;
+    Stream copy_stream; // host -> device segments of ccb_ingest, ahead of the engine
+    Stream res_stream;  // device -> host copies of the per-cell results of a finished segment, behind the engine
+    Grow<Pinned<unsigned char>> h_res; // page-locked bounce buffer of those results ([n] int32 assignments, then [n] stages)
+    Grow<Dev<double>> d_scale;          // [2][CCB_MAX_D] scale_ / min_ of ccb_ingest_scaled
+    Event ev_seg[8];
     // offline results (host copies)
     int64_t off_M = 0;
     std::vector<int64_t> cl_off, cl_members;
     std::vector<double> cl_w, cl_cf1, cl_cf2, cl_cen, cl_pref;
     std::vector<int32_t> cl_label;
     // offline workspace: grow-only device buffers, kept between calls (the white-box export reads them lazily)
-    struct OffBuf {
-        void *p = nullptr;
-        size_t bytes = 0;
-    };
     enum { OB_CORE, OB_CLS, OB_NBR, OB_WNBR, OB_CNT, OB_QUEUE, OB_LABEL, OB_ORDER, OB_CLOFF, OB_NCL, OB_SUBMASK, OB_OMASK,
            OB_D1, OB_D2, OB_DC, OB_DW, OB_COUNT };
-    OffBuf ob[OB_COUNT];
+    Grow<Dev<void>> ob[OB_COUNT];
     int off_csr_min_m = 0;
     ccb_stats st{};
     ccb_stats st_base{}; // device-side counters folded in by ccb_reset
@@ -125,9 +220,9 @@ struct ccb_handle {
     void *dnrm2 = nullptr;
     // optional per-category GPU timing (CUDA events on the handle's stream)
     bool timing = false;
-    struct Ev { cudaEvent_t a, b; int cat; };
+    struct Ev { Event a, b; int cat; };
     std::vector<Ev> ev_pending;
-    std::vector<cudaEvent_t> ev_pool;
+    std::vector<Event> ev_pool;
     double cat_ms[CCB_NCAT] = {0};
     int64_t cat_n[CCB_NCAT] = {0};
 };
@@ -144,14 +239,25 @@ int fail(ccb_handle *h, int code, const char *fmt, ...) {
     g_err = buf;
     return code;
 }
+// A failed call stays the runtime's last error until someone reads it: CK clears it, so that the next launch check
+// does not report it again.
 #define CK(h, call)                                                                                        \
     do {                                                                                                   \
         cudaError_t e_ = (call);                                                                           \
-        if (e_ != cudaSuccess)                                                                             \
+        if (e_ != cudaSuccess) {                                                                           \
+            cudaGetLastError();                                                                            \
             return fail(h, e_ == cudaErrorMemoryAllocation ? CCB_ENOMEM : CCB_ECUDA, "%s:%d %s: %s", __FILE__, \
                         __LINE__, #call, cudaGetErrorString(e_));                                          \
+        }                                                                                                  \
     } while (0)
 #define CKL(h) CK(h, cudaGetLastError())
+
+// first call of every entry point that takes a handle
+int enter(ccb_handle *h) {
+    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
+    CK(h, cudaSetDevice(h->prm.device));
+    return CCB_OK;
+}
 
 // RAII bracket: records CUDA events around the launches of one category when timing is enabled
 struct Timed {
@@ -160,25 +266,23 @@ struct Timed {
     bool on;
     Timed(ccb_handle *h_, int cat) : h(h_), on(h_ && h_->timing) {
         if (!on) return;
-        auto get = [&]() {
-            cudaEvent_t x;
-            if (!h->ev_pool.empty()) {
-                x = h->ev_pool.back();
-                h->ev_pool.pop_back();
-            } else {
-                cudaEventCreate(&x);
+        auto get = [&](Event &x) {
+            if (h->ev_pool.empty()) {
+                create(x, cudaEventDefault);
+                return;
             }
-            return x;
+            x = std::move(h->ev_pool.back());
+            h->ev_pool.pop_back();
         };
-        e.a = get();
-        e.b = get();
+        get(e.a);
+        get(e.b);
         e.cat = cat;
         cudaEventRecord(e.a, h->stream);
     }
     void stop() {
         if (!on) return;
         cudaEventRecord(e.b, h->stream);
-        h->ev_pending.push_back(e);
+        h->ev_pending.push_back(std::move(e));
         on = false;
     }
     ~Timed() { stop(); }
@@ -190,78 +294,55 @@ void drain_timing(ccb_handle *h) { // call after a stream synchronize
             h->cat_ms[e.cat] += ms;
             h->cat_n[e.cat] += 1;
         }
-        h->ev_pool.push_back(e.a);
-        h->ev_pool.push_back(e.b);
+        h->ev_pool.push_back(std::move(e.a));
+        h->ev_pool.push_back(std::move(e.b));
     }
     h->ev_pending.clear();
 }
 
-int alloc_store(ccb_handle *h, Store &S, int cap) {
-    const int D = h->D, DP = h->DP;
-    S = Store{};
+int alloc_store(ccb_handle *h, StoreMem &S, int cap) {
+    const size_t nd = (size_t)cap * h->D + 2; // + slack for 16-byte rounded bulk copies
+    CK(h, alloc(S.cf1, nd * 8));
+    CK(h, alloc(S.cf2, nd * 8));
+    CK(h, alloc(S.cen, nd * 8));
+    CK(h, alloc(S.w, (size_t)cap * 8));
+    CK(h, alloc(S.mask, (size_t)cap * 8));
+    CK(h, alloc(S.id, (size_t)cap * 8));
+    CK(h, alloc(S.uid, (size_t)cap * 4));
+    CK(h, alloc(S.cw, (size_t)cap * h->DP * sizeof(double2)));
     S.cap = cap;
-    const size_t nd = (size_t)cap * D + 2; // + slack for 16-byte rounded bulk copies
-    CK(h, cudaMalloc(&S.cf1, nd * 8));
-    CK(h, cudaMalloc(&S.cf2, nd * 8));
-    CK(h, cudaMalloc(&S.cen, nd * 8));
-    CK(h, cudaMalloc(&S.w, (size_t)cap * 8));
-    CK(h, cudaMalloc(&S.mask, (size_t)cap * 8));
-    CK(h, cudaMalloc(&S.id, (size_t)cap * 8));
-    CK(h, cudaMalloc(&S.uid, (size_t)cap * 4));
-    CK(h, cudaMalloc(&S.cw, (size_t)cap * DP * sizeof(double2)));
     return CCB_OK;
 }
-void free_store(Store &S) {
-    cudaFree(S.cf1);
-    cudaFree(S.cf2);
-    cudaFree(S.cen);
-    cudaFree(S.w);
-    cudaFree(S.mask);
-    cudaFree(S.id);
-    cudaFree(S.uid);
-    cudaFree(S.cw);
-    S = Store{};
-}
-// grows both ping-pong buffers of a list to >= want entries, preserving the first n of the current one
-int grow_store(ccb_handle *h, Store (&S)[2], int cur, int n, int64_t want) {
+// Grows both ping-pong buffers of a list to >= want entries, preserving the first n of the current one.  Both new
+// buffers are allocated and filled before the list takes them: after a failure the list keeps its old pair.
+int grow_store(ccb_handle *h, bool outliers, int n, int64_t want) {
+    StoreMem *S = outliers ? h->Om : h->Pm;
+    const int cur = outliers ? h->ocur : h->pcur;
     if (want <= S[cur].cap) return CCB_OK;
     int64_t cap = S[cur].cap;
     while (cap < want) cap *= 2;
     if (cap > (int64_t)1 << 30) return fail(h, CCB_ELIMIT, "microcluster list would exceed 2^30 entries");
     const int D = h->D, DP = h->DP;
-    Store nw;
-    int rc = alloc_store(h, nw, (int)cap);
-    if (rc) return rc;
-    Store &o = S[cur];
+    StoreMem nw[2];
+    int rc;
+    if ((rc = alloc_store(h, nw[cur], (int)cap)) || (rc = alloc_store(h, nw[1 - cur], (int)cap))) return rc;
+    const StoreMem &o = S[cur];
+    StoreMem &c = nw[cur];
     cudaStream_t s = h->stream;
-    CK(h, cudaMemcpyAsync(nw.cf1, o.cf1, (size_t)n * D * 8, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.cf2, o.cf2, (size_t)n * D * 8, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.cen, o.cen, (size_t)n * D * 8, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.w, o.w, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.mask, o.mask, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.id, o.id, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.uid, o.uid, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
-    CK(h, cudaMemcpyAsync(nw.cw, o.cw, (size_t)n * DP * sizeof(double2), cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.cf1, o.cf1, (size_t)n * D * 8, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.cf2, o.cf2, (size_t)n * D * 8, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.cen, o.cen, (size_t)n * D * 8, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.w, o.w, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.mask, o.mask, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.id, o.id, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.uid, o.uid, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
+    CK(h, cudaMemcpyAsync(c.cw, o.cw, (size_t)n * DP * sizeof(double2), cudaMemcpyDeviceToDevice, s));
     CK(h, cudaStreamSynchronize(s));
-    free_store(S[cur]);
-    free_store(S[1 - cur]);
-    S[cur] = nw;
-    rc = alloc_store(h, S[1 - cur], (int)cap);
-    return rc;
-}
-
-int realloc_aux_for_outlier_cap(ccb_handle *h) {
-    const int cap = h->O[h->ocur].cap;
-    cudaFree(h->d_onew);
-    CK(h, cudaMalloc(&h->d_onew, (size_t)cap * 4));
-    return CCB_OK;
-}
-int realloc_aux_for_pcore_cap(ccb_handle *h) {
-    const int cap = h->P[h->pcur].cap;
-    cudaFree(h->d_pnew);
-    cudaFree(h->d_pfin);
-    CK(h, cudaMalloc(&h->d_pnew, (size_t)cap * 4));
-    CK(h, cudaMalloc(&h->d_pfin, (size_t)cap * 4));
+    Store *V = outliers ? h->O : h->P;
+    for (int i = 0; i < 2; ++i) {
+        S[i] = std::move(nw[i]);
+        V[i] = S[i].view();
+    }
     return CCB_OK;
 }
 
@@ -387,47 +468,35 @@ int launch_nearest_dyn(ccb_handle *h, cudaStream_t s, int DP, int div_mode, cons
     return CCB_OK;
 }
 
-int ensure_point_buffers(ccb_handle *h, int64_t N) {
-    if ((size_t)N > h->n_cap) {
-        cudaFree(h->d_assign);
-        cudaFree(h->d_stage);
-        h->n_cap = 0;
-        CK(h, cudaMalloc(&h->d_assign, (size_t)N * 4));
-        CK(h, cudaMalloc(&h->d_stage, (size_t)N));
-        h->n_cap = (size_t)N;
-    }
-    return CCB_OK;
-}
-
 // ---- block-speculative engine: workspace and block enqueue ------------------------------------------
 constexpr int BS_MAX_SLABS = 256; // (k_topk_merge_dyn: a lane walks up to 8 slab lists)
 
-template <typename T>
-int ws_alloc(ccb_handle *h, T *&p, size_t n) {
-    void *q = nullptr;
-    CK(h, cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T)));
-    h->ws_allocs.push_back(q);
-    p = (T *)q;
-    return CCB_OK;
-}
-
+// The workspace of the engine.  Each part is built aside and taken by the handle (and its view ws) only once every
+// allocation of the part has succeeded.
 int ensure_bs_ws(ccb_handle *h) {
-    int rc;
     const int B = h->bs_bmax, D = h->D;
-    if (!h->d_bc) {
+    if (!h->bs.bc) {
         CCB_DISPATCH_DP(h->DP, {
             CK(h, cudaFuncSetAttribute(k_bs_chain_p<kDP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)ChainPCfg<kDP>::SMEM));
         })
-        CK(h, cudaMalloc(&h->d_bc, sizeof(BsCtl)));
-        CK(h, cudaMemset(h->d_bc, 0, sizeof(BsCtl)));
-        CK(h, cudaMallocHost(&h->h_bc, sizeof(BsCtl)));
-        memset(h->h_bc, 0, sizeof(BsCtl));
-        CK(h, cudaMalloc(&h->d_io, sizeof(EngIo)));
-        CK(h, cudaMallocHost(&h->h_io, sizeof(EngIo)));
-        BsWs &w = h->ws;
+        BsMem m;
+        CK(h, alloc(m.bc, sizeof(BsCtl)));
+        CK(h, cudaMemset(m.bc, 0, sizeof(BsCtl)));
+        CK(h, alloc(m.h_bc, sizeof(BsCtl)));
+        memset(m.h_bc, 0, sizeof(BsCtl));
+        CK(h, alloc(m.io, sizeof(EngIo)));
+        CK(h, alloc(m.h_io, sizeof(EngIo)));
+        BsWs w = h->ws;
         w.bmax = B;
-#define WSA(field, n) if ((rc = ws_alloc(h, w.field, (n)))) return rc
+        auto arr = [&](auto *&p, size_t n) {
+            Dev<void> d;
+            const cudaError_t e = alloc(d, std::max<size_t>(n, 1) * sizeof(*p));
+            p = static_cast<std::remove_reference_t<decltype(p)>>(d.p);
+            m.arrays.push_back(std::move(d));
+            return e;
+        };
+#define WSA(field, n) CK(h, arr(w.field, (n)))
         WSA(pcand, B); WSA(ospec, B); WSA(tkpos, B); WSA(dec, B); WSA(eff, B); WSA(newrank, B); WSA(pend, B); WSA(vpos, B); WSA(pbest, B);
         WSA(pflag, B); WSA(prej, B); WSA(upf, B);
         w.dp = h->DP;
@@ -439,47 +508,44 @@ int ensure_bs_ws(ccb_handle *h) {
         WSA(hkey, BS_RMAX + 1); WSA(hoff, BS_RMAX + 2); WSA(omem, BS_RMAX + 1); WSA(hrank, BS_RMAX + 2);
         WSA(hfirst, BS_RMAX + 1); WSA(okeys, BS_RMAX);
 #undef WSA
-        if ((rc = ws_alloc(h, h->d_bs_tk_dist_slab, (size_t)BS_RMAX * BS_MAX_SLABS * BS_TOPK))) return rc;
-        if ((rc = ws_alloc(h, h->d_bs_tk_idx_slab, (size_t)BS_RMAX * BS_MAX_SLABS * BS_TOPK))) return rc;
+        CK(h, arr(m.tk_dist_slab, (size_t)BS_RMAX * BS_MAX_SLABS * BS_TOPK));
+        CK(h, arr(m.tk_idx_slab, (size_t)BS_RMAX * BS_MAX_SLABS * BS_TOPK));
+        h->bs = std::move(m);
+        h->ws = w;
     }
     // per-(tile, pcore key) tables follow the pcore capacity; the modified-flags follow the outlier capacity
     const int stride = h->P[h->pcur].cap;
     if (stride != h->ws.mp_stride) {
-        for (void *&q : h->ws_tiles) {
-            cudaFree(q);
-            q = nullptr;
-        }
         const size_t n = ((size_t)B / 32 + 2) * stride;
         const size_t npl = (size_t)B + 4 * (size_t)stride + 8; // every key's segment is padded to a multiple of 4
         const size_t ds = (size_t)h->ws.lsp;
-        CK(h, cudaMalloc(&h->ws_tiles[0], n * 4));
-        CK(h, cudaMalloc(&h->ws_tiles[1], n * 4));
-        CK(h, cudaMalloc(&h->ws_tiles[2], ((size_t)stride + 2) * 4));
-        CK(h, cudaMalloc(&h->ws_tiles[3], ((size_t)stride + 2) * 4));
-        CK(h, cudaMalloc(&h->ws_tiles[4], npl * 4));
-        CK(h, cudaMalloc(&h->ws_tiles[5], npl * ds * 8));
-        CK(h, cudaMalloc(&h->ws_tiles[6], npl * ds * 8));
-        h->ws.tilecnt = (int32_t *)h->ws_tiles[0];
-        h->ws.tbase = (int32_t *)h->ws_tiles[1];
-        h->ws.poff = (int32_t *)h->ws_tiles[2];
-        h->ws.pcnt = (int32_t *)h->ws_tiles[3];
-        h->ws.plist = (int32_t *)h->ws_tiles[4];
-        h->ws.xg = (double *)h->ws_tiles[5];
-        h->ws.verp = (double *)h->ws_tiles[6];
-        h->ws.mp_stride = stride;
-        if (h->ws.dbg) {
-            cudaFree(h->ws.dbg);
-            h->ws.dbg = nullptr;
-            CK(h, cudaMalloc(&h->ws.dbg, (size_t)stride * 8 * sizeof(int64_t)));
-            CK(h, cudaMemset(h->ws.dbg, 0, (size_t)stride * 8 * sizeof(int64_t)));
+        const size_t bytes[7] = {n * 4, n * 4, ((size_t)stride + 2) * 4, ((size_t)stride + 2) * 4, npl * 4, npl * ds * 8,
+                                 npl * ds * 8};
+        Dev<void> t[7];
+        for (int i = 0; i < 7; ++i) CK(h, alloc(t[i], bytes[i]));
+        Dev<int64_t> dbg;
+        if (h->ws_dbg) {
+            CK(h, alloc(dbg, (size_t)stride * 8 * sizeof(int64_t)));
+            CK(h, cudaMemset(dbg, 0, (size_t)stride * 8 * sizeof(int64_t)));
         }
+        std::swap(h->ws_tiles, t);
+        h->ws_dbg = std::move(dbg);
+        h->ws.tilecnt = (int32_t *)h->ws_tiles[0].p;
+        h->ws.tbase = (int32_t *)h->ws_tiles[1].p;
+        h->ws.poff = (int32_t *)h->ws_tiles[2].p;
+        h->ws.pcnt = (int32_t *)h->ws_tiles[3].p;
+        h->ws.plist = (int32_t *)h->ws_tiles[4].p;
+        h->ws.xg = (double *)h->ws_tiles[5].p;
+        h->ws.verp = (double *)h->ws_tiles[6].p;
+        h->ws.dbg = h->ws_dbg;
+        h->ws.mp_stride = stride;
     }
     const int ocap = h->O[h->ocur].cap;
     if (ocap != h->ws_first_cap) {
-        cudaFree(h->ws_first);
-        h->ws_first = nullptr;
-        CK(h, cudaMalloc(&h->ws_first, (size_t)ocap * 4));
-        CK(h, cudaMemsetAsync(h->ws_first, 0x7f, (size_t)ocap * 4, h->stream)); // 0x7f7f7f7f: "not modified"
+        Dev<int32_t> f;
+        CK(h, alloc(f, (size_t)ocap * 4));
+        CK(h, cudaMemsetAsync(f, 0x7f, (size_t)ocap * 4, h->stream)); // 0x7f7f7f7f: "not modified"
+        h->ws_first = std::move(f);
         h->ws_first_cap = ocap;
         h->ws.firstmember = h->ws_first;
     }
@@ -488,7 +554,7 @@ int ensure_bs_ws(ccb_handle *h) {
 
 int sync_bc(ccb_handle *h) { // both control blocks -> pinned host mirrors
     CK(h, cudaMemcpyAsync(h->h_ctl, h->d_ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(h->h_bc, h->d_bc, sizeof(BsCtl), cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaMemcpyAsync(h->bs.h_bc, h->bs.bc, sizeof(BsCtl), cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
     if (h->timing) drain_timing(h);
     return CCB_OK;
@@ -499,28 +565,24 @@ int sync_bc(ccb_handle *h) { // both control blocks -> pinned host mirrors
 // launched either on the handle's stream (bs_iters rounds enqueued per block; used when per-kernel timing is on) or
 // captured once into a CUDA graph whose block loop and round loop are WHILE conditional nodes driven from the
 // device (k_bs_begin / k_bs_decide / k_bs_commit call cudaGraphSetConditional): no idle launches, no host round trip.
-// Kernel launch with (pdl) or without the programmatic-stream-serialization attribute (see CCB_PDL in common.cuh)
+// Kernel launch without attributes.  The kernels start with CCB_PDL() (common.cuh), but the host no longer sets the
+// programmatic-stream-serialization attribute: programmatic dependent launch was measured neutral on the B200 (DESIGN.md
+// §6: the gaps between the kernels of a round are not launch latency), so both of its instructions are no-ops.
 template <typename... KA, typename... A>
-cudaError_t launch_k(bool pdl, void (*k)(KA...), dim3 g, dim3 b, size_t smem, cudaStream_t s, A &&...a) {
+cudaError_t launch_k(void (*k)(KA...), dim3 g, dim3 b, size_t smem, cudaStream_t s, A &&...a) {
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = g;
     cfg.blockDim = b;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = pdl ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, k, KA(std::forward<A>(a))...);
 }
 
 int launch_prologue(ccb_handle *h, const Eng &e, cudaStream_t s) {
     const int g_cells = (h->bs_bmax + BS_THREADS - 1) / BS_THREADS;
     Timed tm(h, CCB_CAT_SPEC);
-    const bool pdl = h->pdl;
     k_bs_begin<<<1, 1, 0, s>>>(e);
-    CCB_DISPATCH_DP(h->DP, { launch_k(pdl, k_bs_spec<kDP>, g_cells * BS_SPLIT, BS_THREADS, 0, s, e); })
+    CCB_DISPATCH_DP(h->DP, { launch_k(k_bs_spec<kDP>, g_cells * BS_SPLIT, BS_THREADS, 0, s, e); })
     CKL(h);
     return CCB_OK;
 }
@@ -533,7 +595,6 @@ int launch_round(ccb_handle *h, const Eng &e, cudaStream_t s, int mp_grid, int m
     const int g_cells = (B + BS_THREADS - 1) / BS_THREADS;
     const int g_tiles = (B / 32 + 1 + 3) / 4;
     int rc;
-    const bool pdl = h->pdl;
     cudaStream_t sa = side ? side : s;
     if (side) {
         CK(h, cudaEventRecord(h->ev_fork, s));
@@ -542,24 +603,24 @@ int launch_round(ccb_handle *h, const Eng &e, cudaStream_t s, int mp_grid, int m
     {
         Timed tm(h, CCB_CAT_NEAREST);
         if ((rc = launch_nearest_dyn<BS_TOPK>(nullptr, sa, h->DP, h->div_mode, e.X, e.ws.nrows, e.ld, h->D, e.O.cw, mo_bound,
-                                              h->d_bs_tk_dist_slab, h->d_bs_tk_idx_slab, e.ws.tk_dist, e.ws.tk_idx,
+                                              h->bs.tk_dist_slab, h->bs.tk_idx_slab, e.ws.tk_dist, e.ws.tk_idx,
                                               BS_MAX_SLABS, BS_RMAX, &e.bc->tk_lo, &e.bc->Mo0,
                                               reinterpret_cast<const XRef *>(e.io))))
             return fail(h, rc, "%s", ccb_last_error(nullptr));
     }
     {
         Timed tm(h, CCB_CAT_SPEC);
-        launch_k(pdl, k_bs_spec_o, BS_RMAX / BS_THREADS, BS_THREADS, 0, sa, e);
+        launch_k(k_bs_spec_o, BS_RMAX / BS_THREADS, BS_THREADS, 0, sa, e);
     }
     {
         Timed tm(h, CCB_CAT_LISTS);
-        launch_k(pdl, k_bs_tilecnt, g_tiles, BS_THREADS, 0, s, e);
-        launch_k(pdl, k_bs_pscan, std::max(mp_grid, 1), BS_CTA1, 0, s, e);
-        launch_k(pdl, k_bs_pscatter, B / 32 + 1, BS_THREADS, 0, s, e);
+        launch_k(k_bs_tilecnt, g_tiles, BS_THREADS, 0, s, e);
+        launch_k(k_bs_pscan, std::max(mp_grid, 1), BS_CTA1, 0, s, e);
+        launch_k(k_bs_pscatter, B / 32 + 1, BS_THREADS, 0, s, e);
     }
     {
         Timed tm(h, CCB_CAT_PCORE);
-        CCB_DISPATCH_DP(h->DP, { launch_k(pdl, k_bs_chain_p<kDP>, std::max(mp_grid, 1), BS_CHAINP_THREADS, ChainPCfg<kDP>::SMEM, s, e); })
+        CCB_DISPATCH_DP(h->DP, { launch_k(k_bs_chain_p<kDP>, std::max(mp_grid, 1), BS_CHAINP_THREADS, ChainPCfg<kDP>::SMEM, s, e); })
     }
     if (side) { // join: k_bs_olist needs the speculated outlier decisions, everything below the pcore replay
         CK(h, cudaEventRecord(h->ev_join, side));
@@ -570,23 +631,23 @@ int launch_round(ccb_handle *h, const Eng &e, cudaStream_t s, int mp_grid, int m
     }
     {
         Timed tm(h, CCB_CAT_DERIVE);
-        launch_k(pdl, k_bs_derive_p, g_cells, BS_THREADS, 0, sa, e);
+        launch_k(k_bs_derive_p, g_cells, BS_THREADS, 0, sa, e);
     }
     {
         Timed tm(h, CCB_CAT_RESOLVE);
-        CCB_DISPATCH_DP(h->DP, { launch_k(pdl, k_bs_verify_p<kDP>, B / 32 + 1, BS_VP_THREADS, 0, sa, e); })
+        CCB_DISPATCH_DP(h->DP, { launch_k(k_bs_verify_p<kDP>, B / 32 + 1, BS_VP_THREADS, 0, sa, e); })
     }
     {
         Timed tm(h, CCB_CAT_OLIST);
-        launch_k(pdl, k_bs_olist, BS_OL_CTAS, BS_OL_THREADS, 0, s, e);
+        launch_k(k_bs_olist, BS_OL_CTAS, BS_OL_THREADS, 0, s, e);
     }
     {
         Timed tm(h, CCB_CAT_CHAIN_O);
-        CCB_DISPATCH_DP(h->DP, { launch_k(pdl, k_bs_chain_o<kDP>, 148 * 4, BS_THREADS, 0, s, e); }) // CTAs loop over the keys
+        CCB_DISPATCH_DP(h->DP, { launch_k(k_bs_chain_o<kDP>, 148 * 4, BS_THREADS, 0, s, e); }) // CTAs loop over the keys
     }
     {
         Timed tm(h, CCB_CAT_DERIVE);
-        launch_k(pdl, k_bs_derive_o, BS_RMAX / BS_THREADS, BS_THREADS, 0, s, e);
+        launch_k(k_bs_derive_o, BS_RMAX / BS_THREADS, BS_THREADS, 0, s, e);
     }
     if (side) {
         CK(h, cudaEventRecord(h->ev_join, side));
@@ -594,23 +655,22 @@ int launch_round(ccb_handle *h, const Eng &e, cudaStream_t s, int mp_grid, int m
     }
     {
         Timed tm(h, CCB_CAT_RESOLVE);
-        CCB_DISPATCH_DP(h->DP, { launch_k(pdl, k_bs_verify_o<kDP>, 148 * 4, BS_THREADS, 0, s, e); })
+        CCB_DISPATCH_DP(h->DP, { launch_k(k_bs_verify_o<kDP>, 148 * 4, BS_THREADS, 0, s, e); })
     }
     {
         Timed tm(h, CCB_CAT_DECIDE);
-        launch_k(pdl, k_bs_decide, 1, BS_CTA1, 0, s, e);
+        launch_k(k_bs_decide, 1, BS_CTA1, 0, s, e);
     }
     CKL(h);
     return CCB_OK;
 }
 constexpr int BS_LAUNCHES_PROLOGUE = 2, BS_LAUNCHES_ROUND = 14, BS_LAUNCHES_COMMIT = 1;
 
-int launch_commit(ccb_handle *h, const Eng &e, cudaStream_t s, int mp_grid, cudaStream_t side = nullptr) {
-    (void)side;
+int launch_commit(ccb_handle *h, const Eng &e, cudaStream_t s, int mp_grid) {
     const int g_cells = (h->bs_bmax + BS_THREADS - 1) / BS_THREADS;
     const int rows_ctas = (mp_grid + BS_RMAX + 3) / 4;
     Timed tm(h, CCB_CAT_COMMIT);
-    launch_k(h->pdl, k_bs_commit, rows_ctas + g_cells, BS_THREADS, 0, s, e, rows_ctas); // rows | cells | (last CTA) finish
+    launch_k(k_bs_commit, rows_ctas + g_cells, BS_THREADS, 0, s, e, rows_ctas); // rows | cells | (last CTA) finish
     CKL(h);
     return CCB_OK;
 }
@@ -620,39 +680,45 @@ Eng make_eng(ccb_handle *h) {
     e.P = h->P[h->pcur];
     e.O = h->O[h->ocur];
     e.ctl = h->d_ctl;
-    e.bc = h->d_bc;
+    e.bc = h->bs.bc;
     e.ws = h->ws;
     return e;
 }
 
 // ---- CUDA graph of the whole ordered loop: WHILE(block) { prologue; WHILE(round) { round }; commit } ----------
-void drop_graph(ccb_handle *h) { // (the current slot)
-    if (h->bs_exec) cudaGraphExecDestroy(h->bs_exec);
-    if (h->bs_graph) cudaGraphDestroy(h->bs_graph);
-    h->bs_exec = nullptr;
-    h->bs_graph = nullptr;
-}
-
+// Builds into the current slot, which changes only when the build succeeds.  A failed build ends the captures it opened.
 int build_graph(ccb_handle *h, const Eng &base) {
-    drop_graph(h);
-    if (!h->cap1) {
+    if (!h->cap[0]) {
         // the main line of a round (lists, replay, outlier-side lists ...) is the critical path: its kernels are captured
         // from high-priority streams, the side branches (kernel 1, pcore-side derive / verify) from a low-priority one, so
         // that a small critical kernel is not queued behind the thousand CTAs of a side kernel running next to it
         int prio_lo = 0, prio_hi = 0;
         CK(h, cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-        CK(h, cudaStreamCreateWithPriority(&h->cap1, cudaStreamNonBlocking, prio_hi));
-        CK(h, cudaStreamCreateWithPriority(&h->cap2, cudaStreamNonBlocking, prio_hi));
-        CK(h, cudaStreamCreateWithPriority(&h->cap3, cudaStreamNonBlocking, prio_lo));
-        CK(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-        CK(h, cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
+        Stream c[3];
+        Event fork, join;
+        CK(h, create(c[0], prio_hi));
+        CK(h, create(c[1], prio_hi));
+        CK(h, create(c[2], prio_lo));
+        CK(h, create(fork, cudaEventDisableTiming));
+        CK(h, create(join, cudaEventDisableTiming));
+        std::swap(h->cap, c);
+        h->ev_fork = std::move(fork);
+        h->ev_join = std::move(join);
     }
+    GraphSlot g;
+    struct Capture { // ends the capture of s if the build leaves it open
+        cudaStream_t s = nullptr;
+        ~Capture() {
+            cudaGraph_t body;
+            if (s && cudaStreamEndCapture(s, &body) != cudaSuccess) cudaGetLastError();
+        }
+    } c1, c2;
     Eng e = base;
-    e.io = h->d_io;
-    CK(h, cudaGraphCreate(&h->bs_graph, 0));
+    e.io = h->bs.io;
+    CK(h, make(g.graph, [](cudaGraph_t *q) { return cudaGraphCreate(q, 0); }));
     cudaGraphConditionalHandle ho, hi;
-    CK(h, cudaGraphConditionalHandleCreate(&ho, h->bs_graph, 1, cudaGraphCondAssignDefault));
-    CK(h, cudaGraphConditionalHandleCreate(&hi, h->bs_graph, 0, cudaGraphCondAssignDefault));
+    CK(h, cudaGraphConditionalHandleCreate(&ho, g.graph, 1, cudaGraphCondAssignDefault));
+    CK(h, cudaGraphConditionalHandleCreate(&hi, g.graph, 0, cudaGraphCondAssignDefault));
     e.h_outer = ho;
     e.h_inner = hi;
     cudaGraphNodeParams po = {};
@@ -661,18 +727,19 @@ int build_graph(ccb_handle *h, const Eng &base) {
     po.conditional.type = cudaGraphCondTypeWhile;
     po.conditional.size = 1;
     cudaGraphNode_t outer;
-    CK(h, cudaGraphAddNode(&outer, h->bs_graph, nullptr, 0, &po));
+    CK(h, cudaGraphAddNode(&outer, g.graph, nullptr, 0, &po));
     cudaGraph_t body_o = po.conditional.phGraph_out[0];
     const int mp_grid = e.P.cap, mo_bound = e.O.cap;
     int rc;
-    CK(h, cudaStreamBeginCaptureToGraph(h->cap1, body_o, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
-    if ((rc = launch_prologue(h, e, h->cap1))) return rc;
+    CK(h, cudaStreamBeginCaptureToGraph(h->cap[0], body_o, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+    c1.s = h->cap[0];
+    if ((rc = launch_prologue(h, e, h->cap[0]))) return rc;
     {
         cudaStreamCaptureStatus st;
         cudaGraph_t cg = nullptr;
         const cudaGraphNode_t *deps = nullptr;
         size_t ndeps = 0;
-        CK(h, cudaStreamGetCaptureInfo(h->cap1, &st, nullptr, &cg, &deps, &ndeps));
+        CK(h, cudaStreamGetCaptureInfo(h->cap[0], &st, nullptr, &cg, &deps, &ndeps));
         cudaGraphNodeParams pi = {};
         pi.type = cudaGraphNodeTypeConditional;
         pi.conditional.handle = hi;
@@ -680,16 +747,20 @@ int build_graph(ccb_handle *h, const Eng &base) {
         pi.conditional.size = 1;
         cudaGraphNode_t inner;
         CK(h, cudaGraphAddNode(&inner, cg, deps, ndeps, &pi));
-        CK(h, cudaStreamUpdateCaptureDependencies(h->cap1, &inner, 1, cudaStreamSetCaptureDependencies));
+        CK(h, cudaStreamUpdateCaptureDependencies(h->cap[0], &inner, 1, cudaStreamSetCaptureDependencies));
         cudaGraph_t body_i = pi.conditional.phGraph_out[0];
-        CK(h, cudaStreamBeginCaptureToGraph(h->cap2, body_i, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
-        if ((rc = launch_round(h, e, h->cap2, mp_grid, mo_bound, h->cap3))) return rc;
-        CK(h, cudaStreamEndCapture(h->cap2, nullptr));
+        CK(h, cudaStreamBeginCaptureToGraph(h->cap[1], body_i, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+        c2.s = h->cap[1];
+        if ((rc = launch_round(h, e, h->cap[1], mp_grid, mo_bound, h->cap[2]))) return rc;
+        c2.s = nullptr;
+        CK(h, cudaStreamEndCapture(h->cap[1], nullptr));
     }
-    if ((rc = launch_commit(h, e, h->cap1, mp_grid, h->cap3))) return rc;
-    CK(h, cudaStreamEndCapture(h->cap1, nullptr));
-    CK(h, cudaGraphInstantiate(&h->bs_exec, h->bs_graph, 0));
-    h->bs_graph_eng = base;
+    if ((rc = launch_commit(h, e, h->cap[0], mp_grid))) return rc;
+    c1.s = nullptr;
+    CK(h, cudaStreamEndCapture(h->cap[0], nullptr));
+    CK(h, make(g.exec, [&](cudaGraphExec_t *q) { return cudaGraphInstantiate(q, g.graph, 0); }));
+    g.eng = base;
+    h->graphs[0] = std::move(g);
     return CCB_OK;
 }
 
@@ -697,14 +768,9 @@ int ensure_bsv_capacity(ccb_handle *h, int blocks_ahead) {
     int rc;
     const Ctl &c = *h->h_ctl;
     const int64_t need_o = (int64_t)c.n_outlier + (int64_t)(blocks_ahead + 1) * BS_RMAX + 1;
-    if (need_o > h->O[h->ocur].cap) {
-        if ((rc = grow_store(h, h->O, h->ocur, c.n_outlier, need_o))) return rc;
-        if ((rc = realloc_aux_for_outlier_cap(h))) return rc;
-    }
-    if (c.n_pcore + blocks_ahead + 1 > h->P[h->pcur].cap) {
-        if ((rc = grow_store(h, h->P, h->pcur, c.n_pcore, c.n_pcore + blocks_ahead + 1))) return rc;
-        if ((rc = realloc_aux_for_pcore_cap(h))) return rc;
-    }
+    if ((rc = grow_store(h, true, c.n_outlier, need_o)) ||
+        (rc = grow_store(h, false, c.n_pcore, c.n_pcore + blocks_ahead + 1)))
+        return rc;
     return ensure_bs_ws(h);
 }
 
@@ -719,7 +785,7 @@ int ingest_core_bsv(ccb_handle *h, const double *dX, int64_t N, int64_t ld, int3
     const bool graph = h->bs_use_graph && !h->timing;
     const int bmax = h->bs_bmax, bmin = std::min(h->bs_bmin, h->bs_bmax);
     const int itmax = graph ? (h->prm.bsv_iters > 0 ? h->bs_iters : 8) : h->bs_iters;
-    k_bs_init<<<1, 1, 0, s>>>(h->d_bc, N, itmax, bmin, bmax);
+    k_bs_init<<<1, 1, 0, s>>>(h->bs.bc, N, itmax, bmin, bmax);
     CKL(h);
     h->st.kernel_launches++;
     if ((rc = sync_bc(h))) return rc;
@@ -742,12 +808,12 @@ int ingest_core_bsv(ccb_handle *h, const double *dX, int64_t N, int64_t ld, int3
     io.r2rej = HUGE_VAL;
     io.nm = make_num(h);
     if (graph) {
-        *h->h_io = io;
-        CK(h, cudaMemcpyAsync(h->d_io, h->h_io, sizeof(EngIo), cudaMemcpyHostToDevice, s));
+        *h->bs.h_io = io;
+        CK(h, cudaMemcpyAsync(h->bs.io, h->bs.h_io, sizeof(EngIo), cudaMemcpyHostToDevice, s));
     }
     int guard = 0;
-    while (!h->h_bc->done) {
-        const BsCtl &b = *h->h_bc;
+    while (!h->bs.h_bc->done) {
+        const BsCtl &b = *h->bs.h_bc;
         const int64_t left = N - b.pos;
         // blocks to enqueue before the next look at the control block (stream launches); the graph runs until the
         // input is consumed or a store is full, so give it room for a good stretch of blocks
@@ -755,33 +821,20 @@ int ingest_core_bsv(ccb_handle *h, const double *dX, int64_t N, int64_t ld, int3
         if (G < 1) G = 1;
         if ((rc = ensure_bsv_capacity(h, graph ? 32 : G))) return rc;
         if (b.need_grow) {
-            h->h_bc->need_grow = 0;
-            CK(h, cudaMemcpyAsync(&h->d_bc->need_grow, &h->h_bc->need_grow, sizeof(int32_t), cudaMemcpyHostToDevice, s));
+            h->bs.h_bc->need_grow = 0;
+            CK(h, cudaMemcpyAsync(&h->bs.bc->need_grow, &h->bs.h_bc->need_grow, sizeof(int32_t), cudaMemcpyHostToDevice, s));
         }
         Eng e = make_eng(h);
         const int64_t pos0 = b.pos;
         const int64_t blocks0 = b.blocks, iters0 = b.iters;
         if (graph) {
-            if (!h->bs_exec || memcmp(&h->bs_graph_eng, &e, sizeof(Eng)) != 0) {
+            GraphSlot *g = h->graphs;
+            if (!g[0].exec || memcmp(&g[0].eng, &e, sizeof(Eng)) != 0) {
                 // not the current slot: the other one? (swap); otherwise rebuild the older slot
-                std::swap(h->bs_graph, h->bs_graph_alt);
-                std::swap(h->bs_exec, h->bs_exec_alt);
-                std::swap(h->bs_graph_eng, h->bs_graph_eng_alt);
-                if (!h->bs_exec || memcmp(&h->bs_graph_eng, &e, sizeof(Eng)) != 0) {
-                    rc = build_graph(h, e);
-                    if (rc && h->pdl) { // a driver that cannot take programmatic edges here: the same graph without them
-                        cudaGraph_t junk = nullptr;
-                        cudaStreamEndCapture(h->cap2, &junk);
-                        cudaStreamEndCapture(h->cap1, &junk);
-                        cudaGetLastError();
-                        drop_graph(h);
-                        h->pdl = false;
-                        rc = build_graph(h, e);
-                    }
-                    if (rc) return rc;
-                }
+                std::swap(g[0], g[1]);
+                if ((!g[0].exec || memcmp(&g[0].eng, &e, sizeof(Eng)) != 0) && (rc = build_graph(h, e))) return rc;
             }
-            CK(h, cudaGraphLaunch(h->bs_exec, s));
+            CK(h, cudaGraphLaunch(g[0].exec, s));
         } else {
             const Ctl &c = *h->h_ctl;
             e.X = io.X, e.ld = io.ld, e.assign = io.assign, e.stage = io.stage, e.theta = io.theta, e.r2safe = io.r2safe, e.r2rej = io.r2rej, e.nm = io.nm;
@@ -802,11 +855,11 @@ int ingest_core_bsv(ccb_handle *h, const double *dX, int64_t N, int64_t ld, int3
         }
         if ((rc = sync_bc(h))) return rc;
         if (graph) // kernels the graph executed: per block prologue + commit, per round the round's kernels
-            h->st.kernel_launches += (h->h_bc->blocks - blocks0) * (BS_LAUNCHES_PROLOGUE + BS_LAUNCHES_COMMIT) +
-                                     (h->h_bc->iters - iters0) * BS_LAUNCHES_ROUND + BS_LAUNCHES_PROLOGUE;
-        if (h->h_bc->pos == pos0 && !h->h_bc->need_grow && !h->h_bc->done && ++guard > 4)
+            h->st.kernel_launches += (h->bs.h_bc->blocks - blocks0) * (BS_LAUNCHES_PROLOGUE + BS_LAUNCHES_COMMIT) +
+                                     (h->bs.h_bc->iters - iters0) * BS_LAUNCHES_ROUND + BS_LAUNCHES_PROLOGUE;
+        if (h->bs.h_bc->pos == pos0 && !h->bs.h_bc->need_grow && !h->bs.h_bc->done && ++guard > 4)
             return fail(h, CCB_ESTATE, "internal: block-speculative engine made no progress at row %lld", (long long)pos0);
-        if (h->h_bc->pos != pos0) guard = 0;
+        if (h->bs.h_bc->pos != pos0) guard = 0;
     }
     if (after_first_launch && (rc = (*after_first_launch)())) return rc;
     h->st.points += N;
@@ -822,17 +875,13 @@ double builtin_nrm2(const double *x, int n) {
 
 // grow-only buffer of the handle's offline workspace (contents are NOT preserved across a growth)
 int off_buf(ccb_handle *h, int which, size_t bytes) {
-    ccb_handle::OffBuf &b = h->ob[which];
+    Grow<Dev<void>> &b = h->ob[which];
     bytes = std::max<size_t>(bytes, 16);
-    if (bytes <= b.bytes) return CCB_OK;
+    if (bytes <= b.cap) return CCB_OK;
     CK(h, cudaStreamSynchronize(h->stream));
-    cudaFree(b.p);
-    b.p = nullptr;
-    b.bytes = 0;
     size_t cap = 256;
     while (cap < bytes) cap *= 2;
-    CK(h, cudaMalloc(&b.p, cap));
-    b.bytes = cap;
+    CK(h, b.ensure(cap));
     return CCB_OK;
 }
 
@@ -849,8 +898,7 @@ int launch_off_neighbours(ccb_handle *h, cudaStream_t s, const double *cen, int 
                           uint32_t *nbr, int32_t *cnt, int32_t *border, int border_cap, int32_t *n_border) {
     const int DP = round_dp(D);
     int ok = 0;
-    if (r1 > r0 && cudaMemsetAsync(cnt, 0, (size_t)(r1 - r0) * sizeof(int32_t), s) != cudaSuccess)
-        return fail(h, CCB_ECUDA, "k_off_neighbours: clearing the row counts failed");
+    if (r1 > r0) CK(h, cudaMemsetAsync(cnt, 0, (size_t)(r1 - r0) * sizeof(int32_t), s));
     CCB_DISPATCH_DP(DP, {
         // rows x column slabs: at least ~4 waves of CTAs on 148 SMs so that the tail does not dominate
         const int gx = (r1 - r0 + OffCfg<kDP>::ROWS - 1) / OffCfg<kDP>::ROWS;
@@ -884,60 +932,47 @@ int launch_off_neighbours(ccb_handle *h, cudaStream_t s, const double *cen, int 
 // centroids with upsilon = 0).  Synchronises s once, and once more when pairs exist.  *n_border = the number of pairs.
 int off_neighbours_settled(ccb_handle *h, cudaStream_t s, const double *cen, int M, int D, int r0, int r1, double E,
                            double E2, void *dnrm2, uint32_t *nbr, int32_t *cnt, int64_t *n_border) {
-    int32_t *buf = nullptr; // [0] pair count | [1, 1 + 2 cap) pairs (row, col) | cap bytes of decisions
     int32_t nb = 0;
-    int rc = CCB_OK;
-    auto done = [&](int r) {
-        cudaFreeAsync(buf, s);
-        return r;
-    };
+    int rc;
     for (int cap = 1 << 16;; cap = nb) {
-        cudaError_t e;
-        if ((e = cudaMallocAsync(&buf, 4 + (size_t)cap * 9, s)) != cudaSuccess)
-            return fail(h, CCB_ENOMEM, "borderline pairs (%d): %s", cap, cudaGetErrorString(e));
-        if (cudaMemsetAsync(buf, 0, 4, s) != cudaSuccess) return done(fail(h, CCB_ECUDA, "borderline count: clear failed"));
-        if ((rc = launch_off_neighbours(h, s, cen, M, D, r0, r1, E2, nbr, cnt, buf + 1, cap, buf))) return done(rc);
+        Scratch sc(s); // [0] pair count | [1, 1 + 2 cap) pairs (row, col) | cap bytes of decisions
+        CK(h, sc.alloc(4 + (size_t)cap * 9));
+        int32_t *buf = sc.as<int32_t>();
+        CK(h, cudaMemsetAsync(buf, 0, 4, s));
+        if ((rc = launch_off_neighbours(h, s, cen, M, D, r0, r1, E2, nbr, cnt, buf + 1, cap, buf))) return rc;
         if (h) h->st.kernel_launches++;
-        if ((e = cudaMemcpyAsync(&nb, buf, 4, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
-            (e = cudaStreamSynchronize(s)) != cudaSuccess)
-            return done(fail(h, CCB_ECUDA, "borderline count: %s", cudaGetErrorString(e)));
-        if (nb <= cap) break;
-        cudaFreeAsync(buf, s);
+        CK(h, cudaMemcpyAsync(&nb, buf, 4, cudaMemcpyDeviceToHost, s));
+        CK(h, cudaStreamSynchronize(s));
+        if (nb > cap) continue; // again with a list that holds every pair
+        *n_border = nb;
+        if (nb == 0) return CCB_OK;
+        std::vector<int32_t> pairs(2 * (size_t)nb);
+        std::vector<double> hc((size_t)M * D), x(D);
+        std::vector<uint8_t> dec(nb);
+        CK(h, cudaMemcpy(pairs.data(), buf + 1, pairs.size() * 4, cudaMemcpyDeviceToHost));
+        CK(h, cudaMemcpy(hc.data(), cen, hc.size() * 8, cudaMemcpyDeviceToHost));
+        typedef double (*nrm2_fn)(int *, double *, int *);
+        for (int i = 0; i < nb; ++i) {
+            const int p_ = pairs[2 * i], q_ = pairs[2 * i + 1];
+            for (int d = 0; d < D; ++d) x[d] = hc[(size_t)q_ * D + d] - hc[(size_t)p_ * D + d];
+            int n = D, inc = 1;
+            const double r = dnrm2 ? ((nrm2_fn)dnrm2)(&n, x.data(), &inc) : builtin_nrm2(x.data(), D);
+            dec[i] = r <= E;
+        }
+        uint8_t *ddec = reinterpret_cast<uint8_t *>(buf + 1 + 2 * (size_t)nb);
+        CK(h, cudaMemcpyAsync(ddec, dec.data(), nb, cudaMemcpyHostToDevice, s));
+        k_off_patch<<<(nb + 127) / 128, 128, 0, s>>>(nbr, cnt, buf + 1, ddec, nb, r0, (M + 31) / 32);
+        if ((rc = launched(h, "k_off_patch"))) return rc;
+        if (h) h->st.kernel_launches++;
+        CK(h, cudaStreamSynchronize(s)); // dec (host) is read by the copy above
+        return CCB_OK;
     }
-    *n_border = nb;
-    if (nb == 0) return done(CCB_OK);
-    std::vector<int32_t> pairs(2 * (size_t)nb);
-    std::vector<double> hc((size_t)M * D), x(D);
-    std::vector<uint8_t> dec(nb);
-    cudaError_t e;
-    if ((e = cudaMemcpy(pairs.data(), buf + 1, pairs.size() * 4, cudaMemcpyDeviceToHost)) != cudaSuccess ||
-        (e = cudaMemcpy(hc.data(), cen, hc.size() * 8, cudaMemcpyDeviceToHost)) != cudaSuccess)
-        return done(fail(h, CCB_ECUDA, "borderline pairs: %s", cudaGetErrorString(e)));
-    typedef double (*nrm2_fn)(int *, double *, int *);
-    for (int i = 0; i < nb; ++i) {
-        const int p_ = pairs[2 * i], q_ = pairs[2 * i + 1];
-        for (int d = 0; d < D; ++d) x[d] = hc[(size_t)q_ * D + d] - hc[(size_t)p_ * D + d];
-        int n = D, inc = 1;
-        const double r = dnrm2 ? ((nrm2_fn)dnrm2)(&n, x.data(), &inc) : builtin_nrm2(x.data(), D);
-        dec[i] = r <= E;
-    }
-    uint8_t *ddec = reinterpret_cast<uint8_t *>(buf + 1 + 2 * (size_t)nb);
-    if ((e = cudaMemcpyAsync(ddec, dec.data(), nb, cudaMemcpyHostToDevice, s)) != cudaSuccess)
-        return done(fail(h, CCB_ECUDA, "borderline decisions: %s", cudaGetErrorString(e)));
-    k_off_patch<<<(nb + 127) / 128, 128, 0, s>>>(nbr, cnt, buf + 1, ddec, nb, r0, (M + 31) / 32);
-    if ((rc = launched(h, "k_off_patch"))) return done(rc);
-    if (h) h->st.kernel_launches++;
-    cudaFreeAsync(buf, s);
-    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) // dec (host) is read by the copy above
-        return fail(h, CCB_ECUDA, "k_off_patch: %s", cudaGetErrorString(e));
-    return CCB_OK;
 }
 
 int launch_off_subspace(ccb_handle *h, cudaStream_t s, const double *cen, int M, int D, int r0, int r1, const uint32_t *nbr,
                         const int32_t *cnt, double delta, uint64_t *submask) {
     if (r1 == r0) return CCB_OK;
-    if (cudaMemsetAsync(submask, 0, (size_t)(r1 - r0) * 8, s) != cudaSuccess)
-        return fail(h, CCB_ECUDA, "k_off_subspace: clearing the masks failed");
+    CK(h, cudaMemsetAsync(submask, 0, (size_t)(r1 - r0) * 8, s));
     const int64_t t = (int64_t)(r1 - r0) * D;
     k_off_subspace<<<(unsigned)((t + 127) / 128), 128, 0, s>>>(cen, M, D, r0, r1, nbr, cnt, delta, submask);
     return launched(h, "k_off_subspace");
@@ -974,6 +1009,13 @@ void tune_pool(int device) {
         cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
     }
     done[device] = true;
+}
+
+// first call of every stateless entry point
+int enter_device(int device) {
+    CK(nullptr, cudaSetDevice(device));
+    tune_pool(device);
+    return CCB_OK;
 }
 
 // kernel 4e: ordered cluster growth.  Small M (the online hot path: tens of pcore MCs): the single-launch bit-row
@@ -1024,10 +1066,8 @@ void offc_grow_and_merge(cudaStream_t s, int M, const int64_t *off, const int32_
 
 // off[M] -- the CSR size, the last entry of the exclusive prefix of the row lengths -- read back to the host
 int csr_total(ccb_handle *h, cudaStream_t s, const int64_t *off, int M, int64_t *total) {
-    cudaError_t e;
-    if ((e = cudaMemcpyAsync(total, off + M, 8, cudaMemcpyDeviceToHost, s)) != cudaSuccess ||
-        (e = cudaStreamSynchronize(s)) != cudaSuccess)
-        return fail(h, CCB_ECUDA, "offline CSR size: %s", cudaGetErrorString(e));
+    CK(h, cudaMemcpyAsync(total, off + M, 8, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
     return CCB_OK;
 }
 
@@ -1037,17 +1077,13 @@ int off_clusters_csr(ccb_handle *h, cudaStream_t s, int M, const int64_t *off, c
                      int32_t *label, int32_t *order, int32_t *cl_off, int32_t *n_cl) {
     // int32 scratch of offc_grow_and_merge (7 M + 16) | queue (2 M + 2) | cls (M bytes)
     const size_t m = (size_t)M;
-    int32_t *i32 = nullptr;
-    cudaError_t e;
-    if ((e = cudaMallocAsync(&i32, (9 * m + 18) * 4 + m, s)) != cudaSuccess)
-        return fail(h, CCB_ENOMEM, "offline scratch: %s", cudaGetErrorString(e));
-    int32_t *queue = i32 + 7 * m + 16;
+    Scratch sc(s);
+    CK(h, sc.alloc((9 * m + 18) * 4 + m));
+    int32_t *i32 = sc.as<int32_t>(), *queue = i32 + 7 * m + 16;
     uint8_t *cls = reinterpret_cast<uint8_t *>(queue + 2 * m + 2);
     cudaMemsetAsync(cls, 0, m, s);
     offc_grow_and_merge(s, M, off, col, core, iso, submask, cnt_gt1, pi, cls, queue, i32, label, order, cl_off, n_cl, total);
-    const int rc = launched(h, "offline cluster growth");
-    cudaFreeAsync(i32, s);
-    return rc;
+    return launched(h, "offline cluster growth");
 }
 
 // cls [M] and queue [2 M + 2]: scratch of the bit-row scan
@@ -1064,33 +1100,26 @@ int launch_off_clusters(ccb_handle *h, cudaStream_t s, int M, const uint32_t *wn
     if (M < (csr_min_m > 0 ? csr_min_m : OFF_CSR_MIN_M) || M == 0) return bit_rows();
     // off (M + 1) | nnz (M int32) | iso (M bytes)
     const size_t m = (size_t)M;
-    int64_t *off = nullptr;
-    int32_t *col = nullptr;
-    cudaError_t e;
-    if ((e = cudaMallocAsync(&off, (m + 1) * 8 + m * 5, s)) != cudaSuccess)
-        return fail(h, CCB_ENOMEM, "offline scratch: %s", cudaGetErrorString(e));
+    Scratch sc(s), sc_col(s);
+    CK(h, sc.alloc((m + 1) * 8 + m * 5));
+    int64_t *off = sc.as<int64_t>();
     int32_t *nnz = reinterpret_cast<int32_t *>(off + m + 1);
     uint8_t *iso = reinterpret_cast<uint8_t *>(nnz + m);
-    auto done = [&](int r) {
-        cudaFreeAsync(off, s);
-        if (col) cudaFreeAsync(col, s);
-        return r;
-    };
     int rc;
     int64_t total = 0;
-    if ((rc = launch_offc_rowinfo(h, s, wnbr, M, 0, M, iso, nnz))) return done(rc);
+    if ((rc = launch_offc_rowinfo(h, s, wnbr, M, 0, M, iso, nnz))) return rc;
     k_offc_scan<int64_t><<<1, OFFG_THREADS, 0, s>>>(nnz, M, off);
     *launches += 2;
-    if ((rc = csr_total(h, s, off, M, &total))) return done(rc);
+    if ((rc = csr_total(h, s, off, M, &total))) return rc;
     if (total > (int64_t)INT32_MAX - 1) // a CSR that large buys nothing over the bit rows
-        return done(bit_rows());
-    if ((e = cudaMallocAsync(&col, (size_t)std::max<int64_t>(total, 1) * 4, s)) != cudaSuccess)
-        return done(fail(h, CCB_ENOMEM, "offline CSR (%lld entries): %s", (long long)total, cudaGetErrorString(e)));
-    if ((rc = launch_offc_fill(h, s, wnbr, M, 0, M, iso, off, col))) return done(rc);
+        return bit_rows();
+    CK(h, sc_col.alloc((size_t)std::max<int64_t>(total, 1) * 4));
+    int32_t *col = sc_col.as<int32_t>();
+    if ((rc = launch_offc_fill(h, s, wnbr, M, 0, M, iso, off, col))) return rc;
     *launches += 1;
     rc = off_clusters_csr(h, s, M, off, col, total, iso, core, submask, cnt_gt1, pi, label, order, cl_off, n_cl);
     *launches += 8;
-    return done(rc);
+    return rc;
 }
 
 // Probes of the pcore replay pattern (mode 3 of ccb_fp64_peak): one warp runs the CLEAN-stage schedule of k_bs_chain_p over
@@ -1184,7 +1213,7 @@ int ccb_create(const ccb_params *p, ccb_handle **out) {
         return fail(nullptr, CCB_ECUDA, "no CUDA device (%s); this library has no CPU path",
                     e == cudaSuccess ? "device count 0" : cudaGetErrorString(e));
     if (p->device < 0 || p->device >= ndev) return fail(nullptr, CCB_EINVAL, "device %d of %d", p->device, ndev);
-    ccb_handle *h = new (std::nothrow) ccb_handle();
+    std::unique_ptr<ccb_handle> h(new (std::nothrow) ccb_handle());
     if (!h) return fail(nullptr, CCB_ENOMEM, "host allocation failed");
     h->prm = *p;
     h->D = p->D;
@@ -1199,34 +1228,19 @@ int ccb_create(const ccb_params *p, ccb_handle **out) {
     h->div_mode = p2 ? 0 : 1;
     h->wsel = p2 ? 1.0 / p->k : p->k; // exact reciprocal of a power of two, else the divisor itself
     h->cnt_gt1 = p->k > 1.0;
-#define CKC(call)                                                                            \
-    do {                                                                                     \
-        cudaError_t e_ = (call);                                                             \
-        if (e_ != cudaSuccess) {                                                             \
-            int rc_ = fail(nullptr, CCB_ECUDA, "%s: %s", #call, cudaGetErrorString(e_));     \
-            ccb_destroy(h);                                                                  \
-            return rc_;                                                                      \
-        }                                                                                    \
-    } while (0)
-    CKC(cudaSetDevice(p->device));
-    tune_pool(p->device);
-    CKC(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-    CKC(cudaMalloc(&h->d_ctl, sizeof(Ctl)));
-    CKC(cudaMemset(h->d_ctl, 0, sizeof(Ctl)));
-    CKC(cudaMallocHost(&h->h_ctl, sizeof(Ctl)));
+    int rc;
+    if ((rc = enter_device(p->device))) return rc;
+    CK(nullptr, create(h->stream, 0));
+    CK(nullptr, alloc(h->d_ctl, sizeof(Ctl)));
+    CK(nullptr, cudaMemset(h->d_ctl, 0, sizeof(Ctl)));
+    CK(nullptr, alloc(h->h_ctl, sizeof(Ctl)));
     memset(h->h_ctl, 0, sizeof(Ctl));
-    int rc = 0;
-    for (int i = 0; i < 2 && !rc; ++i) rc = alloc_store(h, h->P[i], 256);
-    for (int i = 0; i < 2 && !rc; ++i) rc = alloc_store(h, h->O[i], 8192);
-    if (!rc) rc = realloc_aux_for_outlier_cap(h);
-    if (!rc) rc = realloc_aux_for_pcore_cap(h);
-    if (rc) {
-        g_err = h->err;
-        ccb_destroy(h);
-        return rc;
+    for (int i = 0; i < 2; ++i) {
+        if ((rc = alloc_store(h.get(), h->Pm[i], 256)) || (rc = alloc_store(h.get(), h->Om[i], 8192))) return rc;
+        h->P[i] = h->Pm[i].view();
+        h->O[i] = h->Om[i].view();
     }
-#undef CKC
-    *out = h;
+    *out = h.release();
     return CCB_OK;
 }
 
@@ -1234,48 +1248,6 @@ void ccb_destroy(ccb_handle *h) {
     if (!h) return;
     cudaSetDevice(h->prm.device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    for (int i = 0; i < 2; ++i) {
-        free_store(h->P[i]);
-        free_store(h->O[i]);
-    }
-    cudaFree(h->d_ctl);
-    if (h->h_ctl) cudaFreeHost(h->h_ctl);
-    cudaFree(h->d_X);
-    cudaFree(h->d_assign);
-    cudaFree(h->d_stage);
-    cudaFree(h->d_pnew);
-    cudaFree(h->d_pfin);
-    cudaFree(h->d_onew);
-    drop_graph(h);
-    std::swap(h->bs_graph, h->bs_graph_alt);
-    std::swap(h->bs_exec, h->bs_exec_alt);
-    drop_graph(h);
-    if (h->cap1) cudaStreamDestroy(h->cap1);
-    if (h->cap2) cudaStreamDestroy(h->cap2);
-    if (h->cap3) cudaStreamDestroy(h->cap3);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    if (h->res_stream) cudaStreamDestroy(h->res_stream);
-    if (h->h_res) cudaFreeHost(h->h_res);
-    cudaFree(h->d_scale);
-    for (auto &ev : h->ev_seg)
-        if (ev) cudaEventDestroy(ev);
-    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    if (h->ev_join) cudaEventDestroy(h->ev_join);
-    cudaFree(h->d_io);
-    if (h->h_io) cudaFreeHost(h->h_io);
-    cudaFree(h->d_bc);
-    if (h->h_bc) cudaFreeHost(h->h_bc);
-    for (void *q : h->ws_allocs) cudaFree(q);
-    for (void *q : h->ws_tiles) cudaFree(q);
-    cudaFree(h->ws.dbg);
-    cudaFree(h->ws_first);
-    for (auto &b : h->ob) cudaFree(b.p);
-    for (auto &e : h->ev_pending) {
-        cudaEventDestroy(e.a);
-        cudaEventDestroy(e.b);
-    }
-    for (auto &e : h->ev_pool) cudaEventDestroy(e);
-    if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
 }
 
@@ -1288,8 +1260,8 @@ int ccb_get_stats(const ccb_handle *h, ccb_stats *out) {
     out->created = h->st_base.created + c.created;
     out->downgraded = h->st_base.downgraded + c.downgraded;
     out->deleted = h->st_base.deleted + c.deleted;
-    if (h->h_bc) {
-        const BsCtl &b = *h->h_bc, &bb = h->bc_base;
+    if (h->bs.h_bc) {
+        const BsCtl &b = *h->bs.h_bc, &bb = h->bc_base;
         out->bsv_blocks = bb.blocks + b.blocks;
         out->bsv_rounds = bb.iters + b.iters;
         out->bsv_mismatches = bb.mismatches + b.mismatches;
@@ -1303,7 +1275,6 @@ int ccb_get_stats(const ccb_handle *h, ccb_stats *out) {
         out->bsv_serial_cells = bb.serial_cells + b.serial_cells;
         out->nearest_pairs += bb.pairs + b.pairs;
     }
-    out->bsv_pdl = (h->bs_use_graph && h->pdl && (h->bs_exec || h->bs_exec_alt)) ? 1 : 0;
     return CCB_OK;
 }
 
@@ -1342,11 +1313,15 @@ int ccb_debug_counters(ccb_handle *h, int64_t *out16, int32_t reset) {
 
 int ccb_debug_chain(ccb_handle *h, int64_t *out, int32_t max_keys) {
     if (!h || !out) return fail(h, CCB_EINVAL, "null argument");
-    if (!h->ws.dbg) { // first call switches the counters on
+    if (!h->ws_dbg) { // first call switches the counters on
         if (h->ws.mp_stride <= 0) return fail(h, CCB_ESTATE, "no block-speculative workspace yet");
         CK(h, cudaStreamSynchronize(h->stream));
-        CK(h, cudaMalloc(&h->ws.dbg, (size_t)h->ws.mp_stride * 8 * sizeof(int64_t)));
-        CK(h, cudaMemset(h->ws.dbg, 0, (size_t)h->ws.mp_stride * 8 * sizeof(int64_t)));
+        const size_t bytes = (size_t)h->ws.mp_stride * 8 * sizeof(int64_t);
+        Dev<int64_t> dbg;
+        CK(h, alloc(dbg, bytes));
+        CK(h, cudaMemset(dbg, 0, bytes));
+        h->ws_dbg = std::move(dbg);
+        h->ws.dbg = h->ws_dbg;
         memset(out, 0, (size_t)max_keys * 8 * sizeof(int64_t));
         return CCB_OK;
     }
@@ -1358,10 +1333,8 @@ int ccb_debug_chain(ccb_handle *h, int64_t *out, int32_t max_keys) {
 #endif
 
 int ccb_reset(ccb_handle *h) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
-    CK(h, cudaSetDevice(h->prm.device));
-    int rc = sync_ctl(h);
-    if (rc) return rc;
+    int rc;
+    if ((rc = enter(h)) || (rc = sync_ctl(h))) return rc;
     {
         const Ctl &c = *h->h_ctl;
         h->st_base.upgrades += c.upgrades;
@@ -1372,18 +1345,18 @@ int ccb_reset(ccb_handle *h) {
     memset(h->h_ctl, 0, sizeof(Ctl));
     rc = push_ctl(h);
     if (rc) return rc;
-    if (h->d_bc) {
-        CK(h, cudaMemcpyAsync(h->h_bc, h->d_bc, sizeof(BsCtl), cudaMemcpyDeviceToHost, h->stream));
+    if (h->bs.bc) {
+        CK(h, cudaMemcpyAsync(h->bs.h_bc, h->bs.bc, sizeof(BsCtl), cudaMemcpyDeviceToHost, h->stream));
         CK(h, cudaStreamSynchronize(h->stream));
-        const BsCtl &b = *h->h_bc;
+        const BsCtl &b = *h->bs.h_bc;
         BsCtl &bb = h->bc_base;
         bb.blocks += b.blocks, bb.iters += b.iters, bb.mismatches += b.mismatches, bb.cuts_unknown += b.cuts_unknown;
         bb.cuts_iter += b.cuts_iter, bb.cuts_cap += b.cuts_cap, bb.tk_late += b.tk_late, bb.rejects += b.rejects;
         bb.replayed += b.replayed, bb.pairs += b.pairs, bb.rounds_light += b.rounds_light, bb.serial_cells += b.serial_cells;
         const int32_t keep_B = b.next_B;
-        memset(h->h_bc, 0, sizeof(BsCtl));
-        h->h_bc->next_B = keep_B;
-        CK(h, cudaMemcpyAsync(h->d_bc, h->h_bc, sizeof(BsCtl), cudaMemcpyHostToDevice, h->stream));
+        memset(h->bs.h_bc, 0, sizeof(BsCtl));
+        h->bs.h_bc->next_B = keep_B;
+        CK(h, cudaMemcpyAsync(h->bs.bc, h->bs.h_bc, sizeof(BsCtl), cudaMemcpyHostToDevice, h->stream));
     }
     CK(h, cudaStreamSynchronize(h->stream));
     h->have_params = false;
@@ -1401,8 +1374,7 @@ int ccb_enable_timing(ccb_handle *h, int32_t on) {
 }
 
 int ccb_get_timing(ccb_handle *h, double ms[CCB_NCAT], int64_t launches[CCB_NCAT], int32_t reset) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
-    CK(h, cudaSetDevice(h->prm.device));
+    if (int rc = enter(h)) return rc;
     CK(h, cudaStreamSynchronize(h->stream));
     drain_timing(h);
     for (int i = 0; i < CCB_NCAT; ++i) {
@@ -1423,14 +1395,22 @@ int ccb_set_dnrm2(ccb_handle *h, void *fn) {
 }
 
 int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, int32_t decay, double decay_factor) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
-    CK(h, cudaSetDevice(h->prm.device));
+    int rc;
+    if ((rc = enter(h))) return rc;
     h->mu = mu;
     h->omicron = omicron;
     h->pi = pi;
     h->have_params = true;
     if (!decay) return CCB_OK;
     cudaStream_t s = h->stream;
+    if ((rc = sync_ctl(h))) return rc;
+    // every downgraded pcore MC lands in the outlier list: make room first
+    const int64_t need_o = (int64_t)h->h_ctl->n_outlier + h->h_ctl->n_pcore;
+    if ((rc = grow_store(h, true, h->h_ctl->n_outlier, need_o))) return rc;
+    // kernel 3's plan codes: one per entry of either list
+    CK(h, h->d_pnew.ensure((size_t)h->P[h->pcur].cap * 4));
+    CK(h, h->d_pfin.ensure((size_t)h->P[h->pcur].cap * 4));
+    CK(h, h->d_onew.ensure((size_t)h->O[h->ocur].cap * 4));
     MaintArgs ma{};
     ma.P = h->P[h->pcur];
     ma.O = h->O[h->ocur];
@@ -1448,17 +1428,6 @@ int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, in
     ma.DP = h->DP;
     ma.cnt_gt1 = h->cnt_gt1;
     ma.wsel = h->wsel;
-    int rc;
-    if ((rc = sync_ctl(h))) return rc;
-    // every downgraded pcore MC lands in the outlier list: make room first
-    const int64_t need_o = (int64_t)h->h_ctl->n_outlier + h->h_ctl->n_pcore;
-    if (need_o > h->O[h->ocur].cap) {
-        if ((rc = grow_store(h, h->O, h->ocur, h->h_ctl->n_outlier, need_o))) return rc;
-        if ((rc = realloc_aux_for_outlier_cap(h))) return rc;
-        ma.O = h->O[h->ocur];
-        ma.O2 = h->O[1 - h->ocur];
-        ma.o_new = h->d_onew;
-    }
     Timed tm(h, CCB_CAT_MAINT);
     k_maint_plan<<<1, MAINT_THREADS, 0, s>>>(ma);
     CKL(h);
@@ -1477,9 +1446,8 @@ int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, in
 
 int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
                       uint8_t *stage_dev) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
+    if (int rc = enter(h)) return rc;
     if (N < 0 || ld < h->D || (!X_dev && N > 0) || (!assign_uid_dev && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
-    CK(h, cudaSetDevice(h->prm.device));
     return ingest_core_bsv(h, X_dev, N, ld, assign_uid_dev, stage_dev);
 }
 
@@ -1500,21 +1468,16 @@ int ccb_ingest_scaled(ccb_handle *h, const double *X_raw, int64_t N, int64_t ld,
 // (X * scale + shift, two roundings: sklearn MinMaxScaler.transform), segment by segment behind their copies
 static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, int32_t *assign_uid, uint8_t *stage,
                        const double *scale, const double *shift) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
+    int rc;
+    if ((rc = enter(h))) return rc;
     if (N < 0 || ld < h->D || (!X && N > 0) || (!assign_uid && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
     if (N == 0) return CCB_OK;
-    CK(h, cudaSetDevice(h->prm.device));
     const size_t need = (size_t)N * ld;
-    if (need > h->x_cap) {
-        cudaFree(h->d_X);
-        h->x_cap = 0;
-        CK(h, cudaMalloc(&h->d_X, (need + 2) * 8));
-        h->x_cap = need;
-    }
-    int rc = ensure_point_buffers(h, N);
-    if (rc) return rc;
+    CK(h, h->d_X.ensure((need + 2) * 8));
+    CK(h, h->d_assign.ensure((size_t)N * 4));
+    CK(h, h->d_stage.ensure((size_t)N));
     if (scale) {
-        if (!h->d_scale) CK(h, cudaMalloc(&h->d_scale, 2 * CCB_MAX_D * sizeof(double)));
+        CK(h, h->d_scale.ensure(2 * CCB_MAX_D * sizeof(double)));
         CK(h, cudaMemcpyAsync(h->d_scale, scale, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
         CK(h, cudaMemcpyAsync(h->d_scale + CCB_MAX_D, shift, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
     }
@@ -1559,8 +1522,14 @@ static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, in
         // engine starts as soon as the first one has landed: segment k + 1 is queued right after the engine has been
         // launched on segment k (with pageable host memory the staging copy then overlaps the engine, too).
         if (!h->copy_stream) {
-            CK(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-            for (auto &ev : h->ev_seg) CK(h, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+            Stream cs, rs;
+            Event ev[8];
+            CK(h, create(cs, 0));
+            CK(h, create(rs, 0));
+            for (Event &e : ev) CK(h, create(e, cudaEventDisableTiming));
+            h->copy_stream = std::move(cs);
+            h->res_stream = std::move(rs);
+            std::swap(h->ev_seg, ev);
         }
         CK(h, cudaEventRecord(h->ev_seg[0], h->stream)); // earlier work on the handle's stream (previous readers of d_X)
         CK(h, cudaStreamWaitEvent(h->copy_stream, h->ev_seg[0], 0));
@@ -1576,15 +1545,8 @@ static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, in
             CK(h, cudaEventRecord(h->ev_seg[k], h->copy_stream));
             return CCB_OK;
         };
-        if (!h->res_stream) CK(h, cudaStreamCreateWithFlags(&h->res_stream, cudaStreamNonBlocking));
-        if ((size_t)N > h->res_cap) {
-            if (h->h_res) cudaFreeHost(h->h_res);
-            h->h_res = nullptr;
-            h->res_cap = 0;
-            CK(h, cudaHostAlloc((void **)&h->h_res, (size_t)N * 5, cudaHostAllocDefault));
-            h->res_cap = (size_t)N;
-        }
-        int32_t *ba = reinterpret_cast<int32_t *>(h->h_res);
+        CK(h, h->h_res.ensure((size_t)N * 5));
+        int32_t *ba = reinterpret_cast<int32_t *>(h->h_res.p);
         uint8_t *bs = h->h_res + (size_t)N * 4;
         // results of segment k (its engine run is complete: ingest_core_bsv returns after a synchronisation) -> caller
         auto results_seg = [&](int k) -> int {
@@ -1626,10 +1588,10 @@ static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, in
 }
 
 int ccb_counts(ccb_handle *h, int64_t out[4]) {
-    if (!h || !out) return fail(nullptr, CCB_EINVAL, "null argument");
-    CK(h, cudaSetDevice(h->prm.device));
-    int rc = sync_ctl(h);
-    if (rc) return rc;
+    int rc;
+    if ((rc = enter(h))) return rc;
+    if (!out) return fail(h, CCB_EINVAL, "null argument");
+    if ((rc = sync_ctl(h))) return rc;
     out[0] = h->h_ctl->n_pcore;
     out[1] = h->h_ctl->n_outlier_alive;
     out[2] = h->h_ctl->pcore_last_id;
@@ -1639,10 +1601,8 @@ int ccb_counts(ccb_handle *h, int64_t out[4]) {
 
 int ccb_export_list(ccb_handle *h, int32_t which, int64_t *ids, int64_t *uids, double *w, double *cf1, double *cf2,
                     double *cen, double *pref) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
-    CK(h, cudaSetDevice(h->prm.device));
-    int rc = sync_ctl(h);
-    if (rc) return rc;
+    int rc;
+    if ((rc = enter(h)) || (rc = sync_ctl(h))) return rc;
     const Store &S = which ? h->O[h->ocur] : h->P[h->pcur];
     const int n = which ? h->h_ctl->n_outlier : h->h_ctl->n_pcore;
     const int D = h->D;
@@ -1677,18 +1637,11 @@ int ccb_export_list(ccb_handle *h, int32_t which, int64_t *ids, int64_t *uids, d
 
 int ccb_import_list(ccb_handle *h, int32_t which, int64_t n, const int64_t *ids, const int64_t *uids, const double *w,
                     const double *cf1, const double *cf2, const double *cen, const double *pref) {
-    if (!h || n < 0) return fail(nullptr, CCB_EINVAL, "bad argument");
-    CK(h, cudaSetDevice(h->prm.device));
-    int rc = sync_ctl(h);
-    if (rc) return rc;
+    int rc;
+    if ((rc = enter(h))) return rc;
+    if (n < 0) return fail(h, CCB_EINVAL, "bad argument");
+    if ((rc = sync_ctl(h)) || (rc = grow_store(h, which != 0, 0, std::max<int64_t>(n, 1)))) return rc;
     const int D = h->D;
-    if (which) {
-        if ((rc = grow_store(h, h->O, h->ocur, 0, std::max<int64_t>(n, 1)))) return rc;
-        if ((rc = realloc_aux_for_outlier_cap(h))) return rc;
-    } else {
-        if ((rc = grow_store(h, h->P, h->pcur, 0, std::max<int64_t>(n, 1)))) return rc;
-        if ((rc = realloc_aux_for_pcore_cap(h))) return rc;
-    }
     Store &S = which ? h->O[h->ocur] : h->P[h->pcur];
     std::vector<uint64_t> hm(n);
     std::vector<int32_t> hu(n);
@@ -1724,10 +1677,8 @@ int ccb_import_list(ccb_handle *h, int32_t which, int64_t n, const int64_t *ids,
 }
 
 int ccb_set_counters(ccb_handle *h, int64_t pcore_last_id, int64_t outlier_last_id) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
-    CK(h, cudaSetDevice(h->prm.device));
-    int rc = sync_ctl(h);
-    if (rc) return rc;
+    int rc;
+    if ((rc = enter(h)) || (rc = sync_ctl(h))) return rc;
     h->h_ctl->pcore_last_id = pcore_last_id;
     h->h_ctl->outlier_last_id = outlier_last_id;
     if ((rc = push_ctl(h))) return rc;
@@ -1737,11 +1688,10 @@ int ccb_set_counters(ccb_handle *h, int64_t pcore_last_id, int64_t outlier_last_
 
 // ---- offline ------------------------------------------------------------------------------------------
 int ccb_offline(ccb_handle *h, int64_t *n_clusters) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
+    int rc;
+    if ((rc = enter(h))) return rc;
     if (!h->have_params) return fail(h, CCB_ESTATE, "ccb_begin_timepoint must precede ccb_offline");
-    CK(h, cudaSetDevice(h->prm.device));
-    int rc = sync_ctl(h);
-    if (rc) return rc;
+    if ((rc = sync_ctl(h))) return rc;
     cudaStream_t s = h->stream;
     const int M = h->h_ctl->n_pcore, D = h->D;
     const Store &P = h->P[h->pcur];
@@ -1872,10 +1822,9 @@ int ccb_export_clusters(ccb_handle *h, int64_t *off, int64_t *members, double *w
 }
 
 int ccb_export_offline(ccb_handle *h, uint8_t *core, uint8_t *nbr, uint8_t *wnbr, double *subw) {
-    if (!h) return fail(nullptr, CCB_EINVAL, "null handle");
+    if (int rc = enter(h)) return rc;
     const int64_t M = h->off_M;
     if (M == 0) return CCB_OK;
-    CK(h, cudaSetDevice(h->prm.device));
     // read back from the offline workspace of the last ccb_offline (kept on the device until the next one)
     const int D = h->D, words = (int)((M + 31) / 32);
     std::vector<uint8_t> hcore(M);
@@ -1976,25 +1925,19 @@ __global__ void k_fp64_latency(double *sink) {
 
 int ccb_fp64_peak(int32_t device, void *stream, int32_t mode, int32_t iters, int32_t blocks, double *sink,
                   double *flops_out) {
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     if (mode == 3) { // probes of the replay pattern: sink[8..11] = cycles per cell (see k_chain_probe)
         k_chain_probe<<<1, 96, 0, (cudaStream_t)stream>>>(sink);
-        e = cudaGetLastError();
-        if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "k_chain_probe: %s", cudaGetErrorString(e));
         if (flops_out) *flops_out = 0.0;
-        return CCB_OK;
+        return launched(nullptr, "k_chain_probe");
     }
     if (mode == 2) { // latency probes: sink[1..5] = cycles per dependent DADD, DMUL, DFMA, replay step, FADD
         k_fp64_latency<<<1, 32, 0, (cudaStream_t)stream>>>(sink);
-        e = cudaGetLastError();
-        if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "k_fp64_latency: %s", cudaGetErrorString(e));
         if (flops_out) *flops_out = 0.0;
-        return CCB_OK;
+        return launched(nullptr, "k_fp64_latency");
     }
     k_fp64_peak<<<blocks, 256, 0, (cudaStream_t)stream>>>(mode, iters, sink);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "k_fp64_peak: %s", cudaGetErrorString(e));
+    if (int rc = launched(nullptr, "k_fp64_peak")) return rc;
     if (flops_out) *flops_out = (double)blocks * 256.0 * (double)iters * 8.0 * 2.0; // 8 chains x (mul + add)
     return CCB_OK;
 }
@@ -2003,8 +1946,7 @@ int ccb_fp64_peak(int32_t device, void *stream, int32_t mode, int32_t iters, int
 int ccb_nearest(int32_t device, void *stream, const double *X, int64_t N, int64_t ld, int32_t D, const double *cen,
                 const uint64_t *prefmask, int64_t M, double k, int32_t *slot, double *dist) {
     if (D < 1 || D > CCB_MAX_D || N < 0 || M < 0 || ld < D) return fail(nullptr, CCB_EINVAL, "bad ccb_nearest arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (N == 0) return CCB_OK;
     if (M == 0) {
@@ -2014,11 +1956,7 @@ int ccb_nearest(int32_t device, void *stream, const double *X, int64_t N, int64_
     const int DP = round_dp(D);
     const bool p2 = is_pow2(k);
     const double wsel = p2 ? 1.0 / k : k;
-    double2 *cw = nullptr;
-    double *sd = nullptr;
-    int32_t *si = nullptr;
     // scratch: packed rows + per-slab candidates, sized by the split the launch will use
-    tune_pool(device);
     int max_slabs = 1;
     {
         int ok = 0;
@@ -2029,17 +1967,13 @@ int ccb_nearest(int32_t device, void *stream, const double *X, int64_t N, int64_
         })
         if (!ok) return fail(nullptr, CCB_ELIMIT, "unsupported dimensionality %d", D);
     }
-    if ((e = cudaMallocAsync(&cw, (size_t)M * DP * sizeof(double2), s)) != cudaSuccess ||
-        (e = cudaMallocAsync(&sd, (size_t)N * max_slabs * 8, s)) != cudaSuccess ||
-        (e = cudaMallocAsync(&si, (size_t)N * max_slabs * 4, s)) != cudaSuccess)
-        return fail(nullptr, CCB_ENOMEM, "scratch allocation: %s", cudaGetErrorString(e));
-    k_pack_cw<<<(unsigned)(((size_t)M * DP + 255) / 256), 256, 0, s>>>(cen, prefmask, M, D, DP, wsel, cw);
-    int rc = launch_nearest<1>(nullptr, s, DP, p2 ? 0 : 1, X, nullptr, nullptr, 0, N, ld, D, cw, (int)M, sd, si, dist, slot,
-                               max_slabs, nullptr);
-    cudaFreeAsync(cw, s);
-    cudaFreeAsync(sd, s);
-    cudaFreeAsync(si, s);
-    return rc;
+    Scratch cw(s), sd(s), si(s);
+    CK(nullptr, cw.alloc((size_t)M * DP * sizeof(double2)));
+    CK(nullptr, sd.alloc((size_t)N * max_slabs * 8));
+    CK(nullptr, si.alloc((size_t)N * max_slabs * 4));
+    k_pack_cw<<<(unsigned)(((size_t)M * DP + 255) / 256), 256, 0, s>>>(cen, prefmask, M, D, DP, wsel, cw.as<double2>());
+    return launch_nearest<1>(nullptr, s, DP, p2 ? 0 : 1, X, nullptr, nullptr, 0, N, ld, D, cw.as<double2>(), (int)M,
+                             sd.as<double>(), si.as<int32_t>(), dist, slot, max_slabs, nullptr);
 }
 
 int ccb_assoc_nearest(int32_t device, void *stream, const double *cur_cen, const uint64_t *cur_prefmask, int64_t Q,
@@ -2051,8 +1985,7 @@ int ccb_assoc_nearest2(int32_t device, void *stream, const double *cur_cen, cons
                        const double *prev_cen, int64_t P, int32_t D, double k, int32_t *best, double *dist, double *dist2) {
     if (D < 1 || D > CCB_MAX_D || Q < 0 || P < 0 || Q >= ((int64_t)1 << 31) || P >= ((int64_t)1 << 31))
         return fail(nullptr, CCB_EINVAL, "bad ccb_assoc_nearest arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (Q == 0) return CCB_OK;
     if (P == 0) {
@@ -2069,38 +2002,31 @@ int ccb_assoc_nearest2(int32_t device, void *stream, const double *cur_cen, cons
         ok = 1;
     })
     if (!ok) return fail(nullptr, CCB_ELIMIT, "unsupported dimensionality %d", D);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_assoc launch: %s", cudaGetErrorString(e));
+    return launched(nullptr, "k_assoc launch");
 }
 
 int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, int64_t ld, int32_t D, double *min_dev,
                   double *max_dev) {
     if (D < 1 || D > CCB_MAX_D || N < 0 || ld < D) return fail(nullptr, CCB_EINVAL, "bad ccb_colminmax arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    tune_pool(device);
-    unsigned long long *okey = nullptr;
-    if ((e = cudaMallocAsync(&okey, 2 * (size_t)D * 8, s)) != cudaSuccess)
-        return fail(nullptr, CCB_ENOMEM, "scratch allocation: %s", cudaGetErrorString(e));
+    Scratch sc(s);
+    CK(nullptr, sc.alloc(2 * (size_t)D * 8));
+    unsigned long long *okey = sc.as<unsigned long long>();
     cudaMemsetAsync(okey, 0xff, (size_t)D * 8, s);   // running minima: largest key
     cudaMemsetAsync(okey + D, 0x00, (size_t)D * 8, s); // running maxima: smallest key
     const int64_t total = N * D;
     if (total > 0)
         k_colminmax<<<(unsigned)std::min<int64_t>((total + 255) / 256, 148 * 8), 256, 0, s>>>(X_dev, N, ld, D, okey);
     k_colminmax_finish<<<1, 64, 0, s>>>(okey, D, min_dev, max_dev);
-    e = cudaGetLastError();
-    cudaFreeAsync(okey, s);
-    return e == cudaSuccess ? CCB_OK : fail(nullptr, CCB_ECUDA, "k_colminmax: %s", cudaGetErrorString(e));
+    return launched(nullptr, "k_colminmax");
 }
 
 int ccb_off_neighbours(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
                        double E, double E2, void *dnrm2, uint32_t *nbr, int32_t *cnt, int64_t *n_border) {
     if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M || !n_border)
         return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-    tune_pool(device);
+    if (int rc = enter_device(device)) return rc;
     return off_neighbours_settled(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, E, E2, dnrm2, nbr, cnt,
                                   n_border);
 }
@@ -2108,16 +2034,14 @@ int ccb_off_neighbours(int32_t device, void *stream, const double *cen, int64_t 
 int ccb_off_subspace(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
                      const uint32_t *nbr, const int32_t *cnt, double delta, uint64_t *submask) {
     if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     return launch_off_subspace(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, nbr, cnt, delta, submask);
 }
 
 int ccb_off_weighted(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,
                      const uint32_t *nbr, const uint64_t *submask_all, double k, double E2, uint32_t *wnbr) {
     if (D < 1 || D > CCB_MAX_D || M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     return launch_off_weighted(nullptr, (cudaStream_t)stream, cen, (int)M, D, (int)r0, (int)r1, nbr, submask_all, k, E2, wnbr);
 }
 
@@ -2125,36 +2049,27 @@ int ccb_off_clusters(int32_t device, void *stream, int64_t M, const uint32_t *wn
                      const uint64_t *submask_all, double k, int64_t pi, int32_t csr_min_m, int32_t *label, int32_t *order,
                      int32_t *cl_off, int32_t *n_cl) {
     if (M < 0) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    tune_pool(device);
-    uint8_t *cls = nullptr;
-    int32_t *queue = nullptr;
-    if ((e = cudaMallocAsync(&cls, (size_t)std::max<int64_t>(M, 1), s)) != cudaSuccess ||
-        (e = cudaMallocAsync(&queue, (2 * (size_t)M + 2) * 4, s)) != cudaSuccess)
-        return fail(nullptr, CCB_ENOMEM, "scratch allocation: %s", cudaGetErrorString(e));
+    Scratch cls(s), queue(s);
+    CK(nullptr, cls.alloc((size_t)std::max<int64_t>(M, 1)));
+    CK(nullptr, queue.alloc((2 * (size_t)M + 2) * 4));
     int nl = 0;
-    const int rc = launch_off_clusters(nullptr, s, (int)M, wnbr, core, submask_all, k > 1.0, pi, cls, queue, label, order, cl_off,
-                                       n_cl, &nl, csr_min_m);
-    cudaFreeAsync(cls, s);
-    cudaFreeAsync(queue, s);
-    return rc;
+    return launch_off_clusters(nullptr, s, (int)M, wnbr, core, submask_all, k > 1.0, pi, cls.as<uint8_t>(), queue.as<int32_t>(),
+                               label, order, cl_off, n_cl, &nl, csr_min_m);
 }
 
 int ccb_offc_rowinfo(int32_t device, void *stream, const uint32_t *wnbr_rows, int64_t M, int64_t r0, int64_t r1, uint8_t *iso,
                      int32_t *nnz) {
     if (M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     return launch_offc_rowinfo(nullptr, (cudaStream_t)stream, wnbr_rows, (int)M, (int)r0, (int)r1, iso, nnz);
 }
 
 int ccb_offc_fill(int32_t device, void *stream, const uint32_t *wnbr_rows, int64_t M, int64_t r0, int64_t r1,
                   const uint8_t *iso_all, const int64_t *off_all, int32_t *col) {
     if (M < 0 || r0 < 0 || r1 < r0 || r1 > M) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     return launch_offc_fill(nullptr, (cudaStream_t)stream, wnbr_rows, (int)M, (int)r0, (int)r1, iso_all, off_all, col);
 }
 
@@ -2162,10 +2077,8 @@ int ccb_off_clusters_csr(int32_t device, void *stream, int64_t M, const int64_t 
                          const uint8_t *core, const uint64_t *submask_all, double k, int64_t pi, int32_t *label, int32_t *order,
                          int32_t *cl_off, int32_t *n_cl) {
     if (M < 0 || M >= ((int64_t)1 << 31)) return fail(nullptr, CCB_EINVAL, "bad arguments");
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return fail(nullptr, CCB_ECUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+    if (int rc = enter_device(device)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    tune_pool(device);
     if (M == 0) {
         cudaMemsetAsync(n_cl, 0, 4, s);
         cudaMemsetAsync(cl_off, 0, 4, s);

@@ -89,8 +89,9 @@ __device__ __forceinline__ long long globaltimer_ns() {
 // ---- programmatic dependent launch (sm_90+) -------------------------------------------------------
 // Every kernel of the engine starts with CCB_PDL(): it lets the NEXT kernel of the stream be scheduled right away
 // (launch_dependents) and then waits until the kernel BEFORE it has completed and flushed its writes (wait).  Launched with
-// cudaLaunchAttributeProgrammaticStreamSerialization the launch latency of a kernel thus hides behind its predecessor; without
-// the attribute both instructions are no-ops.  Nothing but launch constants may be read before CCB_PDL().
+// cudaLaunchAttributeProgrammaticStreamSerialization the launch latency of a kernel would hide behind its predecessor; the
+// host no longer sets that attribute (measured neutral, DESIGN.md §6), so both instructions are no-ops.  They stay because
+// removing them changes the kernels' code.  Nothing but launch constants may be read before CCB_PDL().
 #define CCB_PDL()                                                      \
     do {                                                               \
         asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); \

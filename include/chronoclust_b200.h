@@ -98,7 +98,7 @@ typedef struct {
     int64_t bsv_light_rounds;        /* refinement rounds that re-ran the outlier side only (pcore side unchanged) */
     int64_t bsv_serial_cells;        /* sum over the pcore replays of the longest chain's member count: x one dependent-add
                                         latency = the serial floor of kernel 2 (what the reference's ordering forces) */
-    int64_t bsv_pdl;                 /* 1: the engine's graph was built with programmatic dependent launches between its kernels */
+    int64_t bsv_pdl;                 /* always 0: the engine no longer uses programmatic dependent launch (field kept for the ABI) */
 } ccb_stats;
 
 int ccb_create(const ccb_params *params, ccb_handle **out);
