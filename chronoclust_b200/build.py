@@ -3,8 +3,8 @@
     python chronoclust_b200/build.py [--force] [--debug]
 
 --debug builds libchronoclust_b200_debug.so instead: the same sources with -DCCB_DEBUG, which adds the diagnostics of
-csrc/debug.h (per-key cycle counters of the replay kernel, switches that deliberately break results).  The product
-library never contains them.
+csrc/debug.h (per-key cycle counters of the replay kernel, event counters, the round-by-round trace ring).  The
+product library never contains them.
 """
 import os
 import subprocess

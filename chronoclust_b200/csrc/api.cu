@@ -1280,14 +1280,7 @@ int ccb_get_stats(const ccb_handle *h, ccb_stats *out) {
 
 #ifdef CCB_DEBUG
 // Diagnostics build only (python chronoclust_b200/build.py --debug -> libchronoclust_b200_debug.so, declared in
-// csrc/debug.h): neither symbol exists in the product library.
-int ccb_debug_set(ccb_handle *h, int32_t mode) {
-    if (!h) return fail(h, CCB_EINVAL, "null argument");
-    CK(h, cudaStreamSynchronize(h->stream));
-    CK(h, cudaMemcpyToSymbol(g_bs_dbg_mode, &mode, sizeof(int)));
-    return CCB_OK;
-}
-
+// csrc/debug.h): none of these symbols exists in the product library.
 int64_t ccb_debug_trace(ccb_handle *h, int64_t *out, int64_t max_records) {
     if (!h || !out) return -1;
     cudaStreamSynchronize(h->stream);

@@ -16,9 +16,6 @@ extern "C" {
  * stages with a CONTESTED cell or a ragged tail, CONTESTED cells, cycles at the head of the stages (flags), cycles at
  * their tail (proxy fence + arrive), clean full stages}.  The first call switches the counters on. */
 int ccb_debug_chain(ccb_handle *h, int64_t *out, int32_t max_keys);
-/* Results may become WRONG: 1 = the store thread of k_bs_chain_p skips its bulk copies, 4 = the replay warp skips the
- * proxy fence before handing a stage to the store thread (timing experiments).  0 restores normal operation. */
-int ccb_debug_set(ccb_handle *h, int32_t mode);
 /* Timeline of the engine: one record of 48 int64 per refinement round (kind 0 / 1, written by k_bs_decide) and per block
  * (kind 2, k_bs_commit): control-block fields and the start time (globaltimer, ns) of every kernel of the round; layout in
  * tools/trace_rounds.py.  Returns the number of records written since the last call (at most max_records are copied) and

@@ -955,10 +955,6 @@ struct ChainPCfg {
 // warp's scheduler) warms the instruction cache of the rare path and exits; warp 3 only fills the CTA up
 constexpr int BS_CHAINP_THREADS = 160;
 
-#ifdef CCB_DEBUG
-__device__ int g_bs_dbg_mode = 0; // diagnostics build only (csrc/debug.h): 1 = storers skip the global stores, 2 = skip the copies
-#endif
-
 // Exact radius test of the tentative MC nv = v + a (mc_functions.py:45-56) for a CONTESTED cell, by the whole replay
 // warp (lane = record element).  Deliberately NOT inlined: the replay warp runs alone on its scheduler, so every cold
 // instruction-cache line it touches is a full miss it cannot hide; one small shared copy keeps the footprint of the
@@ -1466,7 +1462,6 @@ __global__ void __launch_bounds__(BS_CHAINP_THREADS) k_bs_chain_p(Eng e) {
                     CCB_DBG(tw += clock64() - t0;)
                 }
                 const int cnt = min(NB, n - b * NB);
-                CCB_DBG(if (!(g_bs_dbg_mode & 1)))
                 tma_store_1d(vp + (size_t)b * NB * LSP, xs + (size_t)s * NB * LSP, (uint32_t)cnt * LSP * 8u);
                 asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                 if (b > 0) { // the copy before this one has read its stage: hand that stage back to the producer
@@ -1519,15 +1514,8 @@ __global__ void __launch_bounds__(BS_CHAINP_THREADS) k_bs_chain_p(Eng e) {
         for (int o = 16; o > 0; o >>= 1) q2 = dadd(q2, __shfl_xor_sync(0xffffffffu, q2, o));
         cfast.mg = dadd(DP > 16 ? 0.01 : (double)(D + 8), dmul(0x1p-48 * TH, ddiv(ddiv(q2, e.P.w[j]), nm.eps2)));
     }
-#if defined(CCB_CHAIN_PAIRS)
-    bool bmode = false;
-#elif defined(CCB_CHAIN_BATCH)
-    bool bmode = true;
-#else
     bool bmode = bc->it > 0; // (see the CONTESTED groups below)
-#endif
-    CCB_DBG(long long t_wait = 0, t_slow = 0, n_cont = 0, t_head = 0, t_tail = 0, n_clean = 0; const long long t_beg = clock64();
-            const int dbgm = g_bs_dbg_mode;)
+    CCB_DBG(long long t_wait = 0, t_slow = 0, n_cont = 0, t_head = 0, t_tail = 0, n_clean = 0; const long long t_beg = clock64();)
     // The replay warp issues in order and is alone on its scheduler: every dependent instruction costs its full latency.
     // Everything below is arranged for that.  Addresses and the lane number are held in OPAQUE registers (otherwise the
     // compiler re-derives them from special registers -- S2R / S2UR, tens of cycles each -- inside the loop).
@@ -1659,13 +1647,7 @@ __global__ void __launch_bounds__(BS_CHAINP_THREADS) k_bs_chain_p(Eng e) {
                                 atomicAdd(&g_dbg_cnt[4], (unsigned long long)__popc(cg));
                                 atomicAdd(&g_dbg_cnt[5], (unsigned long long)__popc(pgm & cg)); // predicted rejections
                             })
-#if defined(CCB_CHAIN_PAIRS)
-                            bmode = false;
-#elif defined(CCB_CHAIN_BATCH)
-                            bmode = true;
-#else
                             bmode = rd.dev <= 1;
-#endif
                         } else
                             rec = bs_chain_slow_group<DP, NH>(rec, ga, ma + g * (GS * 4), cg, ncell, lane_o, D, nm.delta2, nm.eps2,
                                                               nm.div_mode, nm.k, nm.wsel, e.ws.prej, cfast, (b | g) == 0);
@@ -1682,7 +1664,6 @@ __global__ void __launch_bounds__(BS_CHAINP_THREADS) k_bs_chain_p(Eng e) {
         // the versions were written through the generic proxy; the bulk copy reads them through the async proxy
         CCB_DBG(const long long t_t0 = clock64();)
         __syncwarp();
-        CCB_DBG(if (!(dbgm & 4)))
         fence_proxy_async_smem();
         __syncwarp();
         if (lane_o == 0) mbar_arrive(&done[s]);

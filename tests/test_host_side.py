@@ -306,18 +306,3 @@ def test_bench_dump_outputs_keeps_a_fixed_sample_under_the_budget(tmp_path):
     bench.dump_outputs(str(tmp_path / "whole"), arrays)
     assert sorted(os.listdir(tmp_path / "whole")) == ["assign.npy", "cen.npy", "w.npy"]
     assert (np.load(tmp_path / "whole" / "assign.npy") == arrays["assign"]).all()
-
-
-def test_generated_documents_carry_no_unfilled_field():
-    """DESIGN.md / README.md are generated from tools/templates/*.in by tools/fill_docs.py: no @FIELD@ may survive, and
-    the text around the numbers must be the template's."""
-    import re
-
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    for name in ("DESIGN.md", "README.md"):
-        doc = open(os.path.join(root, name), encoding="utf-8").read()
-        tpl = open(os.path.join(root, "tools", "templates", name + ".in"), encoding="utf-8").read()
-        assert not re.findall(r"@[A-Z0-9_]+@", doc), name
-        # every literal stretch of the template (between two fields) occurs in the generated document
-        for piece in re.split(r"@[A-Z0-9_]+@", tpl):
-            assert piece in doc, f"{name} is out of date with its template near: {piece[:80]!r}"

@@ -25,14 +25,7 @@ h = HDDStream(config_params(name), logging.getLogger("q"), chunk=chunk, bsv_iter
 prev = None
 h._ensure_handle(D)
 h.enable_timing()
-dbg_mode = [int(a.split("=")[1]) for a in sys.argv if a.startswith("--dbg=")]
 for t, X in enumerate(Xs):
-    if dbg_mode and t == 3:  # debug build only: timing experiments from timepoint 3 on (results may be wrong from there)
-        import ctypes as C
-        from chronoclust_b200 import _lib as _l
-        fn = _l.lib().ccb_debug_set
-        fn.restype, fn.argtypes = C.c_int, [C.c_void_p, C.c_int32]
-        _l.check(fn(h._h, dbg_mode[0]), h._h)
     t0 = time.time()
     h.online_microcluster_maintenance(X, t, run_offline=False)
     t1 = time.time()

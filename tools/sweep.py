@@ -26,10 +26,6 @@ GRID = list(itertools.product((0.04, 0.045, 0.05, 0.055), (4.0, 5.5, 6.5, 8.0), 
 
 
 def main():
-    if "--debuglib" in sys.argv:  # experiment knobs (CCB_SLACK, ...) only exist in the debug build
-        sys.argv.remove("--debuglib")
-        from chronoclust_b200 import _lib as _l0, build as _b0
-        _l0.SO_PATH = _b0.build(debug=True)
     ap = argparse.ArgumentParser()
     ap.add_argument("--scale", type=float, default=1.0)
     ap.add_argument("--configs", type=int, default=len(GRID))

@@ -1,6 +1,6 @@
 """Per-timepoint wall time of the device-resident path without event timing (what bench.py's `value` sees).
 
-    python tools/tp_wall.py C2 1.0 [chunk] [--lib path/to/variant.so] [--debuglib] [--eps 0.04] [--iters 12] [--bmin 2048]
+    python tools/tp_wall.py C2 1.0 [chunk] [--eps 0.04] [--iters 12] [--bmin 2048]
                                   [--reps 3] [--tps 5] [--sweep "chunk=24576;iters=12"]
 """
 import logging
@@ -23,14 +23,6 @@ def opt(name, default, cast=float):
     return default
 
 
-if "--debuglib" in sys.argv:  # experiment knobs only exist in the debug build
-    sys.argv.remove("--debuglib")
-    from chronoclust_b200 import _lib as _l0, build as _b0
-    _l0.SO_PATH = _b0.build(debug=True)
-lib = opt("--lib", None, str)
-if lib:  # a variant build of the library (A/B experiments)
-    from chronoclust_b200 import _lib as _l0
-    _l0.SO_PATH = lib
 eps_over = opt("--eps", None)
 reps = opt("--reps", 3, int)
 tps = opt("--tps", 0, int)
@@ -61,7 +53,7 @@ for cfg in settings:
     h = HDDStream(prm, logging.getLogger("q"), chunk=cfg["chunk"], bsv_iters=cfg["iters"], bsv_bmin=cfg["bmin"])
     h.dataset_dimensionality = D
     h._ensure_handle(D)
-    print(f"# {name} x{scale} lib={lib} eps={eps_over} {cfg}")
+    print(f"# {name} x{scale} eps={eps_over} {cfg}")
     for rep in range(reps):
         h.reset()
         prev = h.stats()
@@ -80,5 +72,5 @@ for cfg in settings:
                         f"cuts={st['bsv_cuts_unknown']-prev['bsv_cuts_unknown']}/{st['bsv_cuts_rounds']-prev['bsv_cuts_rounds']}/"
                         f"{st['bsv_cuts_capacity']-prev['bsv_cuts_capacity']} launches={st['kernel_launches']-prev['kernel_launches']}")
             prev = st
-        print(f"rep {rep}: total {tot*1e3:.1f}ms | " + " | ".join(line) + f" | pdl={h.stats()['bsv_pdl']}")
+        print(f"rep {rep}: total {tot*1e3:.1f}ms | " + " | ".join(line))
     del h
