@@ -48,6 +48,7 @@ SYMBOLS = {
     "ccb_begin_timepoint": (C.c_int, [vp, f64, f64, i64, i32, f64]),
     "ccb_ingest": (C.c_int, [vp, vp, i64, i64, vp, vp]),
     "ccb_ingest_device": (C.c_int, [vp, vp, i64, i64, vp, vp]),
+    "ccb_ingest_ex": (C.c_int, [vp, vp, i32, i32, i64, i64, vp, vp, vp, vp]),
     "ccb_offline": (C.c_int, [vp, C.POINTER(i64)]),
     "ccb_counts": (C.c_int, [vp, C.POINTER(i64 * 4)]),
     "ccb_export_list": (C.c_int, [vp, i32] + [vp] * 7),
@@ -60,6 +61,7 @@ SYMBOLS = {
     "ccb_assoc_nearest": (C.c_int, [i32, vp, vp, vp, i64, vp, i64, i32, f64, vp, vp]),
     "ccb_assoc_nearest2": (C.c_int, [i32, vp, vp, vp, i64, vp, i64, i32, f64, vp, vp, vp]),
     "ccb_colminmax": (C.c_int, [i32, vp, vp, i64, i64, i32, vp, vp]),
+    "ccb_colminmax_ex": (C.c_int, [i32, vp, vp, i32, i64, i64, i32, vp, vp]),
     "ccb_ingest_scaled": (C.c_int, [vp, vp, i64, i64, vp, vp, vp, vp]),
     "ccb_off_neighbours": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, f64, f64, vp, vp, vp, C.POINTER(i64)]),
     "ccb_off_subspace": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, vp, vp, f64, vp]),
@@ -70,6 +72,8 @@ SYMBOLS = {
     "ccb_off_clusters_csr": (C.c_int, [i32, vp, i64, vp, vp, vp, vp, vp, f64, i64, vp, vp, vp, vp]),
 }
 
+
+DTYPE_F64, DTYPE_F32 = 0, 1  # CCB_DTYPE_*
 
 CATEGORIES = ["chain_p", "nearest", "verify", "maintenance", "offline", "misc", "copy", "speculate", "lists", "chain_o",
               "olist", "derive", "decide", "commit", "reserved14", "reserved15"]

@@ -180,6 +180,7 @@ struct ccb_handle {
     bool have_params = false;
     // ingest buffers
     Grow<Dev<double>> d_X;
+    Grow<Dev<float>> d_X32; // float32 host rows as copied, before k_stage_rows widens them into d_X
     Grow<Dev<int32_t>> d_assign;
     Grow<Dev<uint8_t>> d_stage;
     Grow<Dev<int32_t>> d_pnew, d_pfin, d_onew; // kernel 3 plan codes
@@ -202,7 +203,7 @@ struct ccb_handle {
     Stream copy_stream; // host -> device segments of ccb_ingest, ahead of the engine
     Stream res_stream;  // device -> host copies of the per-cell results of a finished segment, behind the engine
     Grow<Pinned<unsigned char>> h_res; // page-locked bounce buffer of those results ([n] int32 assignments, then [n] stages)
-    Grow<Dev<double>> d_scale;          // [2][CCB_MAX_D] scale_ / min_ of ccb_ingest_scaled
+    Grow<Dev<double>> d_scale;          // [2][CCB_MAX_D] scale_ / min_ of the scaled ingest
     Event ev_seg[8];
     // offline results (host copies)
     int64_t off_M = 0;
@@ -1437,49 +1438,87 @@ int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, in
     return sync_ctl(h);
 }
 
-int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
-                      uint8_t *stage_dev) {
-    if (int rc = enter(h)) return rc;
-    if (N < 0 || ld < h->D || (!X_dev && N > 0) || (!assign_uid_dev && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
-    return ingest_core_bsv(h, X_dev, N, ld, assign_uid_dev, stage_dev);
+// widen (and, with a scaler, min-max transform) n rows of dtype into double rows, on the handle's stream
+static void stage_rows(ccb_handle *h, int32_t dtype, const void *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t n,
+                       const double *scale, const double *shift) {
+    if (n <= 0) return;
+    const int64_t total = n * h->D;
+    const unsigned gx = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
+    if (dtype == CCB_DTYPE_F32)
+        k_stage_rows<float><<<gx, 256, 0, h->stream>>>(static_cast<const float *>(src), ld_src, dst, ld_dst, n, h->D, scale, shift);
+    else
+        k_stage_rows<double><<<gx, 256, 0, h->stream>>>(static_cast<const double *>(src), ld_src, dst, ld_dst, n, h->D, scale, shift);
+    h->st.kernel_launches++;
 }
 
-static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, int32_t *assign_uid, uint8_t *stage,
-                       const double *scale, const double *shift);
+static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t *assign_uid,
+                       uint8_t *stage, const double *scale, const double *shift);
+
+int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld,
+                  const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
+    int rc;
+    if ((rc = enter(h))) return rc;
+    if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(h, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
+    if (!scale != !min_) return fail(h, CCB_EINVAL, "scale and min_ must both be set or both be NULL");
+    if (ld < h->D) return fail(h, CCB_EINVAL, "leading dimension %lld < D = %d", (long long)ld, h->D);
+    if (N < 0 || (!X && N > 0) || (!assign_uid && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
+    if (scale) { // behind whatever still reads the vectors on the handle's stream
+        CK(h, h->d_scale.ensure(2 * CCB_MAX_D * sizeof(double)));
+        CK(h, cudaMemcpyAsync(h->d_scale, scale, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(h, cudaMemcpyAsync(h->d_scale + CCB_MAX_D, min_, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
+    }
+    const double *d_sc = scale ? h->d_scale.p : nullptr, *d_sh = scale ? h->d_scale + CCB_MAX_D : nullptr;
+    if (!on_device) return ingest_host(h, X, dtype, N, ld, assign_uid, stage, d_sc, d_sh);
+    // device-resident rows: float64 without a scaler go to the engine as they are; anything else is staged into d_X
+    // (leading dimension D) by one launch -- the caller's buffer is never written
+    if (dtype == CCB_DTYPE_F64 && !scale) return ingest_core_bsv(h, static_cast<const double *>(X), N, ld, assign_uid, stage);
+    CK(h, h->d_X.ensure(((size_t)N * h->D + 2) * 8));
+    stage_rows(h, dtype, X, ld, h->d_X, h->D, N, d_sc, d_sh);
+    CKL(h);
+    return ingest_core_bsv(h, h->d_X, N, h->D, assign_uid, stage);
+}
+
+int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
+                      uint8_t *stage_dev) {
+    return ccb_ingest_ex(h, X_dev, CCB_DTYPE_F64, 1, N, ld, nullptr, nullptr, assign_uid_dev, stage_dev);
+}
 
 int ccb_ingest(ccb_handle *h, const double *X, int64_t N, int64_t ld, int32_t *assign_uid, uint8_t *stage) {
-    return ingest_host(h, X, N, ld, assign_uid, stage, nullptr, nullptr);
+    return ccb_ingest_ex(h, X, CCB_DTYPE_F64, 0, N, ld, nullptr, nullptr, assign_uid, stage);
 }
 
 int ccb_ingest_scaled(ccb_handle *h, const double *X_raw, int64_t N, int64_t ld, const double *scale, const double *min_,
                       int32_t *assign_uid, uint8_t *stage) {
     if (!scale || !min_) return fail(h, CCB_EINVAL, "null scaler vectors");
-    return ingest_host(h, X_raw, N, ld, assign_uid, stage, scale, min_);
+    return ccb_ingest_ex(h, X_raw, CCB_DTYPE_F64, 0, N, ld, scale, min_, assign_uid, stage);
 }
 
-// host buffers in, per-cell results out; scale != nullptr: the rows are min-max scaled on the device first
-// (X * scale + shift, two roundings: sklearn MinMaxScaler.transform), segment by segment behind their copies
-static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, int32_t *assign_uid, uint8_t *stage,
-                       const double *scale, const double *shift) {
+// host rows in, per-cell results out.  float64 rows are copied into d_X as they are (leading dimension ld) and, with a
+// scaler (scale / shift: device vectors), min-max transformed there in place; float32 rows are copied into the float32
+// staging buffer and widened (and transformed) from there into d_X with leading dimension D.  Either happens segment by
+// segment behind the segments' copies.  Arguments are checked by ccb_ingest_ex.
+static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t *assign_uid,
+                       uint8_t *stage, const double *scale, const double *shift) {
     int rc;
-    if ((rc = enter(h))) return rc;
-    if (N < 0 || ld < h->D || (!X && N > 0) || (!assign_uid && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
     if (N == 0) return CCB_OK;
-    const size_t need = (size_t)N * ld;
-    CK(h, h->d_X.ensure((need + 2) * 8));
+    const bool f32 = dtype == CCB_DTYPE_F32;
+    const size_t esz = f32 ? 4 : 8;
+    const int64_t ldX = f32 ? h->D : ld; // leading dimension of the rows in d_X
+    // the rows [r0, r0 + n) of the caller occupy (n - 1) * ld + D elements: the last row's padding is not read
+    auto span = [&](int64_t n) { return (size_t)((n - 1) * ld + h->D) * esz; };
+    CK(h, h->d_X.ensure(((size_t)N * ldX + 2) * 8));
+    if (f32) CK(h, h->d_X32.ensure(span(N)));
     CK(h, h->d_assign.ensure((size_t)N * 4));
     CK(h, h->d_stage.ensure((size_t)N));
-    if (scale) {
-        CK(h, h->d_scale.ensure(2 * CCB_MAX_D * sizeof(double)));
-        CK(h, cudaMemcpyAsync(h->d_scale, scale, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
-        CK(h, cudaMemcpyAsync(h->d_scale + CCB_MAX_D, shift, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
-    }
-    auto scale_rows = [&](int64_t r0, int64_t n) { // on the handle's stream, behind the wait for the rows' copy
-        if (!scale || n <= 0) return;
-        const int64_t total = n * h->D;
-        k_scale_rows<<<(unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, h->stream>>>(
-            h->d_X + r0 * ld, n, ld, h->D, h->d_scale, h->d_scale + CCB_MAX_D);
-        h->st.kernel_launches++;
+    const char *src = static_cast<const char *>(X);
+    char *dst = f32 ? reinterpret_cast<char *>(h->d_X32.p) : reinterpret_cast<char *>(h->d_X.p); // where the copies land
+    // the copied rows [r0, r0 + n) -> double rows in d_X, on the handle's stream behind the wait for their copy
+    auto stage_seg = [&](int64_t r0, int64_t n) -> int {
+        if (f32 || scale) {
+            stage_rows(h, dtype, dst + r0 * ld * esz, ld, h->d_X + r0 * ldX, ldX, n, scale, shift);
+            CKL(h);
+        }
+        return CCB_OK;
     };
     // segments of the input: one block's worth of rows first, then doubling, the last one takes the rest -- the engine
     // starts after a 3 MB copy instead of a 24 MB one and the copies (5x faster than the engine) stay ahead of it
@@ -1505,11 +1544,9 @@ static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, in
     if (nseg == 1) {
         {
             Timed tm(h, CCB_CAT_COPY);
-            CK(h, cudaMemcpyAsync(h->d_X, X, need * 8, cudaMemcpyHostToDevice, h->stream));
+            CK(h, cudaMemcpyAsync(dst, src, span(N), cudaMemcpyHostToDevice, h->stream));
         }
-        scale_rows(0, N);
-        rc = ingest_core_bsv(h, h->d_X, N, ld, h->d_assign, h->d_stage);
-        if (rc) return rc;
+        if ((rc = stage_seg(0, N)) || (rc = ingest_core_bsv(h, h->d_X, N, ldX, h->d_assign, h->d_stage))) return rc;
     } else {
         // The ordered engine consumes cells front to back, so the input travels in segments on a copy stream and the
         // engine starts as soon as the first one has landed: segment k + 1 is queued right after the engine has been
@@ -1534,7 +1571,7 @@ static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, in
             int64_t r0, n;
             seg_rows(k, r0, n);
             if (n > 0)
-                CK(h, cudaMemcpyAsync(h->d_X + r0 * ld, X + r0 * ld, (size_t)n * ld * 8, cudaMemcpyHostToDevice, h->copy_stream));
+                CK(h, cudaMemcpyAsync(dst + r0 * ld * esz, src + r0 * ld * esz, span(n), cudaMemcpyHostToDevice, h->copy_stream));
             CK(h, cudaEventRecord(h->ev_seg[k], h->copy_stream));
             return CCB_OK;
         };
@@ -1558,14 +1595,14 @@ static int ingest_host(ccb_handle *h, const double *X, int64_t N, int64_t ld, in
             int64_t r0, n;
             seg_rows(k, r0, n);
             CK(h, cudaStreamWaitEvent(h->stream, h->ev_seg[k], 0));
-            scale_rows(r0, n);
+            if ((rc = stage_seg(r0, n))) return rc;
             // once the engine is running on segment k: queue the input of segment k + 1, fetch the results of segment k - 1
             const std::function<int()> next = [&]() -> int {
                 int r = k + 1 < nseg ? copy_seg(k + 1) : CCB_OK;
                 if (!r && k > 0) r = results_seg(k - 1);
                 return r;
             };
-            if ((rc = ingest_core_bsv(h, h->d_X + r0 * ld, n, ld, h->d_assign + r0, h->d_stage + r0, &next))) return rc;
+            if ((rc = ingest_core_bsv(h, h->d_X + r0 * ldX, n, ldX, h->d_assign + r0, h->d_stage + r0, &next))) return rc;
         }
         if ((rc = results_seg(nseg - 1))) return rc;
         return CCB_OK;
@@ -1998,8 +2035,9 @@ int ccb_assoc_nearest2(int32_t device, void *stream, const double *cur_cen, cons
     return launched(nullptr, "k_assoc launch");
 }
 
-int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, int64_t ld, int32_t D, double *min_dev,
-                  double *max_dev) {
+int ccb_colminmax_ex(int32_t device, void *stream, const void *X_dev, int32_t dtype, int64_t N, int64_t ld, int32_t D,
+                     double *min_dev, double *max_dev) {
+    if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(nullptr, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
     if (D < 1 || D > CCB_MAX_D || N < 0 || ld < D) return fail(nullptr, CCB_EINVAL, "bad ccb_colminmax arguments");
     if (int rc = enter_device(device)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
@@ -2009,10 +2047,18 @@ int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, 
     cudaMemsetAsync(okey, 0xff, (size_t)D * 8, s);   // running minima: largest key
     cudaMemsetAsync(okey + D, 0x00, (size_t)D * 8, s); // running maxima: smallest key
     const int64_t total = N * D;
-    if (total > 0)
-        k_colminmax<<<(unsigned)std::min<int64_t>((total + 255) / 256, 148 * 8), 256, 0, s>>>(X_dev, N, ld, D, okey);
+    const unsigned gx = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 8);
+    if (total > 0 && dtype == CCB_DTYPE_F32)
+        k_colminmax<float><<<gx, 256, 0, s>>>(static_cast<const float *>(X_dev), N, ld, D, okey);
+    else if (total > 0)
+        k_colminmax<double><<<gx, 256, 0, s>>>(static_cast<const double *>(X_dev), N, ld, D, okey);
     k_colminmax_finish<<<1, 64, 0, s>>>(okey, D, min_dev, max_dev);
     return launched(nullptr, "k_colminmax");
+}
+
+int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, int64_t ld, int32_t D, double *min_dev,
+                  double *max_dev) {
+    return ccb_colminmax_ex(device, stream, X_dev, CCB_DTYPE_F64, N, ld, D, min_dev, max_dev);
 }
 
 int ccb_off_neighbours(int32_t device, void *stream, const double *cen, int64_t M, int32_t D, int64_t r0, int64_t r1,

@@ -9,7 +9,8 @@
 // Kernel 3   k_maint_plan + k_maint_gather: fused decay x 2^(-lambda dt) (hddstream.py:247-286), downgrade with the
 //            reference's skip-next-after-removal iteration and outlier deletion (hddstream.py:512-549), order-preserving
 //            compaction.
-// Scaler     k_scale_rows / k_colminmax: the min-max transform and fit reductions (scaling/scaler.py:11-53).
+// Input      k_stage_rows / k_colminmax: float32 / float64 rows widened to double and min-max transformed, and the fit
+//            reductions (scaling/scaler.py:11-53).
 #pragma once
 #include "common.cuh"
 
@@ -283,17 +284,22 @@ __global__ void k_repack_store(Store S, int n, int D, int DP, double wsel) {
     S.cw[i] = cv;
 }
 
-// ---- scaler (SURVEY 8f-3; scaling/scaler.py:11-53 -> sklearn MinMaxScaler) ---------------------------------------
-// transform: X * scale_ + min_ as TWO roundings (sklearn: `X *= self.scale_; X += self.min_`), in place on the device
-// copy of a timepoint, so the host never makes the scaled pass over the data.  HBM-bound: 16 B per element.
-__global__ void k_scale_rows(double *__restrict__ X, int64_t N, int64_t ld, int D, const double *__restrict__ scale,
-                             const double *__restrict__ shift) {
+// ---- input staging and scaler (SURVEY 8f-3; scaling/scaler.py:11-53 -> sklearn MinMaxScaler) --------------------
+// Rows of T (float or double, leading dimension ld_src in elements of T) -> double rows (leading dimension ld_dst).  Every
+// element is widened to double first, which is exact; with a scaler the min-max transform follows as TWO roundings
+// (sklearn: `X *= self.scale_; X += self.min_`), so results equal those of widening and scaling on the host.  src == dst
+// (T = double, ld_src == ld_dst) scales the device copy of a timepoint in place: every element is read and written by
+// the same thread, hence no __restrict__ on src / dst.  HBM-bound: 8 + 8 B (double) or 4 + 8 B (float) per element.
+template <typename T>
+__global__ void k_stage_rows(const T *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t N, int D,
+                             const double *__restrict__ scale, const double *__restrict__ shift) {
     const int64_t total = N * D;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = e / D;
         const int d = (int)(e - r * D);
-        double *p = X + r * ld + d;
-        *p = dadd(dmul(*p, scale[d]), shift[d]);
+        double x = (double)src[r * ld_src + d];
+        if (scale) x = dadd(dmul(x, scale[d]), shift[d]);
+        dst[r * ld_dst + d] = x;
     }
 }
 
@@ -304,7 +310,8 @@ __device__ __forceinline__ unsigned long long ordered_key(double v) {
     const unsigned long long b = (unsigned long long)__double_as_longlong(v);
     return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
-__global__ void k_colminmax(const double *__restrict__ X, int64_t N, int64_t ld, int D, unsigned long long *okey) {
+template <typename T>
+__global__ void k_colminmax(const T *__restrict__ X, int64_t N, int64_t ld, int D, unsigned long long *okey) {
     __shared__ unsigned long long s_min[CCB_MAX_D], s_max[CCB_MAX_D];
     for (int d = threadIdx.x; d < D; d += blockDim.x) {
         s_min[d] = ~0ull;
@@ -320,7 +327,7 @@ __global__ void k_colminmax(const double *__restrict__ X, int64_t N, int64_t ld,
         const int d = (int)(e0 % D);
         unsigned long long lo = ~0ull, hi = 0ull;
         for (int64_t e = e0; e < total; e += stride) {
-            const double v = X[(e / D) * ld + d];
+            const double v = (double)X[(e / D) * ld + d]; // widened first (exact): the keys are those of the doubles
             if (v == v) { // not NaN
                 const unsigned long long k = ordered_key(v);
                 lo = k < lo ? k : lo;

@@ -17,10 +17,43 @@ from . import _lib
 from .objects import FinalCluster, Microcluster
 
 
+_NP_DTYPES = {np.dtype(np.float64): _lib.DTYPE_F64, np.dtype(np.float32): _lib.DTYPE_F32}
+
+
+def _input_rows(x, device):
+    """How input_dataset goes to ccb_ingest_ex: (pointer, CCB_DTYPE_*, on_device, ld, rows), `rows` being the array or
+    tensor the pointer points into (the caller's own where possible; keep it alive until the call returns).
+
+    float32 / float64 rows with unit column stride and a row stride >= D go in without a copy, with ld = the row stride:
+    numpy arrays and CPU tensors as host input, CUDA tensors on the handle's `device` as device input (a CUDA tensor on
+    another device raises ValueError).  Everything else is made float64 and C-contiguous on the host, as numpy does."""
+    torch = sys.modules.get("torch")  # a caller that passes a tensor has imported torch
+    if torch is not None and isinstance(x, torch.Tensor):
+        x = x.detach()
+        if x.is_cuda:
+            if x.device.index != device:
+                raise ValueError(f"input_dataset is on {x.device}, this HDDStream runs on cuda:{device}")
+            code = {torch.float64: _lib.DTYPE_F64, torch.float32: _lib.DTYPE_F32}.get(x.dtype)
+            if code is not None and x.dim() == 2 and x.shape[0] > 0 and x.stride(1) == 1:
+                ld = x.stride(0) if x.shape[0] > 1 else x.shape[1]  # (the stride of a single row means nothing)
+                if ld >= x.shape[1]:
+                    return x.data_ptr(), code, True, ld, x
+        x = x.cpu().numpy()
+    if isinstance(x, np.ndarray) and x.ndim == 2 and x.shape[0] > 0 and x.flags.aligned:
+        code, isz = _NP_DTYPES.get(x.dtype), x.dtype.itemsize  # (a byte-swapped dtype is not among the keys)
+        ld = x.strides[0] // isz if x.shape[0] > 1 else x.shape[1]  # (the stride of a single row means nothing)
+        if code is not None and x.strides[1] == isz and x.strides[0] % isz == 0 and ld >= x.shape[1]:
+            return x.ctypes.data, code, False, ld, x
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    return x.ctypes.data, _lib.DTYPE_F64, False, (x.shape[1] if x.ndim == 2 else 0), x
+
+
 class _PointsView(object):
-    """Per-timepoint cell -> MC assignment; builds Microcluster.points dicts on demand.  The input arrays are BORROWED, not
-    copied (the reference copies every row into a Python list, microcluster.py:149): a caller that overwrites its array
-    in place after the call changes what `points` hands out."""
+    """Per-timepoint cell -> MC assignment; builds Microcluster.points dicts on demand.  The input arrays or tensors are
+    BORROWED, not copied (the reference copies every row into a Python list, microcluster.py:149): a caller that
+    overwrites its array or tensor in place after the call changes what `points` hands out.  float32 rows are handed out
+    widened to float64, and the rows of a CUDA tensor are gathered on its device and brought back as float64 -- the same
+    values the float64 path hands out."""
 
     def __init__(self):
         self.segments = []  # [(X, assign_uid)] since the last reset (hddstream.py:208-213)
@@ -59,7 +92,12 @@ class _PointsView(object):
         out = {}
         for si, rows in self.rows_of(uid):
             X, _, sc = self.segments[si]
-            sel = X[rows]
+            if isinstance(X, np.ndarray):
+                sel = X[rows].astype(np.float64, copy=False)  # (widened before the scaler arithmetic)
+            else:  # a CUDA tensor
+                import torch
+
+                sel = X[torch.from_numpy(rows).to(X.device)].to(torch.float64).cpu().numpy()
             if sc is not None:
                 sel = sel * sc[0]
                 sel = sel + sc[1]
@@ -193,15 +231,28 @@ class HDDStream(object):
     # ------------------------------------------------------------------------------------------
     def online_microcluster_maintenance(self, input_dataset, input_dataset_daystamp, reset_param=True,
                                         run_offline=True, scaler=None):
-        """scaler (extension, SURVEY 8f-3): a fitted sklearn MinMaxScaler (or a (scale_, min_) pair) -- input_dataset then
+        """input_dataset: [N, D] cells -- a numpy array, a CPU tensor or a CUDA tensor on this instance's device.  float32 and
+        float64 rows with unit column stride go in without a copy (row-strided views included); float32 rows are widened
+        to float64 on the device, which is exact, so results are those of the float64 path on the widened rows.  Other
+        inputs are made float64 on the host first.  For a CUDA tensor the call waits for the work queued on the current
+        torch stream of its device; last_assignment / last_stage come back to the host either way.
+
+        scaler (extension, SURVEY 8f-3): a fitted sklearn MinMaxScaler (or a (scale_, min_) pair) -- input_dataset then
         holds RAW rows and the min-max transform x * scale_ + min_ runs on the device behind the host -> device copy
-        (ccb_ingest_scaled) instead of as a host pass; results are those of scaling on the host first, bit for bit."""
-        X = np.ascontiguousarray(input_dataset, dtype=np.float64)
+        (ccb_ingest_ex) instead of as a host pass; results are those of scaling on the host first, bit for bit."""
+        xp, dtype, on_device, ld, X = _input_rows(input_dataset, self._device)
         if X.ndim != 2:
             raise ValueError("input_dataset must be 2-D")
         if reset_param:
             self._set_dataset_dependent_parameters(X)
         self._ensure_handle(X.shape[1])
+        sc = mn = None
+        if scaler is not None:
+            sc, mn = (scaler.scale_, scaler.min_) if hasattr(scaler, "scale_") else scaler
+            sc = np.ascontiguousarray(sc, np.float64)
+            mn = np.ascontiguousarray(mn, np.float64)
+            if sc.shape != (X.shape[1],) or mn.shape != (X.shape[1],):
+                raise ValueError("scaler vectors must have one entry per marker")
         L, h, logger = _lib.lib(), self._h, self.logger
         logger.info(f"Setting up online phase for timepoint {input_dataset_daystamp} with following params:\n"
                     f"Pcore density threshold factor(beta) = {self.beta}\n"
@@ -226,20 +277,14 @@ class HDDStream(object):
                                          float(factor)), h)
         N = X.shape[0]
         logger.info("Starting online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
-        assign = np.empty(N, np.int32)
-        stage = np.empty(N, np.uint8)
-        if scaler is None:
-            _lib.check(L.ccb_ingest(h, _lib.ptr(X), N, X.shape[1], _lib.ptr(assign), _lib.ptr(stage)), h)
-            self._views.add(X, assign)
+        if on_device:
+            assign, stage = self._ingest_tensor(X, xp, dtype, ld, sc, mn)
         else:
-            sc, mn = (scaler.scale_, scaler.min_) if hasattr(scaler, "scale_") else scaler
-            sc = np.ascontiguousarray(sc, np.float64)
-            mn = np.ascontiguousarray(mn, np.float64)
-            if sc.shape != (X.shape[1],) or mn.shape != (X.shape[1],):
-                raise ValueError("scaler vectors must have one entry per marker")
-            _lib.check(L.ccb_ingest_scaled(h, _lib.ptr(X), N, X.shape[1], _lib.ptr(sc), _lib.ptr(mn), _lib.ptr(assign),
-                                           _lib.ptr(stage)), h)
-            self._views.add(X, assign, (sc, mn))
+            assign = np.empty(N, np.int32)
+            stage = np.empty(N, np.uint8)
+            _lib.check(L.ccb_ingest_ex(h, xp, dtype, 0, N, ld, _lib.ptr(sc), _lib.ptr(mn), _lib.ptr(assign),
+                                       _lib.ptr(stage)), h)
+        self._views.add(X, assign, None if sc is None else (sc, mn))
         self.last_assignment, self.last_stage = assign, stage
         self._lists = [None, None]
         logger.info("Finish online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
@@ -248,6 +293,23 @@ class HDDStream(object):
         self.last_data_timestamp = input_dataset_daystamp
         if run_offline:
             self.offline_clustering(input_dataset_daystamp)
+
+    def _ingest_tensor(self, X, xp, dtype, ld, sc, mn):
+        """ccb_ingest_ex on the rows of a CUDA tensor X: the handle's stream first waits for the work queued on the
+        current torch stream (whatever produced X), and the per-cell results come back to the host behind the engine."""
+        import torch
+
+        N = X.shape[0]
+        mine = torch.cuda.ExternalStream(self.stream_ptr, device=X.device)
+        cur = torch.cuda.current_stream(X.device)
+        assign_d = torch.empty(N, dtype=torch.int32, device=X.device)
+        stage_d = torch.empty(N, dtype=torch.uint8, device=X.device)
+        mine.wait_stream(cur)  # (after the allocations: earlier users of that memory on `cur` are done first)
+        _lib.check(_lib.lib().ccb_ingest_ex(self._h, xp, dtype, 1, N, ld, _lib.ptr(sc), _lib.ptr(mn), assign_d.data_ptr(),
+                                            stage_d.data_ptr()), self._h)
+        # the copies, and the release of the temporaries, are ordered on `cur` behind everything the handle queued
+        cur.wait_stream(mine)
+        return assign_d.cpu().numpy(), stage_d.cpu().numpy()
 
     def offline_clustering(self, dataset_daystamp):
         L, h = _lib.lib(), self._h

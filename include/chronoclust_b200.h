@@ -13,7 +13,7 @@
  *   ccb_create              HDDStream.__init__                      clustering/hddstream.py:30-67
  *   ccb_begin_timepoint     decay + downgrade + reset               clustering/hddstream.py:199-213,
  *                                                                    247-286, 512-549
- *   ccb_ingest[_device]     the ordered per-point loop              clustering/hddstream.py:220-237,
+ *   ccb_ingest[_device|_ex] the ordered per-point loop              clustering/hddstream.py:220-237,
  *                           (_add_to_pcore, _add_to_outlier,          288-343, 345-395, 397-430, 434-462
  *                            _upgrade_outlier_microcluster,          objects/microcluster.py:89-153,
  *                            _create_new_outlier_cluster)             167-197, 213-233
@@ -154,6 +154,19 @@ int ccb_ingest_scaled(ccb_handle *h, const double *X_raw, int64_t N, int64_t ld,
 /* Same with X, assign_uid and stage already resident on the handle's device (stage may be NULL). */
 int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
                       uint8_t *stage_dev);
+/* Element types of the rows handed to ccb_ingest_ex / ccb_colminmax_ex. */
+#define CCB_DTYPE_F64 0
+#define CCB_DTYPE_F32 1
+/* The ordered loop over N cells (clustering/hddstream.py:220-237, as ccb_ingest) for rows of either element type.
+ * X: row-major, leading dimension ld in ELEMENTS of dtype.  on_device != 0: X, assign_uid and stage are device pointers
+ * on the handle's device (as ccb_ingest_device), else host pointers (as ccb_ingest).  scale, min_: host [D], both NULL or
+ * both set (the transform of ccb_ingest_scaled, scaling/scaler.py:43-47).  Every element is widened to double first
+ * (exact): results are those of ccb_ingest[_scaled] on the widened rows, bit for bit.  X is never written.  Device-resident
+ * float64 rows without a scaler go to the engine as they are; any other device input is widened / scaled by one launch
+ * into a handle-owned buffer first; float32 host rows travel as float32 and are widened on the device.
+ * An unknown dtype, only one of scale / min_, or ld < D: CCB_EINVAL. */
+int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld,
+                  const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage);
 
 /* Offline phase over the current pcore list; returns the number of clusters. */
 int ccb_offline(ccb_handle *h, int64_t *n_clusters);
@@ -194,6 +207,10 @@ int ccb_nearest(int32_t device, void *stream, const double *X, int64_t N, int64_
  * The transform itself is part of ccb_ingest_scaled (below the handle API). */
 int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, int64_t ld, int32_t D, double *min_dev,
                   double *max_dev);
+/* The same for rows of either element type (CCB_DTYPE_*; ld in elements of dtype): the results are np.nanmin / np.nanmax
+ * of the rows widened to double.  An unknown dtype: CCB_EINVAL. */
+int ccb_colminmax_ex(int32_t device, void *stream, const void *X_dev, int32_t dtype, int64_t N, int64_t ld, int32_t D,
+                     double *min_dev, double *max_dev);
 
 /* Association scan (SURVEY 8f-1; replaces the inner loops of TrackByHistoricalAssociation.track_cluster_history,
  * tracking/cluster_tracker.py:127-144): for every CURRENT pcore microcluster q the index of the previous-timepoint
