@@ -70,6 +70,8 @@ SYMBOLS = {
     "ccb_offc_rowinfo": (C.c_int, [i32, vp, vp, i64, i64, i64, vp, vp]),
     "ccb_offc_fill": (C.c_int, [i32, vp, vp, i64, i64, i64, vp, vp, vp]),
     "ccb_off_clusters_csr": (C.c_int, [i32, vp, i64, vp, vp, vp, vp, vp, f64, i64, vp, vp, vp, vp]),
+    "ccb_group_stats": (C.c_int, [i32, vp, vp, i32, i64, i64, i32, vp, i32, i32, vp, vp, vp, vp, vp]),
+    "ccb_cluster_stats": (C.c_int, [vp, vp, i64, i32, i32, vp, vp, vp, vp, vp]),
 }
 
 

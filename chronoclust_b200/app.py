@@ -28,7 +28,7 @@ from decimal import ROUND_HALF_UP, Decimal
 import numpy as np
 import pandas as pd
 
-from . import _hostio
+from . import _hostio, cellstats
 from .hddstream import HDDStream
 from .objects import Cluster
 from .scaling import Scaler
@@ -111,9 +111,10 @@ class _PointsWriter(object):
     close = wait
 
 
-def _cell_labels(hddstream, clusters):
-    """Per input row the index of its lineage label (app.py:263-360 without the per-cell objects): row -> uid of the MC that
-    absorbed it (device array) -> pcore id -> the cluster holding that pcore id; everything else is 'None'."""
+def _pcore_labels(hddstream, clusters):
+    """Lineage label of every pcore MC -- its index into `labels`, in pcore list order, 0 = 'None' -- and the MCs' uids:
+    the one mapping behind both the per-cell table and cluster_statistics.csv.  A label shared by several clusters is
+    one entry of `labels`."""
     labels = ["None"]
     index_of = {}
     label_of_pcore = {}
@@ -124,11 +125,25 @@ def _cell_labels(hddstream, clusters):
         for pid in cluster.pcore_ids:
             label_of_pcore[int(pid)] = idx
     ids, uids = hddstream.export_arrays(0)[:2]
+    return np.array([label_of_pcore.get(pid, 0) for pid in ids.tolist()], np.int32), uids, labels
+
+
+def _cell_labels(hddstream, clusters):
+    """Per input row the index of its lineage label (app.py:263-360 without the per-cell objects): row -> uid of the MC that
+    absorbed it (device array) -> pcore id -> the cluster holding that pcore id; everything else is 'None'."""
+    label_idx, uids, labels = _pcore_labels(hddstream, clusters)
     assign = hddstream.last_assignment
     lut = np.zeros(int(max(int(assign.max(initial=0)), int(uids.max(initial=0)))) + 1, np.int32)
-    for pid, uid in zip(ids.tolist(), uids.tolist()):
-        lut[uid] = label_of_pcore.get(pid, 0)
+    for uid, idx in zip(uids.tolist(), label_idx.tolist()):
+        lut[uid] = idx
     return lut[assign], labels
+
+
+def _statistics_rows(timepoint, hddstream, clusters):
+    """cluster_statistics.csv rows of a timepoint: per lineage label the cells the per-cell table gives that label, their
+    count and per-marker medians and means, computed on the device; then the 'None' row."""
+    label_idx, _, labels = _pcore_labels(hddstream, clusters)
+    return cellstats.statistics_rows(timepoint, labels, hddstream.cluster_statistics(groups=label_idx - 1))
 
 
 def _result_rows(timepoint, clusters, scaler, gate_labels):
@@ -253,9 +268,11 @@ def setup_logger(log_dir):
 # ---- entry point ------------------------------------------------------------------------------------------------------------
 def run(data, output_directory, gating_centroid_file=None, normalise_data=True, restore_program=False,
         param_beta=0.8, param_delta=0.0, param_epsilon=0.03, param_lambda=0, param_k=1,
-        param_mu=0.001, param_pi=0, param_omicron=0.0, param_upsilon=1, device=0):
+        param_mu=0.001, param_pi=0, param_omicron=0.0, param_upsilon=1, device=0, cluster_statistics=False):
     """Run ChronoClust on a list of per-timepoint CSV files (in time order).  See the reference's app.run for the meaning of
-    every parameter; `device` (CUDA ordinal) is the only addition."""
+    every parameter.  Additions: `device` (CUDA ordinal); `cluster_statistics` -- also write cluster_statistics.csv, per
+    timepoint and lineage label the number of cells and their per-marker medians and means (the cells and values of
+    cluster_points_D{t}.csv), computed on the device, then the same for the cells in no cluster ('None')."""
     logger = setup_logger(os.path.join(output_directory, "logs"))
     logger.info("ChronoClust (B200 hot path) starts on cuda:%d with %d timepoint file(s)", device, len(data))
     values = (param_beta, param_delta, param_epsilon, param_lambda, param_k, param_mu, param_pi, param_omicron,
@@ -286,6 +303,11 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
         result_path = os.path.join(output_directory, "result.csv")
         with open(result_path, 'w') as f:
             csv.writer(f).writerow(header)
+        stats_path = os.path.join(output_directory, "cluster_statistics.csv")
+        if cluster_statistics:
+            with open(stats_path, 'w') as f:
+                csv.writer(f).writerow(['timepoint', 'tracking_by_lineage', 'cell_count'] +
+                                       [f'median_{a}' for a in attributes] + [f'mean_{a}' for a in attributes])
 
         scaler = None
         if normalise_data:
@@ -318,6 +340,9 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
             with open(result_path, 'a') as f:
                 csv.writer(f).writerows(_result_rows(timepoint, clusters, scaler, gate_labels))
 
+            if cluster_statistics:
+                with open(stats_path, 'a') as f:
+                    csv.writer(f).writerows(_statistics_rows(timepoint, hddstream, by_lineage.child_clusters))
             label_idx, labels = _cell_labels(hddstream, by_lineage.child_clusters)
             writer.submit(os.path.join(output_directory, f"cluster_points_D{timepoint}.csv"),
                           ['id', 'cluster_id'] + attributes, raw, scaler, label_idx, labels)

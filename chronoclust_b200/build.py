@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "api.cu")
 DEPS = [os.path.join(HERE, "csrc", f) for f in ("api.cu", "common.cuh", "nearest.cuh", "online.cuh", "offline.cuh",
-                                                "engine.cuh", "debug.h")]
+                                                "engine.cuh", "stats.cuh", "debug.h")]
 DEPS.append(os.path.join(os.path.dirname(HERE), "include", "chronoclust_b200.h"))
 SO = os.path.join(HERE, "libchronoclust_b200.so")
 SO_DEBUG = os.path.join(HERE, "libchronoclust_b200_debug.so")

@@ -21,6 +21,7 @@
 #include "offline.cuh"
 #include "online.cuh"
 #include "engine.cuh"
+#include "stats.cuh"
 
 using namespace ccb;
 
@@ -204,6 +205,14 @@ struct ccb_handle {
     Stream res_stream;  // device -> host copies of the per-cell results of a finished segment, behind the engine
     Grow<Pinned<unsigned char>> h_res; // page-locked bounce buffer of those results ([n] int32 assignments, then [n] stages)
     Grow<Dev<double>> d_scale;          // [2][CCB_MAX_D] scale_ / min_ of the scaled ingest
+    // where the rows and per-cell results of the last ingest live (ccb_cluster_stats): the double rows the engine read
+    // (d_X or the caller's device rows) and the assignments (d_assign or the caller's device buffer) -- recorded, not copied
+    struct {
+        const double *X = nullptr;
+        int64_t ld = 0, N = 0;
+        const int32_t *assign = nullptr;
+        bool scaled = false, valid = false;
+    } last;
     Event ev_seg[8];
     // offline results (host copies)
     int64_t off_M = 0;
@@ -1196,6 +1205,148 @@ __global__ void k_chain_probe(double *sink) {
     }
 }
 
+// ---- per-group statistics (stats.cuh) ---------------------------------------------------------------------------------
+constexpr int ST_MAX_Q = 64; // quantiles per call: the radix histograms of 2 + 2 nq ranks sit in shared memory
+
+int stats_args(ccb_handle *h, int64_t N, int64_t ld, int D, int G, int nq, const double *q, const int64_t *count,
+               const double *mean, const double *median, const double *quant) {
+    if (D < 1 || D > CCB_MAX_D || N < 0 || ld < D) return fail(h, CCB_EINVAL, "bad rows: N=%lld ld=%lld D=%d", (long long)N,
+                                                                (long long)ld, D);
+    if (N >= ((int64_t)1 << 31)) return fail(h, CCB_ELIMIT, "more than 2^31 - 1 cells in one call");
+    if (G < 1) return fail(h, CCB_EINVAL, "G = %d < 1", G);
+    if (nq < 0 || (nq > 0 && (!q || !quant))) return fail(h, CCB_EINVAL, "bad quantile arguments");
+    if (nq > ST_MAX_Q) return fail(h, CCB_ELIMIT, "%d quantiles > %d", nq, ST_MAX_Q);
+    for (int j = 0; j < nq; ++j)
+        if (!(q[j] >= 0.0 && q[j] <= 1.0)) return fail(h, CCB_EINVAL, "quantile %d = %g outside [0, 1]", j, q[j]);
+    if (!count || !mean || !median) return fail(h, CCB_EINVAL, "null output");
+    return CCB_OK;
+}
+
+// The pipeline of stats.cuh over the rows X [N][ld] (CCB_DTYPE_*) grouped by d_group [N] (device; values outside [0, G)
+// are skipped).  scale: device [2][CCB_MAX_D] (scale_, min_) of min-max scaled rows, or null.  Outputs are host arrays.
+// Synchronises s.  h (may be null) receives the error and counts the launches.  Arguments are checked by stats_args.
+int group_stats_run(ccb_handle *h, cudaStream_t s, const void *X, int32_t dtype, int64_t N, int64_t ld, int D,
+                    const int32_t *d_group, int G, int nq, const double *q, const double *scale, int64_t *count,
+                    double *mean, double *median, double *quant) {
+    int64_t launches = 0;
+    const int R = 2 + 2 * nq;
+    const unsigned gN = (unsigned)std::max<int64_t>(1, std::min<int64_t>((N + ST_THREADS - 1) / ST_THREADS, 148 * 8));
+    const unsigned gG = (unsigned)std::min<int64_t>((G + 255) / 256, 148 * 8);
+    // cells per group; slices; the groups that take the radix select and their slices (four scans of G + 1 entries)
+    Scratch qd(s), cs(s);
+    CK(h, qd.alloc((size_t)std::max(nq, 1) * 8));
+    if (nq) CK(h, cudaMemcpyAsync(qd.p, q, (size_t)nq * 8, cudaMemcpyHostToDevice, s));
+    CK(h, cs.alloc(((size_t)G + 4 * (size_t)G + 4 * ((size_t)G + 1) + 4) * 4));
+    unsigned *cnt = cs.as<unsigned>();
+    int32_t *a = reinterpret_cast<int32_t *>(cnt + G), *sc = a + 4 * (size_t)G, *tot = sc + 4 * ((size_t)G + 1);
+    CK(h, cudaMemsetAsync(cnt, 0, (size_t)G * 4, s));
+    const int smem_count = G <= ST_THREADS * 16 ? G * 4 : 0;
+    k_st_count<<<gN, ST_THREADS, smem_count, s>>>(d_group, N, G, smem_count != 0, cnt);
+    k_st_derive<<<gG, 256, 0, s>>>(cnt, G, a);
+    k_st_scan<<<4, 1024, 0, s>>>(a, G, sc, G, tot);
+    launches += 3;
+    CKL(h);
+    int32_t t4[4];
+    CK(h, cudaMemcpyAsync(t4, tot, sizeof t4, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
+    const int64_t Nv = t4[0], NS = t4[1], L = t4[2], NLS = t4[3];
+
+    StGeom geo{};
+    geo.cnt = cnt, geo.goff = sc, geo.soff = sc + (G + 1), geo.Nv = Nv, geo.D = D;
+    Scratch tab(s), srt(s), ks(s), part(s), outd(s), sel_mem(s);
+    CK(h, tab.alloc((size_t)(NS + L + 2 * NLS + 1) * 4));
+    int32_t *slice_group = tab.as<int32_t>(), *large_group = slice_group + NS, *large_slice = large_group + L,
+            *large_slice_l = large_slice + NLS;
+    k_st_slices<<<gG, 256, 0, s>>>(sc, G, slice_group, large_group, large_slice, large_slice_l);
+    launches++;
+    geo.slice_group = slice_group;
+    if (Nv > 0) {
+        // stable LSD counting sort of the grouped rows by group, 8 bits a pass; the first pass drops the other rows
+        int bits = 0;
+        while (bits < 31 && ((int64_t)(G - 1) >> bits) != 0) ++bits;
+        const int passes = std::max(1, (bits + 7) / 8);
+        const int64_t nt_max = (N + ST_TILE - 1) / ST_TILE;
+        CK(h, srt.alloc((size_t)(4 * Nv + 2 * 256 * nt_max + 1) * 4));
+        int32_t *kb[2] = {srt.as<int32_t>(), srt.as<int32_t>() + Nv}, *vb[2] = {kb[1] + Nv, kb[1] + 2 * Nv};
+        int32_t *th = vb[1] + Nv, *toff = th + 256 * nt_max;
+        for (int p = 0; p < passes; ++p) {
+            const int64_t n = p ? Nv : N;
+            const int nt = (int)((n + ST_TILE - 1) / ST_TILE);
+            int32_t *ko = kb[p & 1], *vo = vb[p & 1];
+            if (p == 0) {
+                k_st_sort_hist<true><<<nt, ST_THREADS, 0, s>>>(d_group, n, G, 0, th, nt);
+            } else {
+                k_st_sort_hist<false><<<nt, ST_THREADS, 0, s>>>(kb[(p - 1) & 1], n, G, 8 * p, th, nt);
+            }
+            k_st_scan<<<1, 1024, 0, s>>>(th, 0, toff, 256 * nt, tot);
+            if (p == 0) {
+                k_st_sort_scatter<true><<<nt, ST_THREADS, 0, s>>>(d_group, nullptr, n, G, 0, toff, nt, ko, vo);
+            } else {
+                k_st_sort_scatter<false><<<nt, ST_THREADS, 0, s>>>(kb[(p - 1) & 1], vb[(p - 1) & 1], n, G, 8 * p, toff, nt,
+                                                                   ko, vo);
+            }
+            launches += 3;
+        }
+        geo.perm = vb[(passes - 1) & 1];
+        CKL(h);
+    }
+    // keys [D][Nv] in group order, partial sums / NaN counts [NS][D]
+    CK(h, ks.alloc(std::max<size_t>((size_t)D * Nv, 1) * 8));
+    CK(h, part.alloc(std::max<size_t>((size_t)NS * D, 1) * 12));
+    uint64_t *keys = ks.as<uint64_t>();
+    double *psum = part.as<double>();
+    int32_t *pnan = reinterpret_cast<int32_t *>(psum + (size_t)NS * D);
+    if (NS > 0) {
+        const size_t smem = (size_t)ST_CHUNK * (D + 1) * 8;
+        if (dtype == CCB_DTYPE_F32)
+            k_st_gather<float><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const float *>(X), ld, scale,
+                                                                    scale ? scale + CCB_MAX_D : nullptr, keys, psum, pnan);
+        else
+            k_st_gather<double><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const double *>(X), ld, scale,
+                                                                     scale ? scale + CCB_MAX_D : nullptr, keys, psum, pnan);
+        launches++;
+    }
+    // outputs
+    const size_t GD = (size_t)G * D;
+    CK(h, outd.alloc(GD * (2 + (size_t)nq) * 8));
+    StOut out{};
+    out.q = qd.as<double>(), out.nq = nq, out.G = G;
+    out.mean = outd.as<double>(), out.median = out.mean + GD, out.quant = out.median + GD;
+    k_st_small<<<(unsigned)G, ST_THREADS, 0, s>>>(geo, keys, psum, pnan, out);
+    launches++;
+    if (L > 0) {
+        const int64_t items = L * D * R;
+        CK(h, sel_mem.alloc((size_t)items * (16 + 256 * 4)));
+        StSel sel{};
+        sel.pre = sel_mem.as<uint64_t>();
+        sel.rem = reinterpret_cast<int64_t *>(sel.pre + items);
+        sel.hist = reinterpret_cast<unsigned *>(sel.rem + items);
+        sel.large_group = large_group, sel.large_slice = large_slice, sel.large_slice_l = large_slice_l, sel.R = R;
+        CK(h, cudaMemsetAsync(sel.hist, 0, (size_t)items * 256 * 4, s));
+        const unsigned gi = (unsigned)std::min<int64_t>((items + 255) / 256, 148 * 8);
+        k_st_rsel_init<<<gi, 256, 0, s>>>(geo, sel, out.q, items);
+        const size_t smem = (size_t)R * (256 * 4 + 8);
+        CK(h, cudaFuncSetAttribute(k_st_rsel_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        for (int shift = 56; shift >= 0; shift -= 8) {
+            k_st_rsel_hist<<<dim3((unsigned)NLS, (unsigned)D), ST_THREADS, smem, s>>>(geo, sel, keys, shift);
+            k_st_rsel_fix<<<gi, 256, 0, s>>>(sel, items, shift);
+        }
+        k_st_large_finish<<<(unsigned)std::min<int64_t>((L * D + 255) / 256, 148 * 8), 256, 0, s>>>(geo, sel, psum, pnan, out,
+                                                                                                     L * D);
+        launches += 2 + 2 * 8;
+    }
+    CKL(h);
+    std::vector<unsigned> hc(G);
+    CK(h, cudaMemcpyAsync(hc.data(), cnt, (size_t)G * 4, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaMemcpyAsync(mean, out.mean, GD * 8, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaMemcpyAsync(median, out.median, GD * 8, cudaMemcpyDeviceToHost, s));
+    if (nq) CK(h, cudaMemcpyAsync(quant, out.quant, GD * nq * 8, cudaMemcpyDeviceToHost, s));
+    CK(h, cudaStreamSynchronize(s));
+    for (int g = 0; g < G; ++g) count[g] = hc[g];
+    if (h) h->st.kernel_launches += launches;
+    return CCB_OK;
+}
+
 } // namespace
 
 // =====================================================================================================
@@ -1354,6 +1505,7 @@ int ccb_reset(ccb_handle *h) {
     }
     CK(h, cudaStreamSynchronize(h->stream));
     h->have_params = false;
+    h->last.valid = false;
     h->off_M = 0;
     h->cl_off.assign(1, 0);
     h->cl_members.clear();
@@ -1395,6 +1547,7 @@ int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, in
     h->omicron = omicron;
     h->pi = pi;
     h->have_params = true;
+    h->last.valid = false;
     if (!decay) return CCB_OK;
     cudaStream_t s = h->stream;
     if ((rc = sync_ctl(h))) return rc;
@@ -1468,14 +1621,31 @@ int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device
         CK(h, cudaMemcpyAsync(h->d_scale + CCB_MAX_D, min_, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
     }
     const double *d_sc = scale ? h->d_scale.p : nullptr, *d_sh = scale ? h->d_scale + CCB_MAX_D : nullptr;
-    if (!on_device) return ingest_host(h, X, dtype, N, ld, assign_uid, stage, d_sc, d_sh);
+    h->last.valid = false;
+    auto record = [&](const double *rows, int64_t ldr, const int32_t *assign) {
+        h->last.X = rows, h->last.ld = ldr, h->last.N = N, h->last.assign = assign, h->last.scaled = scale != nullptr;
+        h->last.valid = true;
+    };
+    if (!on_device) {
+        // (ingest_host leaves the rows in d_X: float64 ones with the caller's leading dimension, float32 ones with D)
+        if ((rc = ingest_host(h, X, dtype, N, ld, assign_uid, stage, d_sc, d_sh))) return rc;
+        record(h->d_X, dtype == CCB_DTYPE_F32 ? h->D : ld, h->d_assign);
+        return CCB_OK;
+    }
     // device-resident rows: float64 without a scaler go to the engine as they are; anything else is staged into d_X
     // (leading dimension D) by one launch -- the caller's buffer is never written
-    if (dtype == CCB_DTYPE_F64 && !scale) return ingest_core_bsv(h, static_cast<const double *>(X), N, ld, assign_uid, stage);
+    if (dtype == CCB_DTYPE_F64 && !scale) {
+        const double *Xd = static_cast<const double *>(X);
+        if ((rc = ingest_core_bsv(h, Xd, N, ld, assign_uid, stage))) return rc;
+        record(Xd, ld, assign_uid);
+        return CCB_OK;
+    }
     CK(h, h->d_X.ensure(((size_t)N * h->D + 2) * 8));
     stage_rows(h, dtype, X, ld, h->d_X, h->D, N, d_sc, d_sh);
     CKL(h);
-    return ingest_core_bsv(h, h->d_X, N, h->D, assign_uid, stage);
+    if ((rc = ingest_core_bsv(h, h->d_X, N, h->D, assign_uid, stage))) return rc;
+    record(h->d_X, h->D, assign_uid);
+    return CCB_OK;
 }
 
 int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
@@ -1670,6 +1840,7 @@ int ccb_import_list(ccb_handle *h, int32_t which, int64_t n, const int64_t *ids,
     int rc;
     if ((rc = enter(h))) return rc;
     if (n < 0) return fail(h, CCB_EINVAL, "bad argument");
+    h->last.valid = false;
     if ((rc = sync_ctl(h)) || (rc = grow_store(h, which != 0, 0, std::max<int64_t>(n, 1)))) return rc;
     const int D = h->D;
     Store &S = which ? h->O[h->ocur] : h->P[h->pcur];
@@ -2128,6 +2299,50 @@ int ccb_off_clusters_csr(int32_t device, void *stream, int64_t M, const int64_t 
     return rc ? rc
               : off_clusters_csr(nullptr, s, (int)M, off, col, total, iso, core, submask_all, k > 1.0, pi, label, order, cl_off,
                                  n_cl);
+}
+
+int ccb_group_stats(int32_t device, void *stream, const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t D,
+                    const int32_t *group, int32_t G, int32_t nq, const double *q, int64_t *count, double *mean, double *median,
+                    double *quant) {
+    if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(nullptr, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
+    if (int rc = stats_args(nullptr, N, ld, D, G, nq, q, count, mean, median, quant)) return rc;
+    if (N > 0 && (!X || !group)) return fail(nullptr, CCB_EINVAL, "null rows or groups");
+    if (int rc = enter_device(device)) return rc;
+    return group_stats_run(nullptr, (cudaStream_t)stream, X, dtype, N, ld, D, group, G, nq, q, nullptr, count, mean, median,
+                           quant);
+}
+
+int ccb_cluster_stats(ccb_handle *h, const int32_t *group_of_pcore, int64_t n_pcore, int32_t G, int32_t nq, const double *q,
+                      int64_t *count, double *mean, double *median, double *quant) {
+    int rc;
+    if ((rc = enter(h))) return rc;
+    if (!h->last.valid)
+        return fail(h, CCB_ESTATE, "no ingest since the last ccb_begin_timepoint / ccb_reset / ccb_import_list");
+    if (G < 0 || G == INT32_MAX) return fail(h, CCB_EINVAL, "G = %d", G);
+    if ((rc = stats_args(h, h->last.N, h->last.ld, h->D, G + 1, nq, q, count, mean, median, quant))) return rc;
+    if ((rc = sync_ctl(h))) return rc;
+    const int np = h->h_ctl->n_pcore;
+    if (n_pcore != np) return fail(h, CCB_EINVAL, "n_pcore = %lld, the pcore list holds %d", (long long)n_pcore, np);
+    if (np > 0 && !group_of_pcore) return fail(h, CCB_EINVAL, "null group_of_pcore");
+    for (int p = 0; p < np; ++p)
+        if (group_of_pcore[p] >= G) return fail(h, CCB_EINVAL, "group_of_pcore[%d] = %d >= G = %d", p, group_of_pcore[p], G);
+    cudaStream_t s = h->stream;
+    const int64_t N = h->last.N, nlut = std::max<int64_t>(h->h_ctl->outlier_last_id, 1);
+    Scratch sc(s);
+    CK(h, sc.alloc(((size_t)nlut + np + N) * 4));
+    int32_t *lut = sc.as<int32_t>(), *gop = lut + nlut, *group = gop + np;
+    const unsigned gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>((std::max<int64_t>(nlut, N) + 255) / 256, 148 * 8));
+    k_st_lut_fill<<<gx, 256, 0, s>>>(lut, nlut, G);
+    if (np > 0) {
+        CK(h, cudaMemcpyAsync(gop, group_of_pcore, (size_t)np * 4, cudaMemcpyHostToDevice, s));
+        k_st_lut_pcore<<<(np + 255) / 256, 256, 0, s>>>(h->P[h->pcur].uid, gop, np, nlut, G, lut);
+        h->st.kernel_launches++;
+    }
+    k_st_cell_group<<<gx, 256, 0, s>>>(h->last.assign, N, lut, nlut, G, group);
+    h->st.kernel_launches += 2;
+    CKL(h);
+    return group_stats_run(h, s, h->last.X, CCB_DTYPE_F64, N, h->last.ld, h->D, group, G + 1, nq, q,
+                           h->last.scaled ? h->d_scale.p : nullptr, count, mean, median, quant);
 }
 
 } // extern "C"

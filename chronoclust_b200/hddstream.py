@@ -13,7 +13,7 @@ import sys
 
 import numpy as np
 
-from . import _lib
+from . import _lib, cellstats
 from .objects import FinalCluster, Microcluster
 
 
@@ -143,6 +143,7 @@ class HDDStream(object):
         self.last_assignment = None  # uid of the MC every row of the last call went to
         self.last_stage = None
         self.last_cluster_label = None  # cluster index of every pcore MC (list order) after the offline phase
+        self._last_device_input = None  # (rows, assignments) of the last CUDA-tensor ingest, read by cluster_statistics
 
     # ------------------------------------------------------------------------------------------
     def __del__(self):
@@ -175,6 +176,7 @@ class HDDStream(object):
         self._views = _PointsView()
         self._lists = [None, None]
         self.last_assignment = self.last_stage = self.last_cluster_label = None
+        self._last_device_input = None
         if self.dataset_dimensionality:
             self._ensure_handle(self.dataset_dimensionality)
             self._import(0, pcore)
@@ -277,6 +279,7 @@ class HDDStream(object):
                                          float(factor)), h)
         N = X.shape[0]
         logger.info("Starting online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
+        self._last_device_input = None
         if on_device:
             assign, stage = self._ingest_tensor(X, xp, dtype, ld, sc, mn)
         else:
@@ -309,6 +312,7 @@ class HDDStream(object):
                                             stage_d.data_ptr()), self._h)
         # the copies, and the release of the temporaries, are ordered on `cur` behind everything the handle queued
         cur.wait_stream(mine)
+        self._last_device_input = (X, assign_d)  # the handle reads both again in cluster_statistics
         return assign_d.cpu().numpy(), stage_d.cpu().numpy()
 
     def offline_clustering(self, dataset_daystamp):
@@ -353,6 +357,7 @@ class HDDStream(object):
         self.last_data_timestamp = 0
         self.dataset_size = 0
         self.last_assignment = self.last_stage = self.last_cluster_label = None
+        self._last_device_input = None
 
     @property
     def stream_ptr(self):
@@ -464,3 +469,28 @@ class HDDStream(object):
         uniq, inv = np.unique(a, return_inverse=True)
         m = np.array([lut.get(int(u), -1) for u in uniq], np.int32)
         return m[inv]
+
+    def cluster_statistics(self, quantiles=(), groups=None):
+        """Per-cluster statistics of the cells of the last online_microcluster_maintenance call, computed on the GPU:
+        GroupStats(count, mean, median, quantiles) (chronoclust_b200.cellstats) with one row per cluster -- row c is
+        final_clusters[c] -- and a last row for the cells in no cluster.  The values are the cells as the engine read
+        them, widened to float64 and, with a scaler, brought back to the input scale ((x - min_) / scale_, as
+        cluster_points_D{t}.csv holds them); median and quantiles are numpy's bit for bit (see group_statistics).
+
+        groups: optional integer array over the pcore list (pcore_MC order, -1 = no group) replacing the clusters of the
+        offline phase; the result then has max(groups) + 2 rows.  ValueError without an offline result or `groups`;
+        CCBError when no cells have been ingested since the handle's last timepoint start, reset or restore."""
+        if groups is None:
+            if self.last_cluster_label is None:
+                raise ValueError("no offline result: run the offline phase or pass groups")
+            groups, G = self.last_cluster_label, len(self.final_clusters)
+        else:
+            groups = np.asarray(groups)
+            if groups.ndim != 1 or groups.dtype.kind not in "iu":
+                raise ValueError("groups must be a 1-D integer array over the pcore list")
+            if len(groups) and int(groups.min()) < -1:
+                raise ValueError("groups must be >= -1")
+            G = int(groups.max()) + 1 if len(groups) else 0
+        if self._h is None:
+            raise _lib.CCBError("no cells have been ingested")
+        return cellstats.cluster_statistics(self._h, self.dataset_dimensionality, groups, G, quantiles)

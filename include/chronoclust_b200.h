@@ -30,6 +30,8 @@
  *                           + the strict-< argmin of the scans       clustering/hddstream.py:311-328,371-375
  *   ccb_off_*               the row-sharded stages of PreDeCon      clustering/predecon.py:136-217
  *                           (multi-GPU offline path, config C4)
+ *   ccb_cluster_stats /     (extension) per-cluster cell counts,    replaces grouping cluster_points_D{t}.csv
+ *   ccb_group_stats         means, medians, quantiles of a timepoint  on the host after a run
  *
  * The derived constants (epsilon**2, upsilon*epsilon, delta**2, 2**(-lambda*dt), mu*N, omicron*N_prev,
  * round(pi)) are evaluated by the Python host with Python's own float semantics, exactly where the
@@ -190,6 +192,20 @@ int ccb_export_clusters(ccb_handle *h, int64_t *off, int64_t *members, double *w
 /* White-box: core flags [M], neighbour / weighted-neighbour matrices [M*M] bytes, subspace weights [M][D]. */
 int ccb_export_offline(ccb_handle *h, uint8_t *core, uint8_t *nbr, uint8_t *wnbr, double *subw);
 
+/* Per-cluster statistics of the cells of the LAST ingest call (extension): the cells are grouped through
+ * group_of_pcore [n_pcore] (host, pcore list order as ccb_export_list(0) returns it, -1 = in no group, else < G): a cell
+ * whose assigned MC sits in the pcore list at position p belongs to group group_of_pcore[p]; every other cell (absorbed by
+ * an outlier MC, or by a pcore MC in no group) to the extra last row G.  Outputs as ccb_group_stats with G + 1 rows.
+ * The values are the rows the engine read widened to double; after a scaled ingest they are (x - min_) / scale_ (two
+ * roundings: sklearn's MinMaxScaler.inverse_transform), i.e. the values app.run writes to cluster_points_D{t}.csv.
+ * The rows and assignments are read where the ingest left them: the handle's own buffers, or, for device input
+ * (ccb_ingest_ex with on_device, ccb_ingest_device), the CALLER's device rows and assignment buffer, which must still hold
+ * what they held at the ingest.  Reads only: nothing later computed by the handle changes.
+ * CCB_ESTATE unless an ingest happened since the last ccb_begin_timepoint / ccb_reset / ccb_import_list; CCB_EINVAL if
+ * n_pcore != the pcore count, G < 0, a group_of_pcore entry >= G, or a q outside [0, 1].  Synchronises the handle's stream. */
+int ccb_cluster_stats(ccb_handle *h, const int32_t *group_of_pcore, int64_t n_pcore, int32_t G, int32_t nq, const double *q,
+                      int64_t *count, double *mean, double *median, double *quant);
+
 /* ---------------------------------------------------------------------------------------------
  * Stateless device-pointer entry points (all pointers are device memory on `device`; stream is a
  * cudaStream_t or NULL).  These are what bench.py times for the roofline and what the multi-GPU
@@ -226,6 +242,19 @@ int ccb_assoc_nearest(int32_t device, void *stream, const double *cur_cen, const
  * band and re-evaluates the few near-ties with the reference expression itself. */
 int ccb_assoc_nearest2(int32_t device, void *stream, const double *cur_cen, const uint64_t *cur_prefmask, int64_t Q,
                        const double *prev_cen, int64_t P, int32_t D, double k, int32_t *best, double *dist, double *dist2);
+
+/* Per-group statistics of device rows (extension).  X [N][ld] (CCB_DTYPE_*, ld in elements) on `device`, group [N] int32
+ * on the device: -1 (or any value outside [0, G)) = skip the row, else its group.  q: host [nq], each in [0, 1].
+ * Outputs (host): count [G]; mean / median [G][D]; quant [nq][G][D] (may be NULL when nq == 0).
+ *   median = np.median of the group's values, bit for bit ((a + b) / 2 of the middle two for an even count);
+ *   quant  = np.quantile(values, q, method="linear"), bit for bit (numpy's index rule and _lerp);
+ *   mean   = np.mean up to rounding, summed in a fixed order: identical from call to call.
+ * A group without cells: count 0, NaN elsewhere; a NaN among a marker's values: NaN mean / median / quantiles there.
+ * CCB_EINVAL: bad shapes, G < 1, an unknown dtype, a q outside [0, 1] (or NaN); CCB_ELIMIT: N >= 2^31 or nq > 64.
+ * Scratch from the stream-ordered pool, about N * (8 D + 24) bytes.  Synchronises `stream`. */
+int ccb_group_stats(int32_t device, void *stream, const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t D,
+                    const int32_t *group, int32_t G, int32_t nq, const double *q, int64_t *count, double *mean, double *median,
+                    double *quant);
 
 /* FP64 pipe microbenchmark for the roofline denominators: mode 0 = DFMA stream (2 flop/instr), mode 1 =
  * separate DMUL + DADD (1 flop/instr, the only form the parity contract allows).  Launches `blocks` CTAs of
