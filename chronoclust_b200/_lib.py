@@ -49,6 +49,7 @@ SYMBOLS = {
     "ccb_ingest": (C.c_int, [vp, vp, i64, i64, vp, vp]),
     "ccb_ingest_device": (C.c_int, [vp, vp, i64, i64, vp, vp]),
     "ccb_ingest_ex": (C.c_int, [vp, vp, i32, i32, i64, i64, vp, vp, vp, vp]),
+    "ccb_ingest_cols": (C.c_int, [vp, vp, i32, i32, i64, i64, i32, vp, vp, vp, vp, vp]),
     "ccb_offline": (C.c_int, [vp, C.POINTER(i64)]),
     "ccb_counts": (C.c_int, [vp, C.POINTER(i64 * 4)]),
     "ccb_export_list": (C.c_int, [vp, i32] + [vp] * 7),

@@ -70,12 +70,30 @@ class _Timepoints(object):
         self._pool.shutdown(wait=False)
 
 
-def _fit_joint_scaler(timepoints, wanted):
-    """MinMaxScaler over all timepoints jointly (scaler.py:27-36), fed one parsed array at a time."""
+def _fit_joint_scaler(timepoints, wanted, cols=None):
+    """MinMaxScaler over all timepoints jointly (scaler.py:27-36), fed one parsed array at a time -- on the clustering
+    columns `cols` only when given (the fit is column-wise: the vectors are those of a fit on files holding only them)."""
     scaler = Scaler()
     for t in wanted:
-        scaler.scaler.partial_fit(timepoints.cells(t))
+        cells = timepoints.cells(t)
+        scaler.scaler.partial_fit(cells if cols is None else cells[:, cols])
     return scaler
+
+
+def clustering_columns(attributes, clustering_markers):
+    """Column indices of `clustering_markers` (names from the first file's header, in the order given), or None for every
+    column.  ValueError for an unknown or repeated name, or an empty list."""
+    if clustering_markers is None:
+        return None
+    names = [str(m) for m in clustering_markers]
+    if not names:
+        raise ValueError("clustering_markers is empty")
+    unknown = [m for m in names if m not in attributes]
+    if unknown:
+        raise ValueError(f"clustering_markers not in the header of the first file: {unknown}")
+    if len(set(names)) != len(names):
+        raise ValueError(f"clustering_markers repeats a name: {names}")
+    return [attributes.index(m) for m in names]
 
 
 # ---- outputs --------------------------------------------------------------------------------------------------------------
@@ -86,12 +104,9 @@ class _PointsWriter(object):
         self._thread = None
         self._error = None
 
-    def _job(self, path, header, raw, scaler, label_idx, labels):
+    def _job(self, path, header, raw, scaler, cols, label_idx, labels):
         try:
-            values = raw
-            if scaler is not None:  # what the reference writes: inverse_transform(transform(raw)) (app.py:175, 299-301)
-                values = scaler.reverse_scaling(scaler.scale_data(raw))
-            _hostio.write_points_csv(path, header, values, label_idx, labels)
+            _hostio.write_points_csv(path, header, points_values(raw, scaler, cols), label_idx, labels)
         except BaseException as exc:  # surfaced by the next submit / by close
             self._error = exc
 
@@ -109,6 +124,29 @@ class _PointsWriter(object):
         self._thread.start()
 
     close = wait
+
+
+def output_headers(attributes, markers, gating):
+    """Header rows of result.csv (centroid columns: the clustering `markers`), cluster_points_D{t}.csv and
+    cluster_statistics.csv (every column of the files, `attributes`)."""
+    result = ['timepoint', 'cumulative_size', 'pcore_ids', 'pref_dimensions'] + markers + \
+             ['tracking_by_lineage', 'tracking_by_association'] + (['predicted_label'] if gating else [])
+    stats = ['timepoint', 'tracking_by_lineage', 'cell_count'] + [f'median_{a}' for a in attributes] + \
+            [f'mean_{a}' for a in attributes]
+    return result, ['id', 'cluster_id'] + attributes, stats
+
+
+def points_values(raw, scaler, cols=None):
+    """The values of cluster_points_D{t}.csv for the parsed cells `raw`: with a scaler, the clustering columns (`cols`, or
+    every column) hold inverse_transform(transform(x)), what the reference writes (app.py:175, 299-301); every other
+    column holds the parsed value."""
+    if scaler is None:
+        return raw
+    if cols is None:
+        return scaler.reverse_scaling(scaler.scale_data(raw))
+    values = np.array(raw, np.float64)
+    values[:, cols] = scaler.reverse_scaling(scaler.scale_data(raw[:, cols]))
+    return values
 
 
 def _pcore_labels(hddstream, clusters):
@@ -268,11 +306,16 @@ def setup_logger(log_dir):
 # ---- entry point ------------------------------------------------------------------------------------------------------------
 def run(data, output_directory, gating_centroid_file=None, normalise_data=True, restore_program=False,
         param_beta=0.8, param_delta=0.0, param_epsilon=0.03, param_lambda=0, param_k=1,
-        param_mu=0.001, param_pi=0, param_omicron=0.0, param_upsilon=1, device=0, cluster_statistics=False):
+        param_mu=0.001, param_pi=0, param_omicron=0.0, param_upsilon=1, device=0, cluster_statistics=False,
+        clustering_markers=None):
     """Run ChronoClust on a list of per-timepoint CSV files (in time order).  See the reference's app.run for the meaning of
     every parameter.  Additions: `device` (CUDA ordinal); `cluster_statistics` -- also write cluster_statistics.csv, per
     timepoint and lineage label the number of cells and their per-marker medians and means (the cells and values of
-    cluster_points_D{t}.csv), computed on the device, then the same for the cells in no cluster ('None')."""
+    cluster_points_D{t}.csv), computed on the device, then the same for the cells in no cluster ('None');
+    `clustering_markers` -- names of the markers to cluster on, from the first file's header, in the order given (default:
+    every column).  The scaler is fitted on them, the gating file is read on them and result.csv's centroid columns are
+    them; cluster_points_D{t}.csv and cluster_statistics.csv still cover every column of the files, the others holding
+    the parsed values.  An unknown or repeated name raises ValueError before any clustering."""
     logger = setup_logger(os.path.join(output_directory, "logs"))
     logger.info("ChronoClust (B200 hot path) starts on cuda:%d with %d timepoint file(s)", device, len(data))
     values = (param_beta, param_delta, param_epsilon, param_lambda, param_k, param_mu, param_pi, param_omicron,
@@ -297,22 +340,22 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
     writer = _PointsWriter()
     try:
         attributes = timepoints.attributes()
-        gates = _read_gates(gating_centroid_file, attributes)
-        header = ['timepoint', 'cumulative_size', 'pcore_ids', 'pref_dimensions'] + attributes + \
-                 ['tracking_by_lineage', 'tracking_by_association'] + (['predicted_label'] if gating_centroid_file else [])
+        cols = clustering_columns(attributes, clustering_markers)
+        markers = attributes if cols is None else [attributes[c] for c in cols]
+        gates = _read_gates(gating_centroid_file, markers)
+        header, points_header, stats_header = output_headers(attributes, markers, gating_centroid_file)
         result_path = os.path.join(output_directory, "result.csv")
         with open(result_path, 'w') as f:
             csv.writer(f).writerow(header)
         stats_path = os.path.join(output_directory, "cluster_statistics.csv")
         if cluster_statistics:
             with open(stats_path, 'w') as f:
-                csv.writer(f).writerow(['timepoint', 'tracking_by_lineage', 'cell_count'] +
-                                       [f'median_{a}' for a in attributes] + [f'mean_{a}' for a in attributes])
+                csv.writer(f).writerow(stats_header)
 
         scaler = None
         if normalise_data:
             logger.info("Fitting the joint min-max scaler over all timepoints")
-            scaler = _fit_joint_scaler(timepoints, range(len(data)))
+            scaler = _fit_joint_scaler(timepoints, range(len(data)), cols)
 
         for timepoint in range(len(data)):
             if resumed and hddstream.last_data_timestamp >= timepoint:
@@ -322,7 +365,8 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
             logger.info("Timepoint %d: %d cells x %d markers", timepoint, raw.shape[0], raw.shape[1])
 
             # ---- the hot path: online + offline clustering on the GPU (the min-max transform rides along on the device)
-            hddstream.online_microcluster_maintenance(raw, timepoint, scaler=scaler.scaler if scaler else None)
+            hddstream.online_microcluster_maintenance(raw, timepoint, scaler=scaler.scaler if scaler else None,
+                                                      columns=cols)
 
             pcore_by_id = {mc.id[0]: mc for mc in hddstream.pcore_MC}
             for found in hddstream.final_clusters:
@@ -345,7 +389,7 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
                     csv.writer(f).writerows(_statistics_rows(timepoint, hddstream, by_lineage.child_clusters))
             label_idx, labels = _cell_labels(hddstream, by_lineage.child_clusters)
             writer.submit(os.path.join(output_directory, f"cluster_points_D{timepoint}.csv"),
-                          ['id', 'cluster_id'] + attributes, raw, scaler, label_idx, labels)
+                          points_header, raw, scaler, cols, label_idx, labels)
             timepoints.release(timepoint)
 
             by_lineage.transfer_child_to_parent()

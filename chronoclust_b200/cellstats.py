@@ -94,7 +94,8 @@ def group_statistics(X, groups, n_groups, quantiles=()):
 
 
 def cluster_statistics(h, D, group_of_pcore, G, quantiles=()):
-    """ccb_cluster_stats on handle h: G + 1 rows, the last one the cells in no group (see HDDStream.cluster_statistics)."""
+    """ccb_cluster_stats on handle h: G + 1 rows, the last one the cells in no group (see HDDStream.cluster_statistics).
+    D: the width of the rows of the handle's last ingest (W after a column-subset ingest)."""
     q = quantile_array(quantiles)
     gop = np.ascontiguousarray(group_of_pcore, dtype=np.int32)
     out = _outputs(G + 1, D, len(q))

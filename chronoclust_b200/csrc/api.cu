@@ -181,7 +181,10 @@ struct ccb_handle {
     bool have_params = false;
     // ingest buffers
     Grow<Dev<double>> d_X;
-    Grow<Dev<float>> d_X32; // float32 host rows as copied, before k_stage_rows widens them into d_X
+    // host rows as copied (float32 ones, and the full-width rows of a column-subset ingest), before k_stage_rows gathers /
+    // widens them into d_X
+    Grow<Dev<unsigned char>> d_stg;
+    Grow<Dev<int32_t>> d_cols; // [CCB_MAX_D] column map of a column-subset ingest
     Grow<Dev<int32_t>> d_assign;
     Grow<Dev<uint8_t>> d_stage;
     Grow<Dev<int32_t>> d_pnew, d_pfin, d_onew; // kernel 3 plan codes
@@ -204,13 +207,17 @@ struct ccb_handle {
     Stream copy_stream; // host -> device segments of ccb_ingest, ahead of the engine
     Stream res_stream;  // device -> host copies of the per-cell results of a finished segment, behind the engine
     Grow<Pinned<unsigned char>> h_res; // page-locked bounce buffer of those results ([n] int32 assignments, then [n] stages)
-    Grow<Dev<double>> d_scale;          // [2][CCB_MAX_D] scale_ / min_ of the scaled ingest
+    // [4][CCB_MAX_D] scale_ / min_ of the scaled ingest; after a column-subset ingest also scale_ / min_ by source column
+    Grow<Dev<double>> d_scale;
     // where the rows and per-cell results of the last ingest live (ccb_cluster_stats): the double rows the engine read
-    // (d_X or the caller's device rows) and the assignments (d_assign or the caller's device buffer) -- recorded, not copied
+    // (d_X or the caller's device rows) and the assignments (d_assign or the caller's device buffer) -- recorded, not copied.
+    // After a column-subset ingest, the full-width rows instead (d_stg or the caller's device rows), in their own dtype.
     struct {
-        const double *X = nullptr;
+        const void *X = nullptr;
         int64_t ld = 0, N = 0;
         const int32_t *assign = nullptr;
+        int32_t dtype = CCB_DTYPE_F64, W = 0;
+        uint64_t colmask = 0; // the clustering columns of a column-subset ingest (0: none)
         bool scaled = false, valid = false;
     } last;
     Event ev_seg[8];
@@ -1223,10 +1230,10 @@ int stats_args(ccb_handle *h, int64_t N, int64_t ld, int D, int G, int nq, const
 }
 
 // The pipeline of stats.cuh over the rows X [N][ld] (CCB_DTYPE_*) grouped by d_group [N] (device; values outside [0, G)
-// are skipped).  scale: device [2][CCB_MAX_D] (scale_, min_) of min-max scaled rows, or null.  Outputs are host arrays.
+// are skipped).  xf: the per-column transform of the values (StXf in stats.cuh).  Outputs are host arrays.
 // Synchronises s.  h (may be null) receives the error and counts the launches.  Arguments are checked by stats_args.
 int group_stats_run(ccb_handle *h, cudaStream_t s, const void *X, int32_t dtype, int64_t N, int64_t ld, int D,
-                    const int32_t *d_group, int G, int nq, const double *q, const double *scale, int64_t *count,
+                    const int32_t *d_group, int G, int nq, const double *q, const StXf &xf, int64_t *count,
                     double *mean, double *median, double *quant) {
     int64_t launches = 0;
     const int R = 2 + 2 * nq;
@@ -1299,11 +1306,11 @@ int group_stats_run(ccb_handle *h, cudaStream_t s, const void *X, int32_t dtype,
     if (NS > 0) {
         const size_t smem = (size_t)ST_CHUNK * (D + 1) * 8;
         if (dtype == CCB_DTYPE_F32)
-            k_st_gather<float><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const float *>(X), ld, scale,
-                                                                    scale ? scale + CCB_MAX_D : nullptr, keys, psum, pnan);
+            k_st_gather<float><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const float *>(X), ld, xf, keys, psum,
+                                                                    pnan);
         else
-            k_st_gather<double><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const double *>(X), ld, scale,
-                                                                     scale ? scale + CCB_MAX_D : nullptr, keys, psum, pnan);
+            k_st_gather<double><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const double *>(X), ld, xf, keys, psum,
+                                                                     pnan);
         launches++;
     }
     // outputs
@@ -1591,61 +1598,106 @@ int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, in
     return sync_ctl(h);
 }
 
-// widen (and, with a scaler, min-max transform) n rows of dtype into double rows, on the handle's stream
+// widen (and, with a scaler, min-max transform) n rows of dtype into double rows, on the handle's stream.  cols: the device
+// column map of a column-subset ingest (output column d = source column cols[d]), or null
 static void stage_rows(ccb_handle *h, int32_t dtype, const void *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t n,
-                       const double *scale, const double *shift) {
+                       const int32_t *cols, const double *scale, const double *shift) {
     if (n <= 0) return;
     const int64_t total = n * h->D;
     const unsigned gx = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
     if (dtype == CCB_DTYPE_F32)
-        k_stage_rows<float><<<gx, 256, 0, h->stream>>>(static_cast<const float *>(src), ld_src, dst, ld_dst, n, h->D, scale, shift);
+        k_stage_rows<float><<<gx, 256, 0, h->stream>>>(static_cast<const float *>(src), ld_src, dst, ld_dst, n, h->D, cols,
+                                                       scale, shift);
     else
-        k_stage_rows<double><<<gx, 256, 0, h->stream>>>(static_cast<const double *>(src), ld_src, dst, ld_dst, n, h->D, scale, shift);
+        k_stage_rows<double><<<gx, 256, 0, h->stream>>>(static_cast<const double *>(src), ld_src, dst, ld_dst, n, h->D, cols,
+                                                        scale, shift);
     h->st.kernel_launches++;
 }
 
-static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t *assign_uid,
-                       uint8_t *stage, const double *scale, const double *shift);
+static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int W, const int32_t *cols,
+                       int32_t *assign_uid, uint8_t *stage, const double *scale, const double *shift);
+
+// ccb_ingest_ex (cols null, W == D) and ccb_ingest_cols (cols: host [D] distinct columns of W-wide rows, checked by the
+// caller) after enter().
+static int ingest_rows(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int W,
+                       const int32_t *cols, const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
+    int rc;
+    if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(h, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
+    if (!scale != !min_) return fail(h, CCB_EINVAL, "scale and min_ must both be set or both be NULL");
+    if (ld < W) return fail(h, CCB_EINVAL, "leading dimension %lld < %s = %d", (long long)ld, cols ? "W" : "D", W);
+    if (N < 0 || (!X && N > 0) || (!assign_uid && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
+    // (the copies below run behind whatever still reads the vectors and the column map on the handle's stream)
+    if (scale) {
+        CK(h, h->d_scale.ensure(4 * CCB_MAX_D * sizeof(double)));
+        CK(h, cudaMemcpyAsync(h->d_scale, scale, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(h, cudaMemcpyAsync(h->d_scale + CCB_MAX_D, min_, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
+    }
+    const double *d_sc = scale ? h->d_scale.p : nullptr, *d_sh = scale ? h->d_scale + CCB_MAX_D : nullptr;
+    const int32_t *d_cols = nullptr;
+    uint64_t colmask = 0;
+    if (cols) {
+        CK(h, h->d_cols.ensure(CCB_MAX_D * sizeof(int32_t)));
+        CK(h, cudaMemcpyAsync(h->d_cols, cols, (size_t)h->D * 4, cudaMemcpyHostToDevice, h->stream));
+        d_cols = h->d_cols;
+        double by_col[2][CCB_MAX_D] = {}; // scale_ / min_ by source column, for ccb_cluster_stats over the full rows
+        for (int d = 0; d < h->D; ++d) {
+            colmask |= 1ull << cols[d];
+            if (scale) by_col[0][cols[d]] = scale[d], by_col[1][cols[d]] = min_[d];
+        }
+        if (scale) CK(h, cudaMemcpyAsync(h->d_scale + 2 * CCB_MAX_D, by_col, sizeof by_col, cudaMemcpyHostToDevice, h->stream));
+    }
+    h->last.valid = false;
+    auto record = [&](const void *rows, int32_t rows_dtype, int64_t ldr, const int32_t *assign) {
+        h->last.X = rows, h->last.dtype = rows_dtype, h->last.ld = ldr, h->last.W = cols ? W : h->D, h->last.N = N;
+        h->last.assign = assign, h->last.colmask = colmask, h->last.scaled = scale != nullptr;
+        h->last.valid = true;
+    };
+    if (!on_device) {
+        // (ingest_host leaves the rows in d_X: unstaged float64 ones with the caller's leading dimension, staged ones
+        // -- float32 or a column subset -- with D; the full rows it staged stay in d_stg with the caller's)
+        if ((rc = ingest_host(h, X, dtype, N, ld, W, d_cols, assign_uid, stage, d_sc, d_sh))) return rc;
+        if (cols) record(h->d_stg, dtype, ld, h->d_assign);
+        else record(h->d_X, CCB_DTYPE_F64, dtype == CCB_DTYPE_F32 ? h->D : ld, h->d_assign);
+        return CCB_OK;
+    }
+    // device-resident rows: float64 without a scaler or a column map go to the engine as they are; anything else is staged
+    // into d_X (leading dimension D) by one launch -- the caller's buffer is never written
+    if (dtype == CCB_DTYPE_F64 && !scale && !cols) {
+        const double *Xd = static_cast<const double *>(X);
+        if ((rc = ingest_core_bsv(h, Xd, N, ld, assign_uid, stage))) return rc;
+        record(Xd, CCB_DTYPE_F64, ld, assign_uid);
+        return CCB_OK;
+    }
+    CK(h, h->d_X.ensure(((size_t)N * h->D + 2) * 8));
+    stage_rows(h, dtype, X, ld, h->d_X, h->D, N, d_cols, d_sc, d_sh);
+    CKL(h);
+    if ((rc = ingest_core_bsv(h, h->d_X, N, h->D, assign_uid, stage))) return rc;
+    if (cols) record(X, dtype, ld, assign_uid);
+    else record(h->d_X, CCB_DTYPE_F64, h->D, assign_uid);
+    return CCB_OK;
+}
 
 int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld,
                   const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
     int rc;
     if ((rc = enter(h))) return rc;
-    if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(h, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
-    if (!scale != !min_) return fail(h, CCB_EINVAL, "scale and min_ must both be set or both be NULL");
-    if (ld < h->D) return fail(h, CCB_EINVAL, "leading dimension %lld < D = %d", (long long)ld, h->D);
-    if (N < 0 || (!X && N > 0) || (!assign_uid && N > 0)) return fail(h, CCB_EINVAL, "bad ingest arguments");
-    if (scale) { // behind whatever still reads the vectors on the handle's stream
-        CK(h, h->d_scale.ensure(2 * CCB_MAX_D * sizeof(double)));
-        CK(h, cudaMemcpyAsync(h->d_scale, scale, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
-        CK(h, cudaMemcpyAsync(h->d_scale + CCB_MAX_D, min_, (size_t)h->D * 8, cudaMemcpyHostToDevice, h->stream));
+    return ingest_rows(h, X, dtype, on_device, N, ld, h->D, nullptr, scale, min_, assign_uid, stage);
+}
+
+int ccb_ingest_cols(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int32_t W,
+                    const int32_t *cols, const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
+    int rc;
+    if ((rc = enter(h))) return rc;
+    if (W < h->D || W > CCB_MAX_D) return fail(h, CCB_EINVAL, "row width W = %d outside [D = %d, %d]", W, h->D, CCB_MAX_D);
+    if (!cols) return fail(h, CCB_EINVAL, "null column map");
+    uint64_t seen = 0;
+    for (int d = 0; d < h->D; ++d) {
+        const int32_t c = cols[d];
+        if (c < 0 || c >= W) return fail(h, CCB_EINVAL, "cols[%d] = %d outside [0, W = %d)", d, c, W);
+        if ((seen >> c) & 1ull) return fail(h, CCB_EINVAL, "column %d appears twice in cols", c);
+        seen |= 1ull << c;
     }
-    const double *d_sc = scale ? h->d_scale.p : nullptr, *d_sh = scale ? h->d_scale + CCB_MAX_D : nullptr;
-    h->last.valid = false;
-    auto record = [&](const double *rows, int64_t ldr, const int32_t *assign) {
-        h->last.X = rows, h->last.ld = ldr, h->last.N = N, h->last.assign = assign, h->last.scaled = scale != nullptr;
-        h->last.valid = true;
-    };
-    if (!on_device) {
-        // (ingest_host leaves the rows in d_X: float64 ones with the caller's leading dimension, float32 ones with D)
-        if ((rc = ingest_host(h, X, dtype, N, ld, assign_uid, stage, d_sc, d_sh))) return rc;
-        record(h->d_X, dtype == CCB_DTYPE_F32 ? h->D : ld, h->d_assign);
-        return CCB_OK;
-    }
-    // device-resident rows: float64 without a scaler go to the engine as they are; anything else is staged into d_X
-    // (leading dimension D) by one launch -- the caller's buffer is never written
-    if (dtype == CCB_DTYPE_F64 && !scale) {
-        const double *Xd = static_cast<const double *>(X);
-        if ((rc = ingest_core_bsv(h, Xd, N, ld, assign_uid, stage))) return rc;
-        record(Xd, ld, assign_uid);
-        return CCB_OK;
-    }
-    CK(h, h->d_X.ensure(((size_t)N * h->D + 2) * 8));
-    stage_rows(h, dtype, X, ld, h->d_X, h->D, N, d_sc, d_sh);
-    CKL(h);
-    if ((rc = ingest_core_bsv(h, h->d_X, N, h->D, assign_uid, stage))) return rc;
-    record(h->d_X, h->D, assign_uid);
-    return CCB_OK;
+    return ingest_rows(h, X, dtype, on_device, N, ld, W, cols, scale, min_, assign_uid, stage);
 }
 
 int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
@@ -1664,28 +1716,29 @@ int ccb_ingest_scaled(ccb_handle *h, const double *X_raw, int64_t N, int64_t ld,
 }
 
 // host rows in, per-cell results out.  float64 rows are copied into d_X as they are (leading dimension ld) and, with a
-// scaler (scale / shift: device vectors), min-max transformed there in place; float32 rows are copied into the float32
-// staging buffer and widened (and transformed) from there into d_X with leading dimension D.  Either happens segment by
-// segment behind the segments' copies.  Arguments are checked by ccb_ingest_ex.
-static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t *assign_uid,
-                       uint8_t *stage, const double *scale, const double *shift) {
+// scaler (scale / shift: device vectors), min-max transformed there in place; float32 rows, and the W-wide rows of a
+// column-subset ingest (cols: device column map), are copied into the staging buffer and gathered / widened (and
+// transformed) from there into d_X with leading dimension D.  Either happens segment by segment behind the segments'
+// copies.  Arguments are checked by ingest_rows.
+static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int W, const int32_t *cols,
+                       int32_t *assign_uid, uint8_t *stage, const double *scale, const double *shift) {
     int rc;
     if (N == 0) return CCB_OK;
-    const bool f32 = dtype == CCB_DTYPE_F32;
+    const bool f32 = dtype == CCB_DTYPE_F32, staged = f32 || cols;
     const size_t esz = f32 ? 4 : 8;
-    const int64_t ldX = f32 ? h->D : ld; // leading dimension of the rows in d_X
-    // the rows [r0, r0 + n) of the caller occupy (n - 1) * ld + D elements: the last row's padding is not read
-    auto span = [&](int64_t n) { return (size_t)((n - 1) * ld + h->D) * esz; };
+    const int64_t ldX = staged ? h->D : ld; // leading dimension of the rows in d_X
+    // the rows [r0, r0 + n) of the caller occupy (n - 1) * ld + W elements: the last row's padding is not read
+    auto span = [&](int64_t n) { return (size_t)((n - 1) * ld + W) * esz; };
     CK(h, h->d_X.ensure(((size_t)N * ldX + 2) * 8));
-    if (f32) CK(h, h->d_X32.ensure(span(N)));
+    if (staged) CK(h, h->d_stg.ensure(span(N)));
     CK(h, h->d_assign.ensure((size_t)N * 4));
     CK(h, h->d_stage.ensure((size_t)N));
     const char *src = static_cast<const char *>(X);
-    char *dst = f32 ? reinterpret_cast<char *>(h->d_X32.p) : reinterpret_cast<char *>(h->d_X.p); // where the copies land
+    char *dst = staged ? reinterpret_cast<char *>(h->d_stg.p) : reinterpret_cast<char *>(h->d_X.p); // where the copies land
     // the copied rows [r0, r0 + n) -> double rows in d_X, on the handle's stream behind the wait for their copy
     auto stage_seg = [&](int64_t r0, int64_t n) -> int {
-        if (f32 || scale) {
-            stage_rows(h, dtype, dst + r0 * ld * esz, ld, h->d_X + r0 * ldX, ldX, n, scale, shift);
+        if (staged || scale) {
+            stage_rows(h, dtype, dst + r0 * ld * esz, ld, h->d_X + r0 * ldX, ldX, n, cols, scale, shift);
             CKL(h);
         }
         return CCB_OK;
@@ -2308,7 +2361,7 @@ int ccb_group_stats(int32_t device, void *stream, const void *X, int32_t dtype, 
     if (int rc = stats_args(nullptr, N, ld, D, G, nq, q, count, mean, median, quant)) return rc;
     if (N > 0 && (!X || !group)) return fail(nullptr, CCB_EINVAL, "null rows or groups");
     if (int rc = enter_device(device)) return rc;
-    return group_stats_run(nullptr, (cudaStream_t)stream, X, dtype, N, ld, D, group, G, nq, q, nullptr, count, mean, median,
+    return group_stats_run(nullptr, (cudaStream_t)stream, X, dtype, N, ld, D, group, G, nq, q, StXf{}, count, mean, median,
                            quant);
 }
 
@@ -2319,7 +2372,7 @@ int ccb_cluster_stats(ccb_handle *h, const int32_t *group_of_pcore, int64_t n_pc
     if (!h->last.valid)
         return fail(h, CCB_ESTATE, "no ingest since the last ccb_begin_timepoint / ccb_reset / ccb_import_list");
     if (G < 0 || G == INT32_MAX) return fail(h, CCB_EINVAL, "G = %d", G);
-    if ((rc = stats_args(h, h->last.N, h->last.ld, h->D, G + 1, nq, q, count, mean, median, quant))) return rc;
+    if ((rc = stats_args(h, h->last.N, h->last.ld, h->last.W, G + 1, nq, q, count, mean, median, quant))) return rc;
     if ((rc = sync_ctl(h))) return rc;
     const int np = h->h_ctl->n_pcore;
     if (n_pcore != np) return fail(h, CCB_EINVAL, "n_pcore = %lld, the pcore list holds %d", (long long)n_pcore, np);
@@ -2341,8 +2394,14 @@ int ccb_cluster_stats(ccb_handle *h, const int32_t *group_of_pcore, int64_t n_pc
     k_st_cell_group<<<gx, 256, 0, s>>>(h->last.assign, N, lut, nlut, G, group);
     h->st.kernel_launches += 2;
     CKL(h);
-    return group_stats_run(h, s, h->last.X, CCB_DTYPE_F64, N, h->last.ld, h->D, group, G + 1, nq, q,
-                           h->last.scaled ? h->d_scale.p : nullptr, count, mean, median, quant);
+    StXf xf{};
+    if (h->last.scaled && h->last.colmask) { // raw full rows: the clustering columns are transformed forth and back
+        xf.scale = h->d_scale + 2 * CCB_MAX_D, xf.shift = h->d_scale + 3 * CCB_MAX_D, xf.mask = h->last.colmask, xf.fwd = 1;
+    } else if (h->last.scaled) { // the scaled rows the engine read: transformed back
+        xf.scale = h->d_scale, xf.shift = h->d_scale + CCB_MAX_D, xf.mask = ~0ull >> (64 - h->D);
+    }
+    return group_stats_run(h, s, h->last.X, h->last.dtype, N, h->last.ld, h->last.W, group, G + 1, nq, q, xf, count, mean,
+                           median, quant);
 }
 
 } // extern "C"

@@ -9,7 +9,8 @@
 // Kernel 3   k_maint_plan + k_maint_gather: fused decay x 2^(-lambda dt) (hddstream.py:247-286), downgrade with the
 //            reference's skip-next-after-removal iteration and outlier deletion (hddstream.py:512-549), order-preserving
 //            compaction.
-// Input      k_stage_rows / k_colminmax: float32 / float64 rows widened to double and min-max transformed, and the fit
+// Input      k_stage_rows / k_colminmax: float32 / float64 rows (optionally a subset of their columns) widened to double
+//            and min-max transformed, and the fit
 //            reductions (scaling/scaler.py:11-53).
 #pragma once
 #include "common.cuh"
@@ -290,16 +291,29 @@ __global__ void k_repack_store(Store S, int n, int D, int DP, double wsel) {
 // (sklearn: `X *= self.scale_; X += self.min_`), so results equal those of widening and scaling on the host.  src == dst
 // (T = double, ld_src == ld_dst) scales the device copy of a timepoint in place: every element is read and written by
 // the same thread, hence no __restrict__ on src / dst.  HBM-bound: 8 + 8 B (double) or 4 + 8 B (float) per element.
+// cols (device [D], or null = the identity): output column d is source column cols[d].  The map sits in shared memory; a
+// warp's 32 consecutive outputs still read from one or two source rows, so the reads of a row stay coalesced.
 template <typename T>
 __global__ void k_stage_rows(const T *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t N, int D,
-                             const double *__restrict__ scale, const double *__restrict__ shift) {
-    const int64_t total = N * D;
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t r = e / D;
-        const int d = (int)(e - r * D);
-        double x = (double)src[r * ld_src + d];
-        if (scale) x = dadd(dmul(x, scale[d]), shift[d]);
-        dst[r * ld_dst + d] = x;
+                             const int32_t *__restrict__ cols, const double *__restrict__ scale,
+                             const double *__restrict__ shift) {
+    __shared__ int32_t s_col[CCB_MAX_D];
+    auto rows = [&](auto col_of) { // (one loop body, instantiated for the identity and for the map)
+        const int64_t total = N * D;
+        for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t r = e / D;
+            const int d = (int)(e - r * D);
+            double x = (double)src[r * ld_src + col_of(d)];
+            if (scale) x = dadd(dmul(x, scale[d]), shift[d]);
+            dst[r * ld_dst + d] = x;
+        }
+    };
+    if (cols) {
+        for (int d = threadIdx.x; d < D; d += blockDim.x) s_col[d] = cols[d];
+        __syncthreads();
+        rows([&](int d) { return s_col[d]; });
+    } else {
+        rows([](int d) { return d; });
     }
 }
 

@@ -6,7 +6,7 @@
 //                            slice) and their slices -- four exclusive scans in one launch
 //   3. k_st_sort_hist/scatter stable LSD counting sort of the rows by group (8-bit digits): a deterministic permutation, so
 //                            every later sum runs in the same order on every call
-//   4. k_st_gather           the rows in group order, widened to double (and inverse-scaled) -> column-major order-preserving
+//   4. k_st_gather           the rows in group order, widened to double (and scaled per column) -> column-major order-preserving
 //                            uint64 keys; per (slice, marker) partial sums and NaN counts, each summed in row order
 //   5. k_st_small            groups of <= ST_SLICE cells: one CTA each, bitonic sort of each marker in shared memory
 //      k_st_rsel_*           larger groups: radix select (8 passes x 8 bits) of every needed rank, the histograms of every
@@ -253,12 +253,21 @@ __device__ __forceinline__ void st_slice_range(const StGeom &g, int s, int &grp,
     len = min(ST_SLICE, (int)g.cnt[grp] - j * ST_SLICE);
 }
 
+// Per-column transform of the values k_st_gather summarises.  A column m with bit m of `mask` set holds min-max scaled
+// values, brought back by (x - shift[m]) / scale[m] (sklearn's inverse_transform); with `fwd` the rows hold the raw values
+// and the forward transform x * scale[m] + shift[m] comes first (what the engine read after a column-subset ingest).
+// Every other column is summarised as it is, widened to double.
+struct StXf {
+    const double *scale, *shift; // [CCB_MAX_D], indexed by column
+    uint64_t mask;
+    int fwd;
+};
+
 // One CTA per slice: rows staged ST_CHUNK at a time in shared memory (coalesced row reads, coalesced column writes).
 // Thread m < D sums column m over the chunk in row order and adds the chunk to the slice's sum: a fixed order.
-// scale != nullptr: the rows are min-max scaled; what is summarised is (x - min_) / scale_ (sklearn's inverse_transform).
 template <typename T>
-__global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, int64_t ld, const double *scale,
-                                                          const double *shift, uint64_t *keys, double *psum, int32_t *pnan) {
+__global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, int64_t ld, StXf xf, uint64_t *keys,
+                                                          double *psum, int32_t *pnan) {
     extern __shared__ double st_tile[]; // [ST_CHUNK][D + 1]
     const int D = g.D, P = D + 1, t = threadIdx.x;
     int grp, len;
@@ -271,7 +280,10 @@ __global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, 
         for (int e = t; e < rows * D; e += ST_THREADS) {
             const int r = e / D, m = e - r * D;
             double v = (double)X[(int64_t)g.perm[start + c0 + r] * ld + m];
-            if (scale) v = ddiv(dsub(v, shift[m]), scale[m]);
+            if ((xf.mask >> m) & 1ull) {
+                if (xf.fwd) v = dadd(dmul(v, xf.scale[m]), xf.shift[m]);
+                v = ddiv(dsub(v, xf.shift[m]), xf.scale[m]);
+            }
             st_tile[r * P + m] = v;
         }
         __syncthreads();

@@ -48,30 +48,56 @@ def _input_rows(x, device):
     return x.ctypes.data, _lib.DTYPE_F64, False, (x.shape[1] if x.ndim == 2 else 0), x
 
 
+def column_map(columns, width):
+    """`columns` as int32 indices into rows `width` wide (HDDStream.online_microcluster_maintenance(columns=)).  ValueError
+    for rows wider than 64 columns, an empty list, more than 64 entries, or an entry that is not an integer, lies outside
+    [0, width) or repeats an earlier one."""
+    if width > 64:
+        raise ValueError(f"rows of {width} columns: at most 64 are supported")
+    try:
+        entries = list(columns)
+    except TypeError:
+        raise ValueError("columns must be a sequence of column indices") from None
+    if not 1 <= len(entries) <= 64:
+        raise ValueError(f"columns holds {len(entries)} entries; 1 to 64 are supported")
+    out = []
+    for c in entries:
+        if isinstance(c, (bool, np.bool_)) or not isinstance(c, (int, np.integer)):
+            raise ValueError(f"column {c!r} is not an integer")
+        if not 0 <= int(c) < width:
+            raise ValueError(f"column {int(c)} outside [0, {width})")
+        if int(c) in out:
+            raise ValueError(f"column {int(c)} appears twice")
+        out.append(int(c))
+    return np.array(out, np.int32)
+
+
 class _PointsView(object):
     """Per-timepoint cell -> MC assignment; builds Microcluster.points dicts on demand.  The input arrays or tensors are
     BORROWED, not copied (the reference copies every row into a Python list, microcluster.py:149): a caller that
     overwrites its array or tensor in place after the call changes what `points` hands out.  float32 rows are handed out
     widened to float64, and the rows of a CUDA tensor are gathered on its device and brought back as float64 -- the same
-    values the float64 path hands out."""
+    values the float64 path hands out.  Rows ingested with a column map hand out their clustering columns only, in map
+    order."""
 
     def __init__(self):
-        self.segments = []  # [(X, assign_uid)] since the last reset (hddstream.py:208-213)
+        self.segments = []  # [(X, assign_uid, scaler, column map)] since the last reset (hddstream.py:208-213)
         self._index = None
 
     def reset(self):
         self.segments = []
         self._index = None
 
-    def add(self, X, assign, scaler=None):
+    def add(self, X, assign, scaler=None, cols=None):
         """scaler = (scale_, min_): X holds RAW rows that were scaled on the device; the coordinates handed out are
-        X * scale_ + min_ of the requested rows (numpy's elementwise arithmetic = the device's two roundings)."""
-        self.segments.append((X, assign, scaler))
+        X * scale_ + min_ of the requested rows (numpy's elementwise arithmetic = the device's two roundings).
+        cols: int32 column map into the rows of X (the coordinates are X[:, cols]), or None."""
+        self.segments.append((X, assign, scaler, cols))
         self._index = None
 
     def _build(self):
         idx = {}
-        for si, (_, assign, _sc) in enumerate(self.segments):
+        for si, (_, assign, _sc, _cols) in enumerate(self.segments):
             order = np.argsort(assign, kind="stable")
             sa = assign[order]
             cuts = np.flatnonzero(np.diff(sa)) + 1
@@ -91,13 +117,17 @@ class _PointsView(object):
     def points_of(self, uid):
         out = {}
         for si, rows in self.rows_of(uid):
-            X, _, sc = self.segments[si]
+            X, _, sc, cols = self.segments[si]
             if isinstance(X, np.ndarray):
-                sel = X[rows].astype(np.float64, copy=False)  # (widened before the scaler arithmetic)
+                sel = X[rows] if cols is None else X[np.ix_(rows, cols)]
+                sel = sel.astype(np.float64, copy=False)  # (widened before the scaler arithmetic)
             else:  # a CUDA tensor
                 import torch
 
-                sel = X[torch.from_numpy(rows).to(X.device)].to(torch.float64).cpu().numpy()
+                sel = X[torch.from_numpy(rows).to(X.device)]
+                if cols is not None:
+                    sel = sel[:, torch.from_numpy(cols.astype(np.int64)).to(X.device)]
+                sel = sel.to(torch.float64).cpu().numpy()
             if sc is not None:
                 sel = sel * sc[0]
                 sel = sel + sc[1]
@@ -138,12 +168,14 @@ class HDDStream(object):
         self._device, self._chunk = device, chunk
         self._bsv = (bsv_bmin, bsv_iters, bsv_stream, off_csr_min_m)
         self._h = None
+        self._handle_dim = 0  # D of the handle
         self._views = _PointsView()
         self._lists = [None, None]  # cached Microcluster lists (pcore, outlier)
         self.last_assignment = None  # uid of the MC every row of the last call went to
         self.last_stage = None
         self.last_cluster_label = None  # cluster index of every pcore MC (list order) after the offline phase
         self._last_device_input = None  # (rows, assignments) of the last CUDA-tensor ingest, read by cluster_statistics
+        self._stats_width = None  # columns of the rows of the last ingest, when they are not dataset_dimensionality
 
     # ------------------------------------------------------------------------------------------
     def __del__(self):
@@ -173,10 +205,11 @@ class HDDStream(object):
         self._chunk = 0
         self._bsv = (0, 0, 0, 0)
         self._h = None
+        self._handle_dim = 0
         self._views = _PointsView()
         self._lists = [None, None]
         self.last_assignment = self.last_stage = self.last_cluster_label = None
-        self._last_device_input = None
+        self._last_device_input = self._stats_width = None
         if self.dataset_dimensionality:
             self._ensure_handle(self.dataset_dimensionality)
             self._import(0, pcore)
@@ -202,9 +235,10 @@ class HDDStream(object):
     def calculate_density_threshold(self):
         return float(self.config['mu']) * self.dataset_size
 
-    def _set_dataset_dependent_parameters(self, input_dataset):
+    def _set_dataset_dependent_parameters(self, input_dataset, dataset_dim=None):
         # hddstream.py:89-128: omicron from the PREVIOUS dataset size, then mu from the current one
-        dataset_dim = input_dataset.shape[1]
+        if dataset_dim is None:
+            dataset_dim = input_dataset.shape[1]
         self.dataset_dimensionality = dataset_dim
         config_pi = float(self.config['pi'])
         self.pi = dataset_dim if config_pi <= 0 else round(config_pi)
@@ -224,7 +258,7 @@ class HDDStream(object):
         rc = L.ccb_create(C.byref(prm), C.byref(h))
         if rc != 0:
             _lib.check(rc, None)
-        self._h = h
+        self._h, self._handle_dim = h, D
         try:
             _lib.check(L.ccb_set_dnrm2(h, _lib.scipy_dnrm2_pointer()), h)
         except ImportError:
@@ -232,7 +266,7 @@ class HDDStream(object):
 
     # ------------------------------------------------------------------------------------------
     def online_microcluster_maintenance(self, input_dataset, input_dataset_daystamp, reset_param=True,
-                                        run_offline=True, scaler=None):
+                                        run_offline=True, scaler=None, columns=None):
         """input_dataset: [N, D] cells -- a numpy array, a CPU tensor or a CUDA tensor on this instance's device.  float32 and
         float64 rows with unit column stride go in without a copy (row-strided views included); float32 rows are widened
         to float64 on the device, which is exact, so results are those of the float64 path on the widened rows.  Other
@@ -241,20 +275,30 @@ class HDDStream(object):
 
         scaler (extension, SURVEY 8f-3): a fitted sklearn MinMaxScaler (or a (scale_, min_) pair) -- input_dataset then
         holds RAW rows and the min-max transform x * scale_ + min_ runs on the device behind the host -> device copy
-        (ccb_ingest_ex) instead of as a host pass; results are those of scaling on the host first, bit for bit."""
+        (ccb_ingest_ex) instead of as a host pass; results are those of scaling on the host first, bit for bit.
+
+        columns (extension): a sequence of D distinct column indices into input_dataset's W <= 64 columns -- the engine then
+        clusters input_dataset[:, columns] (dataset_dimensionality = D) and gives bit for bit what the float64 path gives on
+        those gathered rows; the gather runs on the device, the rows go in without a copy as above, and the scaler's vectors
+        have D entries.  `points` hands out the gathered coordinates, and cluster_statistics reports all W columns.
+        ValueError before any device work for a bad entry (see column_map) or a D that differs from the handle's."""
         xp, dtype, on_device, ld, X = _input_rows(input_dataset, self._device)
         if X.ndim != 2:
             raise ValueError("input_dataset must be 2-D")
-        if reset_param:
-            self._set_dataset_dependent_parameters(X)
-        self._ensure_handle(X.shape[1])
+        cols = None if columns is None else column_map(columns, X.shape[1])
+        D = X.shape[1] if cols is None else len(cols)
+        if cols is not None and self._h is not None and D != self._handle_dim:
+            raise ValueError(f"{D} columns given; this HDDStream clusters {self._handle_dim} markers")
         sc = mn = None
         if scaler is not None:
             sc, mn = (scaler.scale_, scaler.min_) if hasattr(scaler, "scale_") else scaler
             sc = np.ascontiguousarray(sc, np.float64)
             mn = np.ascontiguousarray(mn, np.float64)
-            if sc.shape != (X.shape[1],) or mn.shape != (X.shape[1],):
+            if sc.shape != (D,) or mn.shape != (D,):
                 raise ValueError("scaler vectors must have one entry per marker")
+        if reset_param:
+            self._set_dataset_dependent_parameters(X, D)
+        self._ensure_handle(D)
         L, h, logger = _lib.lib(), self._h, self.logger
         logger.info(f"Setting up online phase for timepoint {input_dataset_daystamp} with following params:\n"
                     f"Pcore density threshold factor(beta) = {self.beta}\n"
@@ -279,15 +323,21 @@ class HDDStream(object):
                                          float(factor)), h)
         N = X.shape[0]
         logger.info("Starting online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
-        self._last_device_input = None
+        self._last_device_input = self._stats_width = None
         if on_device:
-            assign, stage = self._ingest_tensor(X, xp, dtype, ld, sc, mn)
+            assign, stage = self._ingest_tensor(X, xp, dtype, ld, sc, mn, cols)
         else:
             assign = np.empty(N, np.int32)
             stage = np.empty(N, np.uint8)
-            _lib.check(L.ccb_ingest_ex(h, xp, dtype, 0, N, ld, _lib.ptr(sc), _lib.ptr(mn), _lib.ptr(assign),
-                                       _lib.ptr(stage)), h)
-        self._views.add(X, assign, None if sc is None else (sc, mn))
+            if cols is None:
+                _lib.check(L.ccb_ingest_ex(h, xp, dtype, 0, N, ld, _lib.ptr(sc), _lib.ptr(mn), _lib.ptr(assign),
+                                           _lib.ptr(stage)), h)
+            else:
+                _lib.check(L.ccb_ingest_cols(h, xp, dtype, 0, N, ld, X.shape[1], _lib.ptr(cols), _lib.ptr(sc), _lib.ptr(mn),
+                                             _lib.ptr(assign), _lib.ptr(stage)), h)
+        if cols is not None:
+            self._stats_width = X.shape[1]
+        self._views.add(X, assign, None if sc is None else (sc, mn), cols)
         self.last_assignment, self.last_stage = assign, stage
         self._lists = [None, None]
         logger.info("Finish online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
@@ -297,9 +347,10 @@ class HDDStream(object):
         if run_offline:
             self.offline_clustering(input_dataset_daystamp)
 
-    def _ingest_tensor(self, X, xp, dtype, ld, sc, mn):
-        """ccb_ingest_ex on the rows of a CUDA tensor X: the handle's stream first waits for the work queued on the
-        current torch stream (whatever produced X), and the per-cell results come back to the host behind the engine."""
+    def _ingest_tensor(self, X, xp, dtype, ld, sc, mn, cols=None):
+        """ccb_ingest_ex (ccb_ingest_cols with a column map) on the rows of a CUDA tensor X: the handle's stream first waits
+        for the work queued on the current torch stream (whatever produced X), and the per-cell results come back to the
+        host behind the engine."""
         import torch
 
         N = X.shape[0]
@@ -308,8 +359,12 @@ class HDDStream(object):
         assign_d = torch.empty(N, dtype=torch.int32, device=X.device)
         stage_d = torch.empty(N, dtype=torch.uint8, device=X.device)
         mine.wait_stream(cur)  # (after the allocations: earlier users of that memory on `cur` are done first)
-        _lib.check(_lib.lib().ccb_ingest_ex(self._h, xp, dtype, 1, N, ld, _lib.ptr(sc), _lib.ptr(mn), assign_d.data_ptr(),
-                                            stage_d.data_ptr()), self._h)
+        if cols is None:
+            _lib.check(_lib.lib().ccb_ingest_ex(self._h, xp, dtype, 1, N, ld, _lib.ptr(sc), _lib.ptr(mn),
+                                                assign_d.data_ptr(), stage_d.data_ptr()), self._h)
+        else:
+            _lib.check(_lib.lib().ccb_ingest_cols(self._h, xp, dtype, 1, N, ld, X.shape[1], _lib.ptr(cols), _lib.ptr(sc),
+                                                  _lib.ptr(mn), assign_d.data_ptr(), stage_d.data_ptr()), self._h)
         # the copies, and the release of the temporaries, are ordered on `cur` behind everything the handle queued
         cur.wait_stream(mine)
         self._last_device_input = (X, assign_d)  # the handle reads both again in cluster_statistics
@@ -357,7 +412,7 @@ class HDDStream(object):
         self.last_data_timestamp = 0
         self.dataset_size = 0
         self.last_assignment = self.last_stage = self.last_cluster_label = None
-        self._last_device_input = None
+        self._last_device_input = self._stats_width = None
 
     @property
     def stream_ptr(self):
@@ -374,6 +429,7 @@ class HDDStream(object):
         _lib.check(L.ccb_begin_timepoint(h, float(self.mu), float(self.omicron), int(self.pi), int(decay),
                                          float(factor)), h)
         _lib.check(L.ccb_ingest_device(h, x_ptr, N, ld, assign_ptr, stage_ptr), h)
+        self._stats_width = None
         self._lists = [None, None]
         self.last_data_timestamp = daystamp
         if run_offline:
@@ -476,6 +532,9 @@ class HDDStream(object):
         final_clusters[c] -- and a last row for the cells in no cluster.  The values are the cells as the engine read
         them, widened to float64 and, with a scaler, brought back to the input scale ((x - min_) / scale_, as
         cluster_points_D{t}.csv holds them); median and quantiles are numpy's bit for bit (see group_statistics).
+        After an ingest with `columns`, the statistics cover every one of the W columns of input_dataset (arrays [.., W]):
+        a clustering column as just described (under a scaler: inverse_transform(transform(x))), every other column as
+        the raw value widened to float64.
 
         groups: optional integer array over the pcore list (pcore_MC order, -1 = no group) replacing the clusters of the
         offline phase; the result then has max(groups) + 2 rows.  ValueError without an offline result or `groups`;
@@ -493,4 +552,4 @@ class HDDStream(object):
             G = int(groups.max()) + 1 if len(groups) else 0
         if self._h is None:
             raise _lib.CCBError("no cells have been ingested")
-        return cellstats.cluster_statistics(self._h, self.dataset_dimensionality, groups, G, quantiles)
+        return cellstats.cluster_statistics(self._h, self._stats_width or self.dataset_dimensionality, groups, G, quantiles)

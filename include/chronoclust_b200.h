@@ -13,8 +13,8 @@
  *   ccb_create              HDDStream.__init__                      clustering/hddstream.py:30-67
  *   ccb_begin_timepoint     decay + downgrade + reset               clustering/hddstream.py:199-213,
  *                                                                    247-286, 512-549
- *   ccb_ingest[_device|_ex] the ordered per-point loop              clustering/hddstream.py:220-237,
- *                           (_add_to_pcore, _add_to_outlier,          288-343, 345-395, 397-430, 434-462
+ *   ccb_ingest[_device|_ex| the ordered per-point loop              clustering/hddstream.py:220-237,
+ *              _cols]       (_add_to_pcore, _add_to_outlier,          288-343, 345-395, 397-430, 434-462
  *                            _upgrade_outlier_microcluster,          objects/microcluster.py:89-153,
  *                            _create_new_outlier_cluster)             167-197, 213-233
  *                                                                    utilities/mc_functions.py:14-62
@@ -169,6 +169,17 @@ int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld,
  * An unknown dtype, only one of scale / min_, or ld < D: CCB_EINVAL. */
 int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld,
                   const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage);
+/* ccb_ingest_ex on a subset of the columns of wider rows (extension): X holds rows of W >= D columns (leading dimension
+ * ld >= W) and the engine clusters the columns cols [D] (host, distinct, each in [0, W)) in that order.  Results are those
+ * of ccb_ingest_ex on the gathered rows X[:, cols], bit for bit; scale / min_ have D entries and belong to the clustering
+ * columns.  X is never written.  Host rows travel W wide through the segmented copy into a handle-owned staging buffer
+ * and are gathered, widened and scaled behind each segment's copy; device rows take one staging launch.
+ * Afterwards ccb_cluster_stats reports all W columns: a clustering column is reported as the engine read it brought back
+ * to the input scale (under a scaler: MinMaxScaler.inverse_transform(transform(x))), every other column as the raw value
+ * widened to double.  CCB_EINVAL: W outside [D, 64], ld < W, a null cols, an entry of cols outside [0, W), a repeated
+ * entry, or anything ccb_ingest_ex rejects. */
+int ccb_ingest_cols(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int32_t W,
+                    const int32_t *cols, const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage);
 
 /* Offline phase over the current pcore list; returns the number of clusters. */
 int ccb_offline(ccb_handle *h, int64_t *n_clusters);
@@ -201,6 +212,8 @@ int ccb_export_offline(ccb_handle *h, uint8_t *core, uint8_t *nbr, uint8_t *wnbr
  * The rows and assignments are read where the ingest left them: the handle's own buffers, or, for device input
  * (ccb_ingest_ex with on_device, ccb_ingest_device), the CALLER's device rows and assignment buffer, which must still hold
  * what they held at the ingest.  Reads only: nothing later computed by the handle changes.
+ * After ccb_ingest_cols the outputs cover all W columns of the rows ([G + 1][W], quantiles [nq][G + 1][W]); otherwise
+ * they have D columns.
  * CCB_ESTATE unless an ingest happened since the last ccb_begin_timepoint / ccb_reset / ccb_import_list; CCB_EINVAL if
  * n_pcore != the pcore count, G < 0, a group_of_pcore entry >= G, or a q outside [0, 1].  Synchronises the handle's stream. */
 int ccb_cluster_stats(ccb_handle *h, const int32_t *group_of_pcore, int64_t n_pcore, int32_t G, int32_t nq, const double *q,
