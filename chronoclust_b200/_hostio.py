@@ -1,4 +1,5 @@
-"""ctypes binding of chronoclust_b200/csrc/hostio.c (host-side writer of the per-cell output table, SURVEY 8f-2)."""
+"""ctypes binding of chronoclust_b200/csrc/hostio.c (host-side writer of the per-cell output table, SURVEY 8f-2, and the
+host side of the arcsinh transform)."""
 import ctypes as C
 import os
 
@@ -20,6 +21,9 @@ def lib():
         L.ccbio_write_points_csv.restype = C.c_int
         L.ccbio_write_points_csv.argtypes = [C.c_char_p, C.c_char_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_int64,
                                              C.c_void_p, C.c_char_p, C.c_void_p, C.c_int32]
+        L.ccbio_arcsinh_host.restype = C.c_int
+        L.ccbio_arcsinh_host.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p,
+                                         C.c_int32]
         L.ccbio_repr.restype = C.c_int
         L.ccbio_repr.argtypes = [C.c_double, C.c_char_p]
         _LIB = L
@@ -57,3 +61,29 @@ def write_points_csv(path, header_names, values, label_idx, labels, id0=0, threa
                                       id0, label_idx.ctypes.data, pool, off.ctypes.data, threads)
     if rc != 0:
         raise OSError(rc, os.strerror(rc), str(path))
+
+
+def arcsinh_host(x, cofactor, threads=0):
+    """ccbio_arcsinh_host: [n, d] float64 rows of the float32 / float64 rows `x` (numpy, unit column stride, any row stride),
+    every column with cofactor[c] != 0 as ccb_asinh(x / cofactor[c]) -- the device's values bit for bit.  `cofactor`:
+    float64 [d], already checked (scaling.cofactor_vector)."""
+    x = np.asarray(x)
+    if x.dtype not in (np.float32, np.float64):
+        x = x.astype(np.float64)
+    if x.ndim != 2:
+        raise ValueError("arcsinh takes 2-D rows")
+    isz = x.itemsize
+    if (x.shape[1] > 1 and x.strides[1] != isz) or (x.shape[0] > 1 and (x.strides[0] % isz or
+                                                                         x.strides[0] < x.shape[1] * isz)):
+        x = np.ascontiguousarray(x)
+    n, d = x.shape
+    ld = x.strides[0] // isz if n > 1 else d
+    cof = np.ascontiguousarray(cofactor, np.float64)
+    if cof.shape != (d,):
+        raise ValueError(f"{cof.size} cofactors for {d} columns")
+    out = np.empty((n, d), np.float64)
+    rc = lib().ccbio_arcsinh_host(x.ctypes.data, 1 if x.dtype == np.float32 else 0, n, ld, d, cof.ctypes.data,
+                                  out.ctypes.data, threads)
+    if rc != 0:
+        raise OSError(rc, os.strerror(rc))
+    return out

@@ -50,6 +50,7 @@ SYMBOLS = {
     "ccb_ingest_device": (C.c_int, [vp, vp, i64, i64, vp, vp]),
     "ccb_ingest_ex": (C.c_int, [vp, vp, i32, i32, i64, i64, vp, vp, vp, vp]),
     "ccb_ingest_cols": (C.c_int, [vp, vp, i32, i32, i64, i64, i32, vp, vp, vp, vp, vp]),
+    "ccb_ingest_tx": (C.c_int, [vp, vp, i32, i32, i64, i64, i32, vp, vp, vp, vp, vp, vp]),
     "ccb_offline": (C.c_int, [vp, C.POINTER(i64)]),
     "ccb_counts": (C.c_int, [vp, C.POINTER(i64 * 4)]),
     "ccb_export_list": (C.c_int, [vp, i32] + [vp] * 7),
@@ -63,6 +64,7 @@ SYMBOLS = {
     "ccb_assoc_nearest2": (C.c_int, [i32, vp, vp, vp, i64, vp, i64, i32, f64, vp, vp, vp]),
     "ccb_colminmax": (C.c_int, [i32, vp, vp, i64, i64, i32, vp, vp]),
     "ccb_colminmax_ex": (C.c_int, [i32, vp, vp, i32, i64, i64, i32, vp, vp]),
+    "ccb_arcsinh": (C.c_int, [i32, vp, vp, i32, i64, i64, i32, vp, vp]),
     "ccb_ingest_scaled": (C.c_int, [vp, vp, i64, i64, vp, vp, vp, vp]),
     "ccb_off_neighbours": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, f64, f64, vp, vp, vp, C.POINTER(i64)]),
     "ccb_off_subspace": (C.c_int, [i32, vp, vp, i64, i32, i64, i64, vp, vp, f64, vp]),

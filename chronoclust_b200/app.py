@@ -31,7 +31,7 @@ import pandas as pd
 from . import _hostio, cellstats
 from .hddstream import HDDStream
 from .objects import Cluster
-from .scaling import Scaler
+from .scaling import Scaler, cofactor_vector
 from .tracking import TrackByHistoricalAssociation, TrackByLineage
 
 STATE_FILES = ("hddstream", "tracking_by_historical_association", "tracking_by_lineage")
@@ -70,13 +70,17 @@ class _Timepoints(object):
         self._pool.shutdown(wait=False)
 
 
-def _fit_joint_scaler(timepoints, wanted, cols=None):
+def _fit_joint_scaler(timepoints, wanted, cols=None, cofactors=None):
     """MinMaxScaler over all timepoints jointly (scaler.py:27-36), fed one parsed array at a time -- on the clustering
-    columns `cols` only when given (the fit is column-wise: the vectors are those of a fit on files holding only them)."""
+    columns `cols` only when given (the fit is column-wise: the vectors are those of a fit on files holding only them),
+    and on their arcsinh-transformed values with `cofactors` (by file column; what the engine then scales)."""
     scaler = Scaler()
     for t in wanted:
         cells = timepoints.cells(t)
-        scaler.scaler.partial_fit(cells if cols is None else cells[:, cols])
+        cells = cells if cols is None else cells[:, cols]
+        if cofactors is not None:
+            cells = _hostio.arcsinh_host(np.asarray(cells, np.float64), cofactors if cols is None else cofactors[cols])
+        scaler.scaler.partial_fit(cells)
     return scaler
 
 
@@ -96,6 +100,31 @@ def clustering_columns(attributes, clustering_markers):
     return [attributes.index(m) for m in names]
 
 
+def arcsinh_cofactors_by_column(attributes, cols, arcsinh_cofactors):
+    """app.run(arcsinh_cofactors=) as one float64 cofactor per column of the files (0: linear), or None.  A number applies
+    to every clustering marker (the columns `cols`, or every column); a dict {marker name: cofactor} to the columns it
+    names, clustering or not.  ValueError for an unknown name or a cofactor that is not 0 or positive and finite."""
+    if arcsinh_cofactors is None:
+        return None
+    W = len(attributes)
+    if isinstance(arcsinh_cofactors, dict):
+        unknown = [m for m in arcsinh_cofactors if str(m) not in attributes]
+        if unknown:
+            raise ValueError(f"arcsinh_cofactors names markers not in the header of the first file: {unknown}")
+        named = {attributes.index(str(m)): c for m, c in arcsinh_cofactors.items()}
+        try:
+            return cofactor_vector([named.get(c, 0.0) for c in range(W)], W)
+        except ValueError as exc:
+            raise ValueError(f"arcsinh_cofactors: {exc}") from None
+    try:
+        value = cofactor_vector(arcsinh_cofactors, 1)[0]
+    except ValueError as exc:
+        raise ValueError(f"arcsinh_cofactors must be a number or a dict of marker names to numbers: {exc}") from None
+    out = np.zeros(W, np.float64)
+    out[slice(None) if cols is None else cols] = value
+    return out
+
+
 # ---- outputs --------------------------------------------------------------------------------------------------------------
 class _PointsWriter(object):
     """cluster_points_D{t}.csv on a background thread; at most one file in flight so that memory stays bounded."""
@@ -104,9 +133,9 @@ class _PointsWriter(object):
         self._thread = None
         self._error = None
 
-    def _job(self, path, header, raw, scaler, cols, label_idx, labels):
+    def _job(self, path, header, raw, scaler, cols, cofactors, label_idx, labels):
         try:
-            _hostio.write_points_csv(path, header, points_values(raw, scaler, cols), label_idx, labels)
+            _hostio.write_points_csv(path, header, points_values(raw, scaler, cols, cofactors), label_idx, labels)
         except BaseException as exc:  # surfaced by the next submit / by close
             self._error = exc
 
@@ -136,10 +165,13 @@ def output_headers(attributes, markers, gating):
     return result, ['id', 'cluster_id'] + attributes, stats
 
 
-def points_values(raw, scaler, cols=None):
-    """The values of cluster_points_D{t}.csv for the parsed cells `raw`: with a scaler, the clustering columns (`cols`, or
-    every column) hold inverse_transform(transform(x)), what the reference writes (app.py:175, 299-301); every other
-    column holds the parsed value."""
+def points_values(raw, scaler, cols=None, cofactors=None):
+    """The values of cluster_points_D{t}.csv for the parsed cells `raw`: a column with an arcsinh cofactor (`cofactors`, by
+    column; 0 = none) holds x = asinh(raw / c) (scaling.arcsinh), every other column x = the parsed value; then, with a
+    scaler, the clustering columns (`cols`, or every column) hold inverse_transform(transform(x)), what the reference
+    writes (app.py:175, 299-301)."""
+    if cofactors is not None:
+        raw = _hostio.arcsinh_host(raw, cofactors)
     if scaler is None:
         return raw
     if cols is None:
@@ -212,6 +244,17 @@ def _read_gates(path, attributes):
     for _, gate in frame.iterrows():
         gates.setdefault(int(gate['Day']), {})[tuple(gate[attributes].values)] = gate['PopName']
     return gates
+
+
+def transform_gates(gates, cofactors):
+    """The gating centroids of _read_gates (in the files' units) in the space the engine clusters: every marker with
+    cofactor c != 0 (`cofactors`, one per clustering marker) as asinh(x / c) (scaling.arcsinh)."""
+    out = {}
+    for day, by_centroid in gates.items():
+        cen = np.array([list(c) for c in by_centroid.keys()], np.float64).reshape(len(by_centroid), len(cofactors))
+        cen = _hostio.arcsinh_host(cen, cofactors)
+        out[day] = {tuple(row): name for row, name in zip(cen.tolist(), by_centroid.values())}
+    return out
 
 
 def find_closest_gating(gating_dict, cluster, scaler):
@@ -307,7 +350,7 @@ def setup_logger(log_dir):
 def run(data, output_directory, gating_centroid_file=None, normalise_data=True, restore_program=False,
         param_beta=0.8, param_delta=0.0, param_epsilon=0.03, param_lambda=0, param_k=1,
         param_mu=0.001, param_pi=0, param_omicron=0.0, param_upsilon=1, device=0, cluster_statistics=False,
-        clustering_markers=None):
+        clustering_markers=None, arcsinh_cofactors=None):
     """Run ChronoClust on a list of per-timepoint CSV files (in time order).  See the reference's app.run for the meaning of
     every parameter.  Additions: `device` (CUDA ordinal); `cluster_statistics` -- also write cluster_statistics.csv, per
     timepoint and lineage label the number of cells and their per-marker medians and means (the cells and values of
@@ -315,7 +358,14 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
     `clustering_markers` -- names of the markers to cluster on, from the first file's header, in the order given (default:
     every column).  The scaler is fitted on them, the gating file is read on them and result.csv's centroid columns are
     them; cluster_points_D{t}.csv and cluster_statistics.csv still cover every column of the files, the others holding
-    the parsed values.  An unknown or repeated name raises ValueError before any clustering."""
+    the parsed values.  An unknown or repeated name raises ValueError before any clustering.
+    `arcsinh_cofactors` -- cluster asinh(x / c) of cytometry intensities (scaling.arcsinh; typically c = 5 for mass and
+    around 150 for flow cytometry): a number applies to every clustering marker, a dict {marker name: cofactor} to the
+    markers it names, clustering or not (the others stay linear; 0 also means linear).  The transform runs on the device
+    as the cells are staged, the scaler is fitted on the transformed values, and the gating file keeps the files' units
+    (its centroids are transformed when read).  result.csv, cluster_points_D{t}.csv and cluster_statistics.csv then
+    hold transformed columns in transformed space; the cofactors are logged.  An unknown name or a cofactor that is not
+    0 or positive and finite raises ValueError before any clustering."""
     logger = setup_logger(os.path.join(output_directory, "logs"))
     logger.info("ChronoClust (B200 hot path) starts on cuda:%d with %d timepoint file(s)", device, len(data))
     values = (param_beta, param_delta, param_epsilon, param_lambda, param_k, param_mu, param_pi, param_omicron,
@@ -342,7 +392,12 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
         attributes = timepoints.attributes()
         cols = clustering_columns(attributes, clustering_markers)
         markers = attributes if cols is None else [attributes[c] for c in cols]
+        cofactors = arcsinh_cofactors_by_column(attributes, cols, arcsinh_cofactors)
         gates = _read_gates(gating_centroid_file, markers)
+        if cofactors is not None:
+            logger.info("arcsinh cofactors (0: linear): %s",
+                        ", ".join(f"{a}={c!r}" for a, c in zip(attributes, cofactors.tolist())))
+            gates = transform_gates(gates, cofactors if cols is None else cofactors[cols])
         header, points_header, stats_header = output_headers(attributes, markers, gating_centroid_file)
         result_path = os.path.join(output_directory, "result.csv")
         with open(result_path, 'w') as f:
@@ -355,7 +410,7 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
         scaler = None
         if normalise_data:
             logger.info("Fitting the joint min-max scaler over all timepoints")
-            scaler = _fit_joint_scaler(timepoints, range(len(data)), cols)
+            scaler = _fit_joint_scaler(timepoints, range(len(data)), cols, cofactors)
 
         for timepoint in range(len(data)):
             if resumed and hddstream.last_data_timestamp >= timepoint:
@@ -366,7 +421,7 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
 
             # ---- the hot path: online + offline clustering on the GPU (the min-max transform rides along on the device)
             hddstream.online_microcluster_maintenance(raw, timepoint, scaler=scaler.scaler if scaler else None,
-                                                      columns=cols)
+                                                      columns=cols, cofactors=cofactors)
 
             pcore_by_id = {mc.id[0]: mc for mc in hddstream.pcore_MC}
             for found in hddstream.final_clusters:
@@ -389,7 +444,7 @@ def run(data, output_directory, gating_centroid_file=None, normalise_data=True, 
                     csv.writer(f).writerows(_statistics_rows(timepoint, hddstream, by_lineage.child_clusters))
             label_idx, labels = _cell_labels(hddstream, by_lineage.child_clusters)
             writer.submit(os.path.join(output_directory, f"cluster_points_D{timepoint}.csv"),
-                          points_header, raw, scaler, cols, label_idx, labels)
+                          points_header, raw, scaler, cols, cofactors, label_idx, labels)
             timepoints.release(timepoint)
 
             by_lineage.transfer_child_to_parent()

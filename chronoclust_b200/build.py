@@ -13,11 +13,12 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "api.cu")
 DEPS = [os.path.join(HERE, "csrc", f) for f in ("api.cu", "common.cuh", "nearest.cuh", "online.cuh", "offline.cuh",
-                                                "engine.cuh", "stats.cuh", "debug.h")]
+                                                "engine.cuh", "stats.cuh", "debug.h", "asinh.h")]
 DEPS.append(os.path.join(os.path.dirname(HERE), "include", "chronoclust_b200.h"))
 SO = os.path.join(HERE, "libchronoclust_b200.so")
 SO_DEBUG = os.path.join(HERE, "libchronoclust_b200_debug.so")
 HOSTIO_SRC = os.path.join(HERE, "csrc", "hostio.c")
+HOSTIO_DEPS = [HOSTIO_SRC, os.path.join(HERE, "csrc", "asinh.h")]
 HOSTIO_SO = os.path.join(HERE, "libccb_hostio.so")
 
 NVCC_FLAGS = [
@@ -50,10 +51,13 @@ def build(force=False, verbose=False, debug=False):
 
 
 def build_hostio(force=False, verbose=False):
-    """The host-side CSV writer (plain C, pthreads; no CUDA): chronoclust_b200/libccb_hostio.so."""
-    if not force and os.path.exists(HOSTIO_SO) and os.path.getmtime(HOSTIO_SO) >= os.path.getmtime(HOSTIO_SRC):
+    """The host-side CSV writer and arcsinh transform (plain C, pthreads; no CUDA): chronoclust_b200/libccb_hostio.so.
+    -ffp-contract=off: csrc/asinh.h gives the device's bits only when no a * b + c is fused (GNU C's default is fast)."""
+    if not force and os.path.exists(HOSTIO_SO) and all(os.path.getmtime(HOSTIO_SO) >= os.path.getmtime(d)
+                                                       for d in HOSTIO_DEPS):
         return HOSTIO_SO
-    cmd = ["gcc", "-O2", "-std=gnu11", "-fPIC", "-shared", "-pthread", "-o", HOSTIO_SO, HOSTIO_SRC, "-lm"]
+    cmd = ["gcc", "-O2", "-std=gnu11", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", "-o", HOSTIO_SO, HOSTIO_SRC,
+           "-lm"]
     if verbose:
         print(" ".join(cmd))
     subprocess.check_call(cmd)

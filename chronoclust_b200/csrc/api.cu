@@ -7,6 +7,7 @@
 #include "debug.h"
 #endif
 
+#include <cfloat>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -185,6 +186,7 @@ struct ccb_handle {
     // widens them into d_X
     Grow<Dev<unsigned char>> d_stg;
     Grow<Dev<int32_t>> d_cols; // [CCB_MAX_D] column map of a column-subset ingest
+    Grow<Dev<double>> d_cof;   // [CCB_MAX_D] arcsinh cofactors of the last ingest by source column (0: linear)
     Grow<Dev<int32_t>> d_assign;
     Grow<Dev<uint8_t>> d_stage;
     Grow<Dev<int32_t>> d_pnew, d_pfin, d_onew; // kernel 3 plan codes
@@ -219,6 +221,7 @@ struct ccb_handle {
         int32_t dtype = CCB_DTYPE_F64, W = 0;
         uint64_t colmask = 0; // the clustering columns of a column-subset ingest (0: none)
         bool scaled = false, valid = false;
+        bool raw_tx = false; // X holds raw values of an ingest with cofactors (d_cof): ccb_cluster_stats transforms them
     } last;
     Event ev_seg[8];
     // offline results (host copies)
@@ -1230,10 +1233,11 @@ int stats_args(ccb_handle *h, int64_t N, int64_t ld, int D, int G, int nq, const
 }
 
 // The pipeline of stats.cuh over the rows X [N][ld] (CCB_DTYPE_*) grouped by d_group [N] (device; values outside [0, G)
-// are skipped).  xf: the per-column transform of the values (StXf in stats.cuh).  Outputs are host arrays.
+// are skipped).  xf: the per-column transform of the values (StXf in stats.cuh); cof: device arcsinh cofactors by column
+// applied first (k_st_gather_tx), or null.  Outputs are host arrays.
 // Synchronises s.  h (may be null) receives the error and counts the launches.  Arguments are checked by stats_args.
 int group_stats_run(ccb_handle *h, cudaStream_t s, const void *X, int32_t dtype, int64_t N, int64_t ld, int D,
-                    const int32_t *d_group, int G, int nq, const double *q, const StXf &xf, int64_t *count,
+                    const int32_t *d_group, int G, int nq, const double *q, const StXf &xf, const double *cof, int64_t *count,
                     double *mean, double *median, double *quant) {
     int64_t launches = 0;
     const int R = 2 + 2 * nq;
@@ -1305,7 +1309,13 @@ int group_stats_run(ccb_handle *h, cudaStream_t s, const void *X, int32_t dtype,
     int32_t *pnan = reinterpret_cast<int32_t *>(psum + (size_t)NS * D);
     if (NS > 0) {
         const size_t smem = (size_t)ST_CHUNK * (D + 1) * 8;
-        if (dtype == CCB_DTYPE_F32)
+        if (cof && dtype == CCB_DTYPE_F32)
+            k_st_gather_tx<float><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const float *>(X), ld, xf, cof, keys,
+                                                                       psum, pnan);
+        else if (cof)
+            k_st_gather_tx<double><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const double *>(X), ld, xf, cof,
+                                                                        keys, psum, pnan);
+        else if (dtype == CCB_DTYPE_F32)
             k_st_gather<float><<<(unsigned)NS, ST_THREADS, smem, s>>>(geo, static_cast<const float *>(X), ld, xf, keys, psum,
                                                                     pnan);
         else
@@ -1598,30 +1608,65 @@ int ccb_begin_timepoint(ccb_handle *h, double mu, double omicron, int64_t pi, in
     return sync_ctl(h);
 }
 
-// widen (and, with a scaler, min-max transform) n rows of dtype into double rows, on the handle's stream.  cols: the device
-// column map of a column-subset ingest (output column d = source column cols[d]), or null
-static void stage_rows(ccb_handle *h, int32_t dtype, const void *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t n,
-                       const int32_t *cols, const double *scale, const double *shift) {
-    if (n <= 0) return;
-    const int64_t total = n * h->D;
+// k_stage_rows over n rows of D columns on stream s: the instance with the arcsinh transform when cof is set
+static void launch_stage_rows(cudaStream_t s, int32_t dtype, const void *src, int64_t ld_src, double *dst, int64_t ld_dst,
+                              int64_t n, int D, const int32_t *cols, const double *cof, const double *scale,
+                              const double *shift) {
+    const int64_t total = n * D;
     const unsigned gx = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
-    if (dtype == CCB_DTYPE_F32)
-        k_stage_rows<float><<<gx, 256, 0, h->stream>>>(static_cast<const float *>(src), ld_src, dst, ld_dst, n, h->D, cols,
-                                                       scale, shift);
+    if (cof && dtype == CCB_DTYPE_F32)
+        k_stage_rows_tx<float><<<gx, 256, 0, s>>>(static_cast<const float *>(src), ld_src, dst, ld_dst, n, D, cols, cof, scale,
+                                                  shift);
+    else if (cof)
+        k_stage_rows_tx<double><<<gx, 256, 0, s>>>(static_cast<const double *>(src), ld_src, dst, ld_dst, n, D, cols, cof,
+                                                   scale, shift);
+    else if (dtype == CCB_DTYPE_F32)
+        k_stage_rows<float><<<gx, 256, 0, s>>>(static_cast<const float *>(src), ld_src, dst, ld_dst, n, D, cols, scale, shift);
     else
-        k_stage_rows<double><<<gx, 256, 0, h->stream>>>(static_cast<const double *>(src), ld_src, dst, ld_dst, n, h->D, cols,
-                                                        scale, shift);
+        k_stage_rows<double><<<gx, 256, 0, s>>>(static_cast<const double *>(src), ld_src, dst, ld_dst, n, D, cols, scale,
+                                                shift);
+}
+
+// widen (and, with cofactors, arcsinh transform, and, with a scaler, min-max transform) n rows of dtype into double rows,
+// on the handle's stream.  cols: the device column map of a column-subset ingest (output column d = source column
+// cols[d]), or null; cof: the device cofactors by source column, or null
+static void stage_rows(ccb_handle *h, int32_t dtype, const void *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t n,
+                       const int32_t *cols, const double *cof, const double *scale, const double *shift) {
+    if (n <= 0) return;
+    launch_stage_rows(h->stream, dtype, src, ld_src, dst, ld_dst, n, h->D, cols, cof, scale, shift);
     h->st.kernel_launches++;
 }
 
 static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int W, const int32_t *cols,
-                       int32_t *assign_uid, uint8_t *stage, const double *scale, const double *shift);
+                       const double *cof, int32_t *assign_uid, uint8_t *stage, const double *scale, const double *shift);
 
-// ccb_ingest_ex (cols null, W == D) and ccb_ingest_cols (cols: host [D] distinct columns of W-wide rows, checked by the
-// caller) after enter().
+// host arcsinh cofactors [n]: each 0 (the column stays linear) or positive and finite
+static int check_cofactors(ccb_handle *h, const double *cof, int n) {
+    for (int c = 0; c < n; ++c)
+        if (!(cof[c] >= 0.0 && cof[c] <= DBL_MAX)) // (NaN fails both)
+            return fail(h, CCB_EINVAL, "cofactor[%d] = %g: a cofactor is 0 (linear) or positive and finite", c, cof[c]);
+    return CCB_OK;
+}
+
+// ccb_ingest_ex (cols and cofactor null, W == D), ccb_ingest_cols (cofactor null) and ccb_ingest_tx after enter(): every
+// argument check, then the ingest.  cols: null (the identity; W must be D) or host [D] distinct columns of W-wide rows;
+// cofactor: null or host [W] arcsinh cofactors by source column.
 static int ingest_rows(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int W,
-                       const int32_t *cols, const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
+                       const int32_t *cols, const double *cofactor, const double *scale, const double *min_,
+                       int32_t *assign_uid, uint8_t *stage) {
     int rc;
+    if (!cols && W != h->D) return fail(h, CCB_EINVAL, "row width W = %d without a column map; D = %d", W, h->D);
+    if (cols) {
+        if (W < h->D || W > CCB_MAX_D) return fail(h, CCB_EINVAL, "row width W = %d outside [D = %d, %d]", W, h->D, CCB_MAX_D);
+        uint64_t seen = 0;
+        for (int d = 0; d < h->D; ++d) {
+            const int32_t c = cols[d];
+            if (c < 0 || c >= W) return fail(h, CCB_EINVAL, "cols[%d] = %d outside [0, W = %d)", d, c, W);
+            if ((seen >> c) & 1ull) return fail(h, CCB_EINVAL, "column %d appears twice in cols", c);
+            seen |= 1ull << c;
+        }
+    }
+    if (cofactor && (rc = check_cofactors(h, cofactor, W))) return rc;
     if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(h, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
     if (!scale != !min_) return fail(h, CCB_EINVAL, "scale and min_ must both be set or both be NULL");
     if (ld < W) return fail(h, CCB_EINVAL, "leading dimension %lld < %s = %d", (long long)ld, cols ? "W" : "D", W);
@@ -1646,30 +1691,37 @@ static int ingest_rows(ccb_handle *h, const void *X, int32_t dtype, int32_t on_d
         }
         if (scale) CK(h, cudaMemcpyAsync(h->d_scale + 2 * CCB_MAX_D, by_col, sizeof by_col, cudaMemcpyHostToDevice, h->stream));
     }
+    const double *d_cof = nullptr;
+    if (cofactor) {
+        CK(h, h->d_cof.ensure(CCB_MAX_D * sizeof(double)));
+        CK(h, cudaMemcpyAsync(h->d_cof, cofactor, (size_t)W * 8, cudaMemcpyHostToDevice, h->stream));
+        d_cof = h->d_cof;
+    }
     h->last.valid = false;
     auto record = [&](const void *rows, int32_t rows_dtype, int64_t ldr, const int32_t *assign) {
         h->last.X = rows, h->last.dtype = rows_dtype, h->last.ld = ldr, h->last.W = cols ? W : h->D, h->last.N = N;
         h->last.assign = assign, h->last.colmask = colmask, h->last.scaled = scale != nullptr;
+        h->last.raw_tx = cols && cofactor; // (the d_X rows the engine read are transformed already)
         h->last.valid = true;
     };
     if (!on_device) {
         // (ingest_host leaves the rows in d_X: unstaged float64 ones with the caller's leading dimension, staged ones
         // -- float32 or a column subset -- with D; the full rows it staged stay in d_stg with the caller's)
-        if ((rc = ingest_host(h, X, dtype, N, ld, W, d_cols, assign_uid, stage, d_sc, d_sh))) return rc;
+        if ((rc = ingest_host(h, X, dtype, N, ld, W, d_cols, d_cof, assign_uid, stage, d_sc, d_sh))) return rc;
         if (cols) record(h->d_stg, dtype, ld, h->d_assign);
         else record(h->d_X, CCB_DTYPE_F64, dtype == CCB_DTYPE_F32 ? h->D : ld, h->d_assign);
         return CCB_OK;
     }
-    // device-resident rows: float64 without a scaler or a column map go to the engine as they are; anything else is staged
-    // into d_X (leading dimension D) by one launch -- the caller's buffer is never written
-    if (dtype == CCB_DTYPE_F64 && !scale && !cols) {
+    // device-resident rows: float64 without a scaler, a column map or cofactors go to the engine as they are; anything else
+    // is staged into d_X (leading dimension D) by one launch -- the caller's buffer is never written
+    if (dtype == CCB_DTYPE_F64 && !scale && !cols && !cofactor) {
         const double *Xd = static_cast<const double *>(X);
         if ((rc = ingest_core_bsv(h, Xd, N, ld, assign_uid, stage))) return rc;
         record(Xd, CCB_DTYPE_F64, ld, assign_uid);
         return CCB_OK;
     }
     CK(h, h->d_X.ensure(((size_t)N * h->D + 2) * 8));
-    stage_rows(h, dtype, X, ld, h->d_X, h->D, N, d_cols, d_sc, d_sh);
+    stage_rows(h, dtype, X, ld, h->d_X, h->D, N, d_cols, d_cof, d_sc, d_sh);
     CKL(h);
     if ((rc = ingest_core_bsv(h, h->d_X, N, h->D, assign_uid, stage))) return rc;
     if (cols) record(X, dtype, ld, assign_uid);
@@ -1681,23 +1733,23 @@ int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device
                   const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
     int rc;
     if ((rc = enter(h))) return rc;
-    return ingest_rows(h, X, dtype, on_device, N, ld, h->D, nullptr, scale, min_, assign_uid, stage);
+    return ingest_rows(h, X, dtype, on_device, N, ld, h->D, nullptr, nullptr, scale, min_, assign_uid, stage);
 }
 
 int ccb_ingest_cols(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int32_t W,
                     const int32_t *cols, const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage) {
     int rc;
     if ((rc = enter(h))) return rc;
-    if (W < h->D || W > CCB_MAX_D) return fail(h, CCB_EINVAL, "row width W = %d outside [D = %d, %d]", W, h->D, CCB_MAX_D);
     if (!cols) return fail(h, CCB_EINVAL, "null column map");
-    uint64_t seen = 0;
-    for (int d = 0; d < h->D; ++d) {
-        const int32_t c = cols[d];
-        if (c < 0 || c >= W) return fail(h, CCB_EINVAL, "cols[%d] = %d outside [0, W = %d)", d, c, W);
-        if ((seen >> c) & 1ull) return fail(h, CCB_EINVAL, "column %d appears twice in cols", c);
-        seen |= 1ull << c;
-    }
-    return ingest_rows(h, X, dtype, on_device, N, ld, W, cols, scale, min_, assign_uid, stage);
+    return ingest_rows(h, X, dtype, on_device, N, ld, W, cols, nullptr, scale, min_, assign_uid, stage);
+}
+
+int ccb_ingest_tx(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int32_t W,
+                  const int32_t *cols, const double *cofactor, const double *scale, const double *min_, int32_t *assign_uid,
+                  uint8_t *stage) {
+    int rc;
+    if ((rc = enter(h))) return rc;
+    return ingest_rows(h, X, dtype, on_device, N, ld, W, cols, cofactor, scale, min_, assign_uid, stage);
 }
 
 int ccb_ingest_device(ccb_handle *h, const double *X_dev, int64_t N, int64_t ld, int32_t *assign_uid_dev,
@@ -1715,13 +1767,13 @@ int ccb_ingest_scaled(ccb_handle *h, const double *X_raw, int64_t N, int64_t ld,
     return ccb_ingest_ex(h, X_raw, CCB_DTYPE_F64, 0, N, ld, scale, min_, assign_uid, stage);
 }
 
-// host rows in, per-cell results out.  float64 rows are copied into d_X as they are (leading dimension ld) and, with a
-// scaler (scale / shift: device vectors), min-max transformed there in place; float32 rows, and the W-wide rows of a
-// column-subset ingest (cols: device column map), are copied into the staging buffer and gathered / widened (and
-// transformed) from there into d_X with leading dimension D.  Either happens segment by segment behind the segments'
-// copies.  Arguments are checked by ingest_rows.
+// host rows in, per-cell results out.  float64 rows are copied into d_X as they are (leading dimension ld) and, with
+// cofactors (cof: device vector) or a scaler (scale / shift: device vectors), transformed there in place; float32 rows,
+// and the W-wide rows of a column-subset ingest (cols: device column map), are copied into the staging buffer and
+// gathered / widened (and transformed) from there into d_X with leading dimension D.  Either happens segment by segment
+// behind the segments' copies.  Arguments are checked by ingest_rows.
 static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, int64_t ld, int W, const int32_t *cols,
-                       int32_t *assign_uid, uint8_t *stage, const double *scale, const double *shift) {
+                       const double *cof, int32_t *assign_uid, uint8_t *stage, const double *scale, const double *shift) {
     int rc;
     if (N == 0) return CCB_OK;
     const bool f32 = dtype == CCB_DTYPE_F32, staged = f32 || cols;
@@ -1737,8 +1789,8 @@ static int ingest_host(ccb_handle *h, const void *X, int32_t dtype, int64_t N, i
     char *dst = staged ? reinterpret_cast<char *>(h->d_stg.p) : reinterpret_cast<char *>(h->d_X.p); // where the copies land
     // the copied rows [r0, r0 + n) -> double rows in d_X, on the handle's stream behind the wait for their copy
     auto stage_seg = [&](int64_t r0, int64_t n) -> int {
-        if (staged || scale) {
-            stage_rows(h, dtype, dst + r0 * ld * esz, ld, h->d_X + r0 * ldX, ldX, n, cols, scale, shift);
+        if (staged || cof || scale) {
+            stage_rows(h, dtype, dst + r0 * ld * esz, ld, h->d_X + r0 * ldX, ldX, n, cols, cof, scale, shift);
             CKL(h);
         }
         return CCB_OK;
@@ -2280,6 +2332,22 @@ int ccb_colminmax_ex(int32_t device, void *stream, const void *X_dev, int32_t dt
     return launched(nullptr, "k_colminmax");
 }
 
+int ccb_arcsinh(int32_t device, void *stream, const void *X_dev, int32_t dtype, int64_t N, int64_t ld, int32_t D,
+                const double *cofactor, double *out_dev) {
+    if (dtype != CCB_DTYPE_F64 && dtype != CCB_DTYPE_F32) return fail(nullptr, CCB_EINVAL, "unknown input dtype %d", (int)dtype);
+    if (D < 1 || D > CCB_MAX_D || N < 0 || ld < D || !cofactor || (N > 0 && (!X_dev || !out_dev)))
+        return fail(nullptr, CCB_EINVAL, "bad ccb_arcsinh arguments");
+    if (int rc = check_cofactors(nullptr, cofactor, D)) return rc;
+    if (int rc = enter_device(device)) return rc;
+    if (N == 0) return CCB_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    Scratch sc(s);
+    CK(nullptr, sc.alloc((size_t)D * 8));
+    CK(nullptr, cudaMemcpyAsync(sc.p, cofactor, (size_t)D * 8, cudaMemcpyHostToDevice, s));
+    launch_stage_rows(s, dtype, X_dev, ld, out_dev, D, N, D, nullptr, sc.as<double>(), nullptr, nullptr);
+    return launched(nullptr, "k_stage_rows (ccb_arcsinh)");
+}
+
 int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, int64_t ld, int32_t D, double *min_dev,
                   double *max_dev) {
     return ccb_colminmax_ex(device, stream, X_dev, CCB_DTYPE_F64, N, ld, D, min_dev, max_dev);
@@ -2361,7 +2429,7 @@ int ccb_group_stats(int32_t device, void *stream, const void *X, int32_t dtype, 
     if (int rc = stats_args(nullptr, N, ld, D, G, nq, q, count, mean, median, quant)) return rc;
     if (N > 0 && (!X || !group)) return fail(nullptr, CCB_EINVAL, "null rows or groups");
     if (int rc = enter_device(device)) return rc;
-    return group_stats_run(nullptr, (cudaStream_t)stream, X, dtype, N, ld, D, group, G, nq, q, StXf{}, count, mean, median,
+    return group_stats_run(nullptr, (cudaStream_t)stream, X, dtype, N, ld, D, group, G, nq, q, StXf{}, nullptr, count, mean, median,
                            quant);
 }
 
@@ -2400,7 +2468,8 @@ int ccb_cluster_stats(ccb_handle *h, const int32_t *group_of_pcore, int64_t n_pc
     } else if (h->last.scaled) { // the scaled rows the engine read: transformed back
         xf.scale = h->d_scale, xf.shift = h->d_scale + CCB_MAX_D, xf.mask = ~0ull >> (64 - h->D);
     }
-    return group_stats_run(h, s, h->last.X, h->last.dtype, N, h->last.ld, h->last.W, group, G + 1, nq, q, xf, count, mean,
+    return group_stats_run(h, s, h->last.X, h->last.dtype, N, h->last.ld, h->last.W, group, G + 1, nq, q, xf,
+                           h->last.raw_tx ? h->d_cof.p : nullptr, count, mean,
                            median, quant);
 }
 

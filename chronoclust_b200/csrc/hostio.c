@@ -13,7 +13,12 @@
  * is found by trying 15, 16 and 17 significant digits (from 1 digit on for subnormals) ("%.{p}e" is correctly rounded in glibc) and checking the round trip
  * with strtod: if p digits suffice, the correctly rounded p-digit decimal is the shortest representation.
  *
- * Plain C (gcc), pthreads; no CUDA here.  Built next to the CUDA library by chronoclust_b200/build.py.
+ * It also holds the host side of the arcsinh transform, ccbio_arcsinh_host: the same csrc/asinh.h the kernels use, so
+ * its output is the device's bit for bit.
+ *
+ * Plain C (gcc), pthreads; no CUDA here.  Built next to the CUDA library by chronoclust_b200/build.py, with
+ * -ffp-contract=off (GNU C contracts a * b + c into an FMA by default where the target has one; asinh.h needs every
+ * operation rounded on its own).
  */
 #define _GNU_SOURCE
 #include <errno.h>
@@ -25,6 +30,8 @@
 #include <stdlib.h>
 #include <string.h>
 #include <unistd.h>
+
+#include "asinh.h"
 
 /* repr(v) into out (at least 32 bytes); returns the length */
 static int fmt_repr(double v, char *out) {
@@ -250,6 +257,54 @@ done:
     free(slabs);
     free(tids);
     return rc;
+}
+
+typedef struct {
+    const void *X;
+    int32_t dtype, D;
+    int64_t r0, r1, ld;
+    const double *cofactor;
+    double *out;
+} asinh_slab_t;
+
+static void *asinh_slab(void *arg) {
+    const asinh_slab_t *s = (const asinh_slab_t *)arg;
+    for (int64_t r = s->r0; r < s->r1; ++r) {
+        double *o = s->out + r * s->D;
+        for (int d = 0; d < s->D; ++d) {
+            double x = s->dtype == 1 ? (double)((const float *)s->X)[r * s->ld + d] : ((const double *)s->X)[r * s->ld + d];
+            if (s->cofactor[d] != 0.0) x = ccb_asinh(x / s->cofactor[d]);
+            o[d] = x;
+        }
+    }
+    return NULL;
+}
+
+/* out [N][D] (float64, contiguous) = X [N][ld] (dtype 0: float64, 1: float32) widened to double, and every column d with
+ * cofactor[d] != 0 transformed to ccb_asinh(x / cofactor[d]) -- ccb_arcsinh's values, bit for bit.  Cofactors are
+ * checked by the caller.  nthreads <= 0: one per online core (at most 64).  Returns 0 or an errno value. */
+int ccbio_arcsinh_host(const void *X, int32_t dtype, int64_t N, int64_t ld, int32_t D, const double *cofactor, double *out,
+                       int32_t nthreads) {
+    if (N < 0 || D < 0 || ld < D || (dtype != 0 && dtype != 1) || (N > 0 && (!X || !cofactor || !out))) return EINVAL;
+    if (nthreads <= 0) nthreads = (int32_t)sysconf(_SC_NPROCESSORS_ONLN);
+    if (nthreads > 64) nthreads = 64;
+    if (nthreads < 1) nthreads = 1;
+    if ((int64_t)nthreads > (N + 4095) / 4096) nthreads = (int32_t)((N + 4095) / 4096); /* >= 4096 rows a thread */
+    if (nthreads < 1) nthreads = 1;
+    asinh_slab_t slabs[64];
+    pthread_t tids[64];
+    for (int k = 0; k < nthreads; ++k) {
+        asinh_slab_t *s = &slabs[k];
+        s->X = X, s->dtype = dtype, s->D = D, s->ld = ld, s->cofactor = cofactor, s->out = out;
+        s->r0 = N * k / nthreads, s->r1 = N * (k + 1) / nthreads;
+        if (k == 0 || pthread_create(&tids[k], NULL, asinh_slab, s) != 0) {
+            asinh_slab(s); /* the first slab, or no thread available: do it here */
+            tids[k] = (pthread_t)0;
+        }
+    }
+    for (int k = 1; k < nthreads; ++k)
+        if (tids[k]) pthread_join(tids[k], NULL);
+    return 0;
 }
 
 /* repr(v) for tests: writes into out (>= 32 bytes), returns the length */

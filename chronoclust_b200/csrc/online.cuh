@@ -9,11 +9,12 @@
 // Kernel 3   k_maint_plan + k_maint_gather: fused decay x 2^(-lambda dt) (hddstream.py:247-286), downgrade with the
 //            reference's skip-next-after-removal iteration and outlier deletion (hddstream.py:512-549), order-preserving
 //            compaction.
-// Input      k_stage_rows / k_colminmax: float32 / float64 rows (optionally a subset of their columns) widened to double
-//            and min-max transformed, and the fit
+// Input      k_stage_rows / k_colminmax: float32 / float64 rows (optionally a subset of their columns) widened to double,
+//            optionally arcsinh(x / cofactor) transformed (asinh.h) and min-max transformed, and the fit
 //            reductions (scaling/scaler.py:11-53).
 #pragma once
 #include "common.cuh"
+#include "asinh.h"
 
 namespace ccb {
 
@@ -293,21 +294,35 @@ __global__ void k_repack_store(Store S, int n, int D, int DP, double wsel) {
 // the same thread, hence no __restrict__ on src / dst.  HBM-bound: 8 + 8 B (double) or 4 + 8 B (float) per element.
 // cols (device [D], or null = the identity): output column d is source column cols[d].  The map sits in shared memory; a
 // warp's 32 consecutive outputs still read from one or two source rows, so the reads of a row stay coalesced.
-template <typename T>
-__global__ void k_stage_rows(const T *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t N, int D,
-                             const int32_t *__restrict__ cols, const double *__restrict__ scale,
-                             const double *__restrict__ shift) {
+// k_stage_rows_tx: the same with the arcsinh transform.  cof (device, indexed by SOURCE column) holds the cofactors, and
+// a column with cofactor c != 0 gets ccb_asinh(x / c) after the widening and before the scaler -- one IEEE division, then
+// asinh.h's restatement of fdlibm, which gives the host's bits.  The cofactors of the D output columns sit in shared
+// memory.  With no map and no scaler this is ccb_arcsinh's kernel.  (Two kernels over one body: the untransformed inputs
+// keep a kernel of their own, with its own register allocation.)
+template <typename T, bool TX>
+__device__ __forceinline__ void stage_rows_body(const T *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t N, int D,
+                                                const int32_t *__restrict__ cols, const double *__restrict__ cof,
+                                                const double *__restrict__ scale, const double *__restrict__ shift) {
     __shared__ int32_t s_col[CCB_MAX_D];
+    __shared__ double s_cof[TX ? CCB_MAX_D : 1];
     auto rows = [&](auto col_of) { // (one loop body, instantiated for the identity and for the map)
         const int64_t total = N * D;
         for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
             const int64_t r = e / D;
             const int d = (int)(e - r * D);
             double x = (double)src[r * ld_src + col_of(d)];
+            if constexpr (TX) {
+                const double c = s_cof[d];
+                if (c != 0.0) x = ccb_asinh(ddiv(x, c));
+            }
             if (scale) x = dadd(dmul(x, scale[d]), shift[d]);
             dst[r * ld_dst + d] = x;
         }
     };
+    if constexpr (TX) {
+        for (int d = threadIdx.x; d < D; d += blockDim.x) s_cof[d] = cof[cols ? cols[d] : d];
+        if (!cols) __syncthreads();
+    }
     if (cols) {
         for (int d = threadIdx.x; d < D; d += blockDim.x) s_col[d] = cols[d];
         __syncthreads();
@@ -315,6 +330,18 @@ __global__ void k_stage_rows(const T *src, int64_t ld_src, double *dst, int64_t 
     } else {
         rows([](int d) { return d; });
     }
+}
+template <typename T>
+__global__ void k_stage_rows(const T *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t N, int D,
+                             const int32_t *__restrict__ cols, const double *__restrict__ scale,
+                             const double *__restrict__ shift) {
+    stage_rows_body<T, false>(src, ld_src, dst, ld_dst, N, D, cols, nullptr, scale, shift);
+}
+template <typename T>
+__global__ void k_stage_rows_tx(const T *src, int64_t ld_src, double *dst, int64_t ld_dst, int64_t N, int D,
+                                const int32_t *__restrict__ cols, const double *__restrict__ cof,
+                                const double *__restrict__ scale, const double *__restrict__ shift) {
+    stage_rows_body<T, true>(src, ld_src, dst, ld_dst, N, D, cols, cof, scale, shift);
 }
 
 // fit: column-wise minimum / maximum ignoring NaN (np.nanmin / np.nanmax, what MinMaxScaler.partial_fit uses).

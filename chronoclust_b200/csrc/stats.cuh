@@ -6,7 +6,7 @@
 //                            slice) and their slices -- four exclusive scans in one launch
 //   3. k_st_sort_hist/scatter stable LSD counting sort of the rows by group (8-bit digits): a deterministic permutation, so
 //                            every later sum runs in the same order on every call
-//   4. k_st_gather           the rows in group order, widened to double (and scaled per column) -> column-major order-preserving
+//   4. k_st_gather           the rows in group order, widened to double (and transformed per column) -> column-major order-preserving
 //                            uint64 keys; per (slice, marker) partial sums and NaN counts, each summed in row order
 //   5. k_st_small            groups of <= ST_SLICE cells: one CTA each, bitonic sort of each marker in shared memory
 //      k_st_rsel_*           larger groups: radix select (8 passes x 8 bits) of every needed rank, the histograms of every
@@ -15,6 +15,7 @@
 // Every reduction is either integer or in a fixed order: two calls give bit-identical results.
 #pragma once
 #include "common.cuh"
+#include "asinh.h"
 
 namespace ccb {
 
@@ -265,9 +266,12 @@ struct StXf {
 
 // One CTA per slice: rows staged ST_CHUNK at a time in shared memory (coalesced row reads, coalesced column writes).
 // Thread m < D sums column m over the chunk in row order and adds the chunk to the slice's sum: a fixed order.
-template <typename T>
-__global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, int64_t ld, StXf xf, uint64_t *keys,
-                                                          double *psum, int32_t *pnan) {
+// k_st_gather_tx (the rows hold raw values of an ingest with arcsinh cofactors): a column m with cof[m] != 0 (device
+// [CCB_MAX_D], indexed by column) is transformed to ccb_asinh(x / cof[m]) first, as k_stage_rows_tx transformed it for
+// the engine.  (Two kernels over one body, as k_stage_rows / k_stage_rows_tx.)
+template <typename T, bool TX>
+__device__ __forceinline__ void st_gather_body(const StGeom &g, const T *X, int64_t ld, const StXf &xf, const double *cof,
+                                               uint64_t *keys, double *psum, int32_t *pnan) {
     extern __shared__ double st_tile[]; // [ST_CHUNK][D + 1]
     const int D = g.D, P = D + 1, t = threadIdx.x;
     int grp, len;
@@ -280,6 +284,10 @@ __global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, 
         for (int e = t; e < rows * D; e += ST_THREADS) {
             const int r = e / D, m = e - r * D;
             double v = (double)X[(int64_t)g.perm[start + c0 + r] * ld + m];
+            if constexpr (TX) {
+                const double c = cof[m];
+                if (c != 0.0) v = ccb_asinh(ddiv(v, c));
+            }
             if ((xf.mask >> m) & 1ull) {
                 if (xf.fwd) v = dadd(dmul(v, xf.scale[m]), xf.shift[m]);
                 v = ddiv(dsub(v, xf.shift[m]), xf.scale[m]);
@@ -306,6 +314,17 @@ __global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, 
         psum[(int64_t)blockIdx.x * D + t] = sum;
         pnan[(int64_t)blockIdx.x * D + t] = nan;
     }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(ST_THREADS) k_st_gather(StGeom g, const T *X, int64_t ld, StXf xf, uint64_t *keys,
+                                                          double *psum, int32_t *pnan) {
+    st_gather_body<T, false>(g, X, ld, xf, nullptr, keys, psum, pnan);
+}
+template <typename T>
+__global__ void __launch_bounds__(ST_THREADS) k_st_gather_tx(StGeom g, const T *X, int64_t ld, StXf xf, const double *cof,
+                                                             uint64_t *keys, double *psum, int32_t *pnan) {
+    st_gather_body<T, true>(g, X, ld, xf, cof, keys, psum, pnan);
 }
 
 // sum / NaN count of (group, marker) over the group's slices, in slice order

@@ -13,7 +13,8 @@ import sys
 
 import numpy as np
 
-from . import _lib, cellstats
+from . import _hostio, _lib, cellstats
+from .scaling import cofactor_vector
 from .objects import FinalCluster, Microcluster
 
 
@@ -78,26 +79,28 @@ class _PointsView(object):
     overwrites its array or tensor in place after the call changes what `points` hands out.  float32 rows are handed out
     widened to float64, and the rows of a CUDA tensor are gathered on its device and brought back as float64 -- the same
     values the float64 path hands out.  Rows ingested with a column map hand out their clustering columns only, in map
-    order."""
+    order; rows ingested with arcsinh cofactors hand out the transformed values (the host's ccbio_arcsinh_host, the
+    device's bits)."""
 
     def __init__(self):
-        self.segments = []  # [(X, assign_uid, scaler, column map)] since the last reset (hddstream.py:208-213)
+        self.segments = []  # [(X, assign_uid, scaler, column map, cofactors)] since the last reset (hddstream.py:208-213)
         self._index = None
 
     def reset(self):
         self.segments = []
         self._index = None
 
-    def add(self, X, assign, scaler=None, cols=None):
+    def add(self, X, assign, scaler=None, cols=None, cof=None):
         """scaler = (scale_, min_): X holds RAW rows that were scaled on the device; the coordinates handed out are
         X * scale_ + min_ of the requested rows (numpy's elementwise arithmetic = the device's two roundings).
-        cols: int32 column map into the rows of X (the coordinates are X[:, cols]), or None."""
-        self.segments.append((X, assign, scaler, cols))
+        cols: int32 column map into the rows of X (the coordinates are X[:, cols]), or None.  cof: float64 arcsinh
+        cofactors by column of X (applied before the scaler), or None."""
+        self.segments.append((X, assign, scaler, cols, cof))
         self._index = None
 
     def _build(self):
         idx = {}
-        for si, (_, assign, _sc, _cols) in enumerate(self.segments):
+        for si, (_, assign, _sc, _cols, _cof) in enumerate(self.segments):
             order = np.argsort(assign, kind="stable")
             sa = assign[order]
             cuts = np.flatnonzero(np.diff(sa)) + 1
@@ -117,17 +120,20 @@ class _PointsView(object):
     def points_of(self, uid):
         out = {}
         for si, rows in self.rows_of(uid):
-            X, _, sc, cols = self.segments[si]
+            X, _, sc, cols, cof = self.segments[si]
             if isinstance(X, np.ndarray):
                 sel = X[rows] if cols is None else X[np.ix_(rows, cols)]
-                sel = sel.astype(np.float64, copy=False)  # (widened before the scaler arithmetic)
             else:  # a CUDA tensor
                 import torch
 
                 sel = X[torch.from_numpy(rows).to(X.device)]
                 if cols is not None:
                     sel = sel[:, torch.from_numpy(cols.astype(np.int64)).to(X.device)]
-                sel = sel.to(torch.float64).cpu().numpy()
+                sel = sel.cpu().numpy()
+            if cof is not None:  # (widened, then transformed, before the scaler arithmetic)
+                sel = _hostio.arcsinh_host(sel, cof if cols is None else cof[cols])
+            else:
+                sel = sel.astype(np.float64, copy=False)
             if sc is not None:
                 sel = sel * sc[0]
                 sel = sel + sc[1]
@@ -266,7 +272,7 @@ class HDDStream(object):
 
     # ------------------------------------------------------------------------------------------
     def online_microcluster_maintenance(self, input_dataset, input_dataset_daystamp, reset_param=True,
-                                        run_offline=True, scaler=None, columns=None):
+                                        run_offline=True, scaler=None, columns=None, cofactors=None):
         """input_dataset: [N, D] cells -- a numpy array, a CPU tensor or a CUDA tensor on this instance's device.  float32 and
         float64 rows with unit column stride go in without a copy (row-strided views included); float32 rows are widened
         to float64 on the device, which is exact, so results are those of the float64 path on the widened rows.  Other
@@ -281,7 +287,16 @@ class HDDStream(object):
         clusters input_dataset[:, columns] (dataset_dimensionality = D) and gives bit for bit what the float64 path gives on
         those gathered rows; the gather runs on the device, the rows go in without a copy as above, and the scaler's vectors
         have D entries.  `points` hands out the gathered coordinates, and cluster_statistics reports all W columns.
-        ValueError before any device work for a bad entry (see column_map) or a D that differs from the handle's."""
+        ValueError before any device work for a bad entry (see column_map) or a D that differs from the handle's.
+
+        cofactors (extension): the arcsinh transform of cytometry intensities, run on the device as the rows are staged --
+        a number for every column, or one per column of input_dataset (W entries with `columns`, by input column); a
+        column with cofactor c > 0 is clustered as asinh(x / c) (scaling.arcsinh: widened first, one IEEE division, then
+        csrc/asinh.h, the same bits on host and device), one with c = 0 stays linear.  The order is: widen, gather,
+        asinh, scaler, so the scaler belongs to the transformed values.  Results are those of the float64 path on
+        scaling.arcsinh(input_dataset, cofactors) (then gathered), bit for bit; `points` and cluster_statistics report
+        transformed columns in transformed space.  ValueError before any device work for a bad cofactor (see
+        scaling.cofactor_vector)."""
         xp, dtype, on_device, ld, X = _input_rows(input_dataset, self._device)
         if X.ndim != 2:
             raise ValueError("input_dataset must be 2-D")
@@ -289,6 +304,7 @@ class HDDStream(object):
         D = X.shape[1] if cols is None else len(cols)
         if cols is not None and self._h is not None and D != self._handle_dim:
             raise ValueError(f"{D} columns given; this HDDStream clusters {self._handle_dim} markers")
+        cof = None if cofactors is None else cofactor_vector(cofactors, X.shape[1])
         sc = mn = None
         if scaler is not None:
             sc, mn = (scaler.scale_, scaler.min_) if hasattr(scaler, "scale_") else scaler
@@ -325,19 +341,15 @@ class HDDStream(object):
         logger.info("Starting online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
         self._last_device_input = self._stats_width = None
         if on_device:
-            assign, stage = self._ingest_tensor(X, xp, dtype, ld, sc, mn, cols)
+            assign, stage = self._ingest_tensor(X, xp, dtype, ld, sc, mn, cols, cof)
         else:
             assign = np.empty(N, np.int32)
             stage = np.empty(N, np.uint8)
-            if cols is None:
-                _lib.check(L.ccb_ingest_ex(h, xp, dtype, 0, N, ld, _lib.ptr(sc), _lib.ptr(mn), _lib.ptr(assign),
-                                           _lib.ptr(stage)), h)
-            else:
-                _lib.check(L.ccb_ingest_cols(h, xp, dtype, 0, N, ld, X.shape[1], _lib.ptr(cols), _lib.ptr(sc), _lib.ptr(mn),
-                                             _lib.ptr(assign), _lib.ptr(stage)), h)
+            _lib.check(L.ccb_ingest_tx(h, xp, dtype, 0, N, ld, X.shape[1], _lib.ptr(cols), _lib.ptr(cof), _lib.ptr(sc),
+                                       _lib.ptr(mn), _lib.ptr(assign), _lib.ptr(stage)), h)
         if cols is not None:
             self._stats_width = X.shape[1]
-        self._views.add(X, assign, None if sc is None else (sc, mn), cols)
+        self._views.add(X, assign, None if sc is None else (sc, mn), cols, cof)
         self.last_assignment, self.last_stage = assign, stage
         self._lists = [None, None]
         logger.info("Finish online microcluster maintenance for timepoint {}".format(input_dataset_daystamp))
@@ -347,10 +359,9 @@ class HDDStream(object):
         if run_offline:
             self.offline_clustering(input_dataset_daystamp)
 
-    def _ingest_tensor(self, X, xp, dtype, ld, sc, mn, cols=None):
-        """ccb_ingest_ex (ccb_ingest_cols with a column map) on the rows of a CUDA tensor X: the handle's stream first waits
-        for the work queued on the current torch stream (whatever produced X), and the per-cell results come back to the
-        host behind the engine."""
+    def _ingest_tensor(self, X, xp, dtype, ld, sc, mn, cols=None, cof=None):
+        """ccb_ingest_tx on the rows of a CUDA tensor X: the handle's stream first waits for the work queued on the current
+        torch stream (whatever produced X), and the per-cell results come back to the host behind the engine."""
         import torch
 
         N = X.shape[0]
@@ -359,12 +370,8 @@ class HDDStream(object):
         assign_d = torch.empty(N, dtype=torch.int32, device=X.device)
         stage_d = torch.empty(N, dtype=torch.uint8, device=X.device)
         mine.wait_stream(cur)  # (after the allocations: earlier users of that memory on `cur` are done first)
-        if cols is None:
-            _lib.check(_lib.lib().ccb_ingest_ex(self._h, xp, dtype, 1, N, ld, _lib.ptr(sc), _lib.ptr(mn),
-                                                assign_d.data_ptr(), stage_d.data_ptr()), self._h)
-        else:
-            _lib.check(_lib.lib().ccb_ingest_cols(self._h, xp, dtype, 1, N, ld, X.shape[1], _lib.ptr(cols), _lib.ptr(sc),
-                                                  _lib.ptr(mn), assign_d.data_ptr(), stage_d.data_ptr()), self._h)
+        _lib.check(_lib.lib().ccb_ingest_tx(self._h, xp, dtype, 1, N, ld, X.shape[1], _lib.ptr(cols), _lib.ptr(cof),
+                                            _lib.ptr(sc), _lib.ptr(mn), assign_d.data_ptr(), stage_d.data_ptr()), self._h)
         # the copies, and the release of the temporaries, are ordered on `cur` behind everything the handle queued
         cur.wait_stream(mine)
         self._last_device_input = (X, assign_d)  # the handle reads both again in cluster_statistics
@@ -534,7 +541,8 @@ class HDDStream(object):
         cluster_points_D{t}.csv holds them); median and quantiles are numpy's bit for bit (see group_statistics).
         After an ingest with `columns`, the statistics cover every one of the W columns of input_dataset (arrays [.., W]):
         a clustering column as just described (under a scaler: inverse_transform(transform(x))), every other column as
-        the raw value widened to float64.
+        the raw value widened to float64.  After an ingest with `cofactors`, every column with a cofactor is reported in
+        transformed space (asinh(x / c), then as just described).
 
         groups: optional integer array over the pcore list (pcore_MC order, -1 = no group) replacing the clusters of the
         offline phase; the result then has max(groups) + 2 rows.  ValueError without an offline result or `groups`;

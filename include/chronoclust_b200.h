@@ -14,7 +14,7 @@
  *   ccb_begin_timepoint     decay + downgrade + reset               clustering/hddstream.py:199-213,
  *                                                                    247-286, 512-549
  *   ccb_ingest[_device|_ex| the ordered per-point loop              clustering/hddstream.py:220-237,
- *              _cols]       (_add_to_pcore, _add_to_outlier,          288-343, 345-395, 397-430, 434-462
+ *              _cols|_tx]   (_add_to_pcore, _add_to_outlier,          288-343, 345-395, 397-430, 434-462
  *                            _upgrade_outlier_microcluster,          objects/microcluster.py:89-153,
  *                            _create_new_outlier_cluster)             167-197, 213-233
  *                                                                    utilities/mc_functions.py:14-62
@@ -32,6 +32,9 @@
  *                           (multi-GPU offline path, config C4)
  *   ccb_cluster_stats /     (extension) per-cluster cell counts,    replaces grouping cluster_points_D{t}.csv
  *   ccb_group_stats         means, medians, quantiles of a timepoint  on the host after a run
+ *   ccb_ingest_tx /         (extension) arcsinh(x / cofactor) of    replaces the caller's host pass (or
+ *   ccb_arcsinh             cytometry intensities, one definition    torch.asinh) before clustering
+ *                           for host and device (csrc/asinh.h)
  *
  * The derived constants (epsilon**2, upsilon*epsilon, delta**2, 2**(-lambda*dt), mu*N, omicron*N_prev,
  * round(pi)) are evaluated by the Python host with Python's own float semantics, exactly where the
@@ -180,6 +183,19 @@ int ccb_ingest_ex(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device
  * entry, or anything ccb_ingest_ex rejects. */
 int ccb_ingest_cols(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int32_t W,
                     const int32_t *cols, const double *scale, const double *min_, int32_t *assign_uid, uint8_t *stage);
+/* ccb_ingest_cols with the arcsinh transform of cytometry intensities (extension).  cols: as ccb_ingest_cols, or NULL for
+ * the identity (then W must be D).  cofactor: host [W] by SOURCE column, or NULL for none; a column with cofactor c != 0
+ * is read as asinh((double)x / c) (csrc/asinh.h's ccb_asinh: widened first, one IEEE division, then a restatement of fdlibm's
+ * asinh that gives the same bits on host and device), a column with c == 0 stays linear.  The order is: widen, gather,
+ * asinh, scaler.  Results are those of ccb_ingest_ex on ccbio_arcsinh_host's output (gathered), bit for bit.  X is never
+ * written: host float64 rows are transformed in their device copy, every other input by the staging launch.
+ * Afterwards ccb_cluster_stats reports the transformed columns in transformed space (clustering columns under a scaler
+ * brought back through it as after the other ingests).  CCB_EINVAL: a cofactor that is NaN, negative or infinite, W != D
+ * without cols, or anything ccb_ingest_cols rejects; with cols and cofactor NULL this is ccb_ingest_cols, without both
+ * ccb_ingest_ex. */
+int ccb_ingest_tx(ccb_handle *h, const void *X, int32_t dtype, int32_t on_device, int64_t N, int64_t ld, int32_t W,
+                  const int32_t *cols, const double *cofactor, const double *scale, const double *min_, int32_t *assign_uid,
+                  uint8_t *stage);
 
 /* Offline phase over the current pcore list; returns the number of clusters. */
 int ccb_offline(ccb_handle *h, int64_t *n_clusters);
@@ -240,6 +256,14 @@ int ccb_colminmax(int32_t device, void *stream, const double *X_dev, int64_t N, 
  * of the rows widened to double.  An unknown dtype: CCB_EINVAL. */
 int ccb_colminmax_ex(int32_t device, void *stream, const void *X_dev, int32_t dtype, int64_t N, int64_t ld, int32_t D,
                      double *min_dev, double *max_dev);
+/* The arcsinh transform of ccb_ingest_tx on its own (extension): out_dev [N][D] (float64, contiguous) = X_dev [N][ld]
+ * (CCB_DTYPE_*, ld in elements) widened to double, every column d with cofactor[d] != 0 as asinh(x / cofactor[d]) (ccb_asinh).
+ * cofactor: host [D].  The values the engine clusters, for plots or for fitting the scaler with ccb_colminmax_ex; the
+ * host library's ccbio_arcsinh_host (chronoclust_b200/csrc/hostio.c) gives the same bits.  Asynchronous on `stream`.
+ * CCB_EINVAL: an unknown dtype, D outside [1, 64], ld < D, N < 0, null pointers, or a cofactor that is NaN, negative or
+ * infinite. */
+int ccb_arcsinh(int32_t device, void *stream, const void *X_dev, int32_t dtype, int64_t N, int64_t ld, int32_t D,
+                const double *cofactor, double *out_dev);
 
 /* Association scan (SURVEY 8f-1; replaces the inner loops of TrackByHistoricalAssociation.track_cluster_history,
  * tracking/cluster_tracker.py:127-144): for every CURRENT pcore microcluster q the index of the previous-timepoint
