@@ -12,7 +12,7 @@ ENGINE_CATEGORIES = ("chain_p", "nearest", "verify", "speculate", "lists", "chai
 
 
 def golden():
-    z = load("stress_downgrade.npz")  # 4 timepoints of 2 500 cells, decay and downgrades from the second one on
+    z = load("stress_downgrade.npz")  # 4 timepoints of 2 500 cells, decay and outlier deletions from the second one on
     return z, stress_inputs(z)
 
 
